@@ -1,9 +1,10 @@
 """Timing of the UNMODIFIED reference rollout loop (src/main.py:673-737) on host cores.
 
 Used only by bench.py (`cpu_baseline_reference`, kind "reference") next to the oracle port.  The reference's own
-classes are imported from the staged copy baseline/_ref/src (written by __graft_entry__.build() where /root/reference
-exists; git-ignored); gymnasium / matplotlib / torch_geometric, which the reference imports but this image lacks,
-are stubbed by tools/ref_stubs.py.  P worker processes (SURVEY 8d: one per host core, torch threads = 1) each run
+classes are imported from an unedited copy of its src/ placed at baseline/_ref/src (git-ignored, not part of this
+repository; without it the reference arm is skipped); gymnasium / matplotlib / torch_geometric, which the reference
+imports for features this timing does not use, are stubbed by tools/ref_stubs.py.  P worker processes (SURVEY 8d: one
+per host core, torch threads = 1) each run
 
     policy(obs, adj) -> NetMonWrapper.step(actions) -> buff.add(...)            [one env instance per process]
 

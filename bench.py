@@ -3,6 +3,7 @@
 forward; % of HBM roofline for the env-step kernel).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload cfg2|cfg2ln|cfg3|cfg4]
+                    [--dump-outputs DIR]
 
 One "step" = one batched rollout step over B environment instances per GPU
 (src/main.py:673-737): DQN epsilon-greedy action selection -> Routing env step with agent and
@@ -193,8 +194,8 @@ def cpu_arm(cfg_name, steps, warmup, envs=None, budget_s=20.0):
 
 
 def reference_arm(cfg_name, seconds=8.0):
-    """The UNMODIFIED Python reference (staged at baseline/_ref/src) running its own rollout loop, one process per
-    host core (baseline/ref_rollout.py).  None when the staged copy is absent or the workload is not config 2's."""
+    """The UNMODIFIED Python reference (a copy of its src/ placed at baseline/_ref/src) running its own rollout loop, one
+    process per host core (baseline/ref_rollout.py).  None when that copy is absent or the workload is not config 2's."""
     try:
         from baseline import ref_rollout
         from graph_marl_b200.rollout import CONFIGS
@@ -205,6 +206,35 @@ def reference_arm(cfg_name, seconds=8.0):
         return ref_rollout.time_reference(c, seconds=seconds, warmup_steps=5 if c["n_nodes"] <= 50 else 1)
     except Exception as ex:  # never hide the GPU number behind the baseline
         return dict(value=None, unit=UNIT, kind="reference", sample=f"failed: {ex}")
+
+
+def dump_outputs(ro, out_dir, budget_bytes=60_000_000):
+    """Writes what the rollout's last step handed its caller to out_dir/<name>.npy (float32): the next agent and graph
+    observations, agent adjacency and NetMon state, and the actions, rewards and done flags the step wrote into the
+    replay ring.  The rollout acts with epsilon 1 (random actions), so `q_values` adds the DQN's Q-values on the next
+    observations (a greedy act(): no random draws) to cover its GEMMs.  Files hold the same fixed, seeded sample of env
+    instances, as many as fit `budget_bytes`."""
+    import math
+
+    import numpy as np
+    import torch
+
+    ro.join_streams()  # a dense-ring insert may still run on its side stream
+    B, buff = ro.B, ro.buff
+    slots = (buff.index - B + torch.arange(B, device=buff.reward.device)) % buff.buffer_size  # env e -> its ring slot
+    obs_a, obs_g = ro.obs  # obs_g may exist only tile-packed (model.PackedRows): .float() unpacks it
+    with torch.no_grad():
+        q, _ = ro.model.act(obs_a, obs_g, epsilon=0.0, want_q=True)
+    full = dict(obs_agent=obs_a, obs_graph=obs_g, adj=ro.adj, netmon_state=ro.env.current_netmon_state,
+                action=buff.action[slots], reward=buff.reward[slots], done=buff.done[slots], q_values=q)
+    per_env = 4 * sum(math.prod(t.shape[1:]) for t in full.values())
+    k = min(B, budget_bytes // per_env)
+    env = np.sort(np.random.default_rng(0).choice(B, k, replace=False))
+    sel = torch.from_numpy(env).to(obs_a.device)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in full.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.float().index_select(0, sel).cpu().numpy())
+    print(f"dump: outputs of the last timed step, {k} of {B} env instances -> {out_dir}", file=sys.stderr)
 
 
 _REAL_STDOUT = None
@@ -251,7 +281,14 @@ def main():
                          "(cfg2 4096, cfg3 16384) sharded over the ranks")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--per-kernel", action="store_true", help="also print a per-stage CUDA-event breakdown to stderr")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the outputs of the last one and the DQN's Q-values on its next "
+                         "observations to DIR/<name>.npy (float32, rank 0's env instances, a fixed seeded sample of them "
+                         "under 64 MB): same arguments, same inputs, so that two builds can be compared output for output")
     a = ap.parse_args()
+    if a.dump_outputs and (a.impl != "ours" or a.no_replay):
+        ap.error("--dump-outputs reads the last step's actions, rewards and done flags from the replay ring of the GPU "
+                 "rollout: it needs --impl ours without --no-replay")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
@@ -292,9 +329,9 @@ def main():
         if rank != 0:
             return
         # The reference's own CPU implementation of the path: the UNMODIFIED Python rollout loop (src/main.py:673-737,
-        # staged at baseline/_ref/src) with one process per host core -- the reference has no batching, every process
+        # a copy placed at baseline/_ref/src) with one process per host core -- the reference has no batching, every process
         # advances one env instance.  The oracle port (C env + torch CPU tensors, all cores, the GPU arm's env count) is
-        # timed beside it and becomes the line's value only where the staged reference is absent.
+        # timed beside it and becomes the line's value only where that copy is absent.
         cbr = reference_arm(a.workload, seconds=max(6.0, min(20.0, 0.4 * (a.steps + a.warmup))))
         cb, sec_per_step, Bc = cpu_arm(a.workload, a.steps, a.warmup, envs=(B_weak if N <= 50 else None), budget_s=45.0)
         use_ref = cbr is not None and cbr.get("value")
@@ -374,6 +411,8 @@ def main():
     value, ms, launches, w0, w1 = timed(ro, a.steps, max(a.warmup, 3), host=False)
     clocks = sampler.stop(w0, w1) if sampler else None
     host_issue_ms = host_ms[0]
+    if a.dump_outputs and rank == 0:
+        dump_outputs(ro, a.dump_outputs)
 
     # ---- per-kernel timing for the roofline (CUDA events on the launching stream) -------------
     stage = ro.profile_stages(iters=max(5, min(a.steps, 20)))

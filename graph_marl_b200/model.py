@@ -65,6 +65,18 @@ class PackedRows:
     def device(self):
         return self.buf.device
 
+    def float(self):
+        """The rows as an fp32 tensor of `shape` (hi + lo; hi alone in single-pass bf16, which writes no lo part)."""
+        K = self.shape[-1]
+        R = 1
+        for n in self.shape[:-1]:
+            R *= n
+        mt, kb = -(-R // 128), K // 32
+        # block (mt, kb) -> [hi|lo] planes of [r>>3][(k&31)>>3][r&7][k&7] bf16 elements (layout in csrc/gemm_sm100.cuh)
+        x = self.buf.reshape(-1)[:mt * kb * 16384].view(torch.bfloat16).view(mt, kb, 2, 16, 4, 8, 8).float()
+        x = x[:, :, 0] if self.math == "bf16" else x[:, :, 0] + x[:, :, 1]
+        return x.permute(0, 2, 4, 1, 3, 5).reshape(mt * 128, K)[:R].reshape(self.shape)
+
 
 class _PackedWeights:
     """Cache of the tensor-core weight pack (bf16 hi/lo tiles) of a module; rebuilt whenever a

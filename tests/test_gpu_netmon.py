@@ -343,7 +343,7 @@ def test_unmodified_reference_main_py_runs_on_the_package(tmp_path):
 
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
     if not os.path.exists(os.path.join(root, "baseline", "_ref", "src", "main.py")):
-        pytest.skip("baseline/_ref/src is not staged (run __graft_entry__.build() where /root/reference exists)")
+        pytest.skip("runs the original project's own driver: needs a copy of its src/ at baseline/_ref/src")
     cmd = [sys.executable, os.path.join(root, "tools", "run_reference_driver.py"), "main.py"] + (
         "--model=dqn --hidden-dim=8 --random-topology=1 --mini-batch-size=32 --device=cuda --episode-steps=1 "
         "--eval-episode-steps=1 --lr=0.001 --tau=0.01 --netmon --netmon-encoder-dim=4 --hidden-dim=4 --netmon-dim=2 "
@@ -365,7 +365,7 @@ def test_unmodified_reference_sl_py_runs_on_the_package(tmp_path):
 
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
     if not os.path.exists(os.path.join(root, "baseline", "_ref", "src", "sl.py")):
-        pytest.skip("baseline/_ref/src is not staged (run __graft_entry__.build() where /root/reference exists)")
+        pytest.skip("runs the original project's own driver: needs a copy of its src/ at baseline/_ref/src")
     cmd = [sys.executable, os.path.join(root, "tools", "run_reference_driver.py"), "sl.py", "--iterations", "40",
            "--num-samples-train", "200", "--validate-after", "20", "--test-sequence-lengths", "1,4", "--disable-progressbar"]
     r = subprocess.run(cmd, cwd=tmp_path, capture_output=True, text=True, timeout=1200)

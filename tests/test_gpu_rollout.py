@@ -204,3 +204,42 @@ def test_random_topology_pool_rollout_graph_equals_eager(rnn, H, enc):
             d = (x.float() - y.float()).abs().reshape(x.shape[0], -1).max(dim=1)[0]
             bad.append((name, int((d > 0).sum()), float(d.max()), (d > 0).nonzero().flatten()[:8].tolist()))
     assert not bad, bad
+
+
+def test_bench_dump_outputs_are_the_last_step(tmp_path):
+    """bench.py --dump-outputs: after eager steps the arrays are what the last step handed its caller (the graph
+    observation, kept only tile-packed, unpacks to the rows the ring's rebuild of the transition computes in fp32, up to
+    the bf16 hi/lo split; the Q-values are the DQN's on the next observations).  After the same steps run as replayed
+    CUDA-graph units -- the path bench.py times, where the ring index and the carried tensors come from the replay
+    bookkeeping -- the dump is the same, array for array."""
+    import bench
+    from graph_marl_b200.model import PackedRows
+    from oracle import netmon_oracle as NO
+
+    a = _mk(0, replay="compact", B=40)
+    a.run(9)
+    reward, done, _ = a.step()
+    b = _mk(5, replay="compact", B=40)
+    b.run(10)
+    assert b._graphs and not a._graphs
+    dumps = []
+    for ro, sub in ((a, "eager"), (b, "graph")):
+        bench.dump_outputs(ro, str(tmp_path / sub))
+        dumps.append({p.stem: np.load(p) for p in (tmp_path / sub).iterdir()})
+    d, dg = dumps
+    assert sorted(d) == sorted(dg) == sorted(("obs_agent", "obs_graph", "adj", "netmon_state", "action", "reward", "done", "q_values"))
+    assert all(v.dtype == np.float32 and v.shape[0] == a.B for v in d.values())  # 40 envs fit: no sampling
+    assert np.array_equal(d["reward"], reward.cpu().numpy()) and np.array_equal(d["done"], done.float().cpu().numpy())
+    assert np.array_equal(d["obs_agent"], a.obs[0].cpu().numpy()) and np.array_equal(d["adj"], a.adj.float().cpu().numpy())
+    assert np.array_equal(d["netmon_state"], a.env.current_netmon_state.cpu().numpy())
+    assert isinstance(a.obs[1], PackedRows)
+    tb = a.buff._get_transition_batch((a.buff.index - a.B + np.arange(a.B)) % a.buff.buffer_size, "cuda")
+    assert np.array_equal(d["action"], tb.action.float().cpu().numpy())
+    tail = tb.next_obs[..., a.sizes["Da"]:].cpu().numpy()
+    assert d["obs_graph"].shape == tail.shape and np.abs(tail).max() > 0
+    assert np.abs(d["obs_graph"] - tail).max() <= 2.0 ** -14 * np.abs(tail).max()
+    w_dq = {k: v.detach().cpu().numpy() for k, v in a.model.state_dict().items()}
+    q_ref = NO.dqn_forward(w_dq, np.concatenate([d["obs_agent"], tail], -1))
+    assert d["q_values"].shape == (a.B, 20, 4) and np.abs(d["q_values"] - q_ref).max() < 1e-3
+    for name in d:
+        assert np.array_equal(d[name], dg[name]), name

@@ -356,6 +356,30 @@ def test_dqn_tensorcore_q_values(math, tol):
         assert np.array_equal(a2.cpu().numpy(), g["q"].argmax(-1))
 
 
+def test_dqn_q_head_with_several_tiles_per_cta():
+    """The config-2 DQN over 4096 envs x 20 agents (640 M tiles, several per CTA): the Q head's epilogue sums the partial
+    Q-values of its four column groups through shared memory behind a barrier of all epilogue warps.  Every row must match
+    the fp64 oracle, in every call (greedy actions = argmax)."""
+    from graph_marl_b200.model import DQN
+    from oracle import netmon_oracle as NO
+
+    torch.manual_seed(4)
+    dqn = DQN(130 + 512, (512, 256), 4, F.leaky_relu, math="bf16x3").cuda().eval()
+    w = {k: v.detach().cpu().numpy() for k, v in dqn.state_dict().items()}
+    rng = np.random.default_rng(4)
+    obs_a = torch.from_numpy((rng.random((4096, 20, 130)) < 0.1).astype(np.float32)).cuda()
+    obs_g = torch.from_numpy(rng.standard_normal((4096, 20, 512)).astype(np.float32) * 0.3).cuda()
+    rows = rng.choice(4096 * 20, 4096, replace=False)
+    x = torch.cat((obs_a, obs_g), -1).reshape(-1, 642).cpu().numpy()[rows]
+    ref = NO.dqn_forward(w, x, dtype=np.float64)
+    for _ in range(3):
+        with torch.no_grad():
+            q, a = dqn.act(obs_a, obs_g)
+        q = q.reshape(-1, 4).cpu().numpy()
+        assert np.abs(q[rows] - ref).max() < 1e-4
+        assert np.array_equal(a.reshape(-1).cpu().numpy(), q.argmax(-1))
+
+
 @pytest.mark.parametrize("switch", ["GM_TC_PAIR", "GM_TC_WIDE", "GM_TC_CLUSTER", "GM_AGG_MAP=2", "GM_AGG_MAP=2:mean", "GM_AGG_MAP=2:wrap",
                                     "GM_AGG_PIPE_GENERIC=1", "GM_AGG_MAP=8:mean", "GM_AGG_MAP=8", "GM_AGG_STAGE_LISTS=0"])
 def test_optional_kernel_variants_match(switch):

@@ -4,8 +4,8 @@
     python tools/run_reference_driver.py main.py --env-type=simple --model=dqn --netmon ... --device=cuda
     GM_DEFAULT_DEVICE=cuda python tools/run_reference_driver.py sl.py --iterations 200 ...      # sl.py has no --device
 
-The drivers are executed from the staged copy of the reference (baseline/_ref/src, written by
-__graft_entry__.build(); git-ignored, never edited).  Before the driver starts, the modules it imports for the
+The drivers are executed from an unedited copy of the reference's src/ (baseline/_ref/src, git-ignored and not part of
+this repository, or $GM_REFERENCE_SRC).  Before the driver starts, the modules it imports for the
 hot path are aliased in sys.modules to this package -- the import swap INTEGRATION.md section 2 describes:
 
     env.network / env.routing / env.simple_environment / env.wrapper / env.environment / env.constants,
@@ -71,7 +71,7 @@ def main():
         raise SystemExit(__doc__)
     driver = os.path.join(REF_SRC, sys.argv[1])
     if not os.path.exists(driver):
-        raise SystemExit(f"{driver} is missing: run `python __graft_entry__.py` where /root/reference exists to stage it")
+        raise SystemExit(f"{driver} is missing: copy the src/ directory of jw3il/graph-marl to {REF_SRC}")
     install_aliases()
     if os.environ.get("GM_DEFAULT_DEVICE"):
         # sl.py has no --device flag: it builds its tensors on torch's default device (the CPU); this package has no CPU
