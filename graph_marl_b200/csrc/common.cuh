@@ -60,33 +60,6 @@ struct ProfileScope {
     }
 };
 
-// ---- programmatic dependent launch -------------------------------------------------------------------------------
-// Every kernel of the rollout step calls pdl_trigger() first and pdl_wait() before it touches anything an earlier
-// kernel wrote, and is launched with the "programmatic stream serialization" attribute (launch_pdl): the CTAs of
-// kernel i+1 become resident on each SM as soon as kernel i's CTA there has exited, run their prologue (barrier
-// init, TMEM allocation, index arithmetic) and then block until kernel i has completed and flushed.  That takes the
-// launch latency and the prologue of the ~16 kernels of a step off the critical path -- in principle: measured on the
-// B200 the captured step got SLOWER (0.775 -> 0.82 ms), so the attribute is off unless GM_PDL=1 (the instructions are
-// no-ops then).
-bool pdl_enabled();
-__device__ __forceinline__ void pdl_trigger() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
-__device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
-
-template <typename... KArgs, typename... Args>
-inline cudaError_t launch_pdl(void (*kern)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t s, Args... args) {
-    cudaLaunchConfig_t cfg{};
-    cfg.gridDim = grid;
-    cfg.blockDim = block;
-    cfg.dynamicSmemBytes = smem;
-    cfg.stream = s;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = pdl_enabled() ? 1 : 0;
-    cfg.attrs = attr;
-    cfg.numAttrs = 1;
-    return cudaLaunchKernelEx(&cfg, kern, KArgs(args)...);
-}
-
 constexpr unsigned FULL = 0xffffffffu;
 constexpr int kNumSMs = 148;
 

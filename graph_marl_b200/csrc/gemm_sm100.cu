@@ -67,7 +67,6 @@ namespace tc {
 #endif
 
 constexpr int BM = TC_BM, BK = TC_BK, STAGES = 4, ACC_STAGES = 2;
-constexpr int PAIR_STAGES = 6;  // 2-CTA pairs stage half a weight tile per CTA: 32 KiB per stage at BN = 256
 constexpr int EPI_WARPS = 8, PROD_WARPS = 8;
 constexpr int MMA_WARP = 16, W_WARP = 17;
 constexpr int THREADS = 32 * 18;
@@ -107,29 +106,6 @@ __device__ __forceinline__ void fence_proxy_async_smem() { asm volatile("fence.p
 __device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
 __device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
 
-// multicast form: the bytes land at the same CTA-relative smem offset of every CTA in `mask` and
-// complete_tx on the mbarrier at the same offset in each of them
-__device__ __forceinline__ void bulk_g2s_mc(uint32_t dst, const void* src, uint32_t bytes, uint32_t bar, uint16_t mask) {
-    asm volatile(
-        "cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster [%0], [%1], %2, [%3], %4;" ::"r"(dst),
-        "l"(src), "r"(bytes), "r"(bar), "h"(mask)
-        : "memory");
-}
-__device__ __forceinline__ void umma_commit_mc(uint32_t bar, uint16_t mask) {
-    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(bar),
-                 "h"(mask)
-                 : "memory");
-}
-__device__ __forceinline__ void cluster_sync_all() {
-    asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory");
-    asm volatile("barrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
-__device__ __forceinline__ uint32_t cluster_ctarank() {
-    uint32_t r;
-    asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
-    return r;
-}
-
 __device__ __forceinline__ void bulk_g2s(uint32_t dst, const void* src, uint32_t bytes, uint32_t bar) {
     asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(dst),
                  "l"(src), "r"(bytes), "r"(bar)
@@ -154,51 +130,6 @@ __device__ __forceinline__ void umma(uint32_t tmem_d, uint64_t da, uint64_t db, 
         "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}" ::"r"(tmem_d),
         "l"(da), "l"(db), "r"(idesc), "r"(accumulate)
         : "memory");
-}
-__host__ __device__ constexpr uint32_t umma_idesc_m(int BN, int M) {
-    return (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(BN >> 3) << 17) | ((uint32_t)(M >> 4) << 24);
-}
-// cta_group::2: one instruction drives the tensor cores of both SMs of the pair (M = 256: rows 0-127 from the leader's
-// shared memory / TMEM, rows 128-255 from the peer's; each CTA holds half of the B rows)
-__device__ __forceinline__ void umma2(uint32_t tmem_d, uint64_t da, uint64_t db, uint32_t idesc, uint32_t accumulate) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "setp.ne.b32 p, %4, 0;\n\t"
-        "tcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n\t}" ::"r"(tmem_d),
-        "l"(da), "l"(db), "r"(idesc), "r"(accumulate)
-        : "memory");
-}
-// arrives (once) on the mbarrier at the same shared-memory offset in every CTA of `mask`
-__device__ __forceinline__ void umma2_commit_mc(uint32_t bar, uint16_t mask) {
-    asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(bar),
-                 "h"(mask)
-                 : "memory");
-}
-// arrive on the mbarrier at this CTA-relative address in CTA `cta` of the cluster
-__device__ __forceinline__ void mbar_arrive_remote(uint32_t bar, uint32_t cta) {
-    asm volatile(
-        "{\n\t.reg .b32 ra;\n\t"
-        "mapa.shared::cluster.u32 ra, %0, %1;\n\t"
-        "mbarrier.arrive.release.cluster.shared::cluster.b64 _, [ra];\n\t}" ::"r"(bar),
-        "r"(cta)
-        : "memory");
-}
-__device__ __forceinline__ bool mbar_try_wait_cluster(uint32_t bar, uint32_t parity) {
-    uint32_t ok;
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "mbarrier.try_wait.parity.acquire.cluster.shared::cta.b64 p, [%1], %2;\n\t"
-        "selp.u32 %0, 1, 0, p;\n\t}"
-        : "=r"(ok)
-        : "r"(bar), "r"(parity)
-        : "memory");
-    return ok != 0;
-}
-__device__ __forceinline__ void mbar_wait_cluster(uint32_t bar, uint32_t parity) {
-    uint32_t spins = 0;
-    while (!mbar_try_wait_cluster(bar, parity)) {
-        if (++spins > (1u << 22)) __trap();
-    }
 }
 __device__ __forceinline__ void umma_commit(uint32_t bar) {
     asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
@@ -326,24 +257,16 @@ __device__ __forceinline__ int ptr_align_floats(const float* p, int64_t ld) {
 // byte offset of the 16-byte chunk (row r, k-chunk kc) inside one bf16 part of a [128 x 32] block
 __device__ __forceinline__ uint32_t core_off(int r, int kc) { return (uint32_t)((r >> 3) * SBO_BYTES + kc * 128 + (r & 7) * 16); }
 
-// PAIR: the CTAs of a 2-CTA cluster (one TPC) run ONE tcgen05.mma.cta_group::2 (M = 256) per step: each CTA stages the
-// activation block of its own M tile and HALF of the weight tile (rows rank*BN/2 ..), the tensor cores of both SMs
-// read the two halves from both shared memories.  Weight bytes per CTA and shared-memory operand reads per MMA
-// halve.  Only the leader (cluster rank 0) issues MMAs; the peer's MMA thread relays "my stage is full" to the
-// leader, both CTAs' epilogue threads release the accumulator stage on the leader's barrier.
-template <int BN, int PASSES, int EPI, int NCG, bool PAIR>
+template <int BN, int PASSES, int EPI, int NCG>
 // 18 warps: 5 on one SM sub-partition (16K registers each) -> 96 registers per thread at most
 __global__ void __launch_bounds__(THREADS, 1) linear_tc_kernel(const TcArgs p) {
-    constexpr int W_PART_BYTES = (PAIR ? BN / 2 : BN) * BK * 2;  // this CTA's rows of one bf16 part of a weight stage
-    constexpr int W_SRC_PART_BYTES = BN * BK * 2;                // one bf16 part of the packed weight tile in global memory
+    constexpr int W_PART_BYTES = BN * BK * 2;  // one bf16 part of a weight stage
     constexpr int STAGE_BYTES = 2 * A_PART_BYTES + 2 * W_PART_BYTES;
-    constexpr int NST = PAIR ? PAIR_STAGES : STAGES;
-    constexpr uint32_t IDESC = PAIR ? umma_idesc_m(BN, 2 * BM) : umma_idesc(BN);
-    static_assert(!PAIR || EPI != EPI_LNLSTM, "the LayerNormLSTM mode owns whole M tiles per CTA");
+    constexpr uint32_t IDESC = umma_idesc(BN);
     constexpr bool LN = EPI == EPI_LNLSTM;
     constexpr int ACC_COLS = LN ? 2 * BN : BN;  // LayerNormLSTM: separate accumulators for x W_ih^T and h W_hh^T
     extern __shared__ __align__(128) uint8_t smem[];
-    __shared__ __align__(8) uint64_t bars[3 * NST + 2 * ACC_STAGES];
+    __shared__ __align__(8) uint64_t bars[2 * STAGES + 2 * ACC_STAGES];
     __shared__ uint32_t tmem_base_smem;
     __shared__ float qpart[EPI == EPI_QHEAD ? 2 : 1][EPI == EPI_QHEAD ? NCG - 1 : 1][EPI == EPI_QHEAD ? BM : 1][TC_MAX_ACT];
     // Q-head weights [n_act, N <= 256]: every epilogue thread needs all of them for every tile; from global memory (the L1
@@ -362,38 +285,28 @@ __global__ void __launch_bounds__(THREADS, 1) linear_tc_kernel(const TcArgs p) {
     __shared__ __align__(16) float ln_prm_s[LN ? 16 * BN : 4];
     __shared__ __align__(16) float ln_cin_s[LN ? 16 * 32 : 1][8];  // per epilogue thread: previous cell state of the tile's 8 units (cp.async)
 
-    pdl_trigger();  // the next kernel's CTAs may take this SM as soon as this CTA has exited
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const uint32_t smem_base = smem_u32(smem);
-    const uint32_t bar_full = smem_u32(&bars[0]), bar_empty = smem_u32(&bars[NST]);
-    const uint32_t bar_tfull = smem_u32(&bars[2 * NST]), bar_tempty = smem_u32(&bars[2 * NST + ACC_STAGES]);
-    const uint32_t bar_pfull = smem_u32(&bars[2 * NST + 2 * ACC_STAGES]);  // PAIR, leader: the peer's stage is full
+    const uint32_t bar_full = smem_u32(&bars[0]), bar_empty = smem_u32(&bars[STAGES]);
+    const uint32_t bar_tfull = smem_u32(&bars[2 * STAGES]), bar_tempty = smem_u32(&bars[2 * STAGES + ACC_STAGES]);
 
     if (threadIdx.x == 0) {
-        for (int s = 0; s < NST; s++) {
+        for (int s = 0; s < STAGES; s++) {
             // the copy thread's expect_tx arrive, plus the 256 producer threads when a segment is fp32
             mbar_init(bar_full + 8 * s, 1 + (p.has_prod ? PROD_WARPS * 32 : 0));
-            // one tcgen05.commit per CTA of the cluster when weights are multicast; the leader's commit alone for a pair
-            mbar_init(bar_empty + 8 * s, PAIR ? 1 : p.csz);
-            mbar_init(bar_pfull + 8 * s, 1);
+            mbar_init(bar_empty + 8 * s, 1);  // tcgen05.commit
         }
         for (int a = 0; a < ACC_STAGES; a++) {
-            mbar_init(bar_tfull + 8 * a, 1);                              // tcgen05.commit
-            // every epilogue thread; in a pair one elected lane per epilogue warp of both CTAs (remote arrives are not free)
-            mbar_init(bar_tempty + 8 * a, PAIR ? 2 * EPI_W : EPI_W * 32);
+            mbar_init(bar_tfull + 8 * a, 1);           // tcgen05.commit
+            mbar_init(bar_tempty + 8 * a, EPI_W * 32);  // every epilogue thread
         }
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
     if (warp == MMA_WARP) {  // TMEM: ACC_STAGES x BN fp32 columns x 128 lanes
         uint32_t dst = smem_u32(&tmem_base_smem);
         uint32_t cols = ACC_STAGES * ACC_COLS;
-        if (PAIR) {
-            asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(dst), "r"(cols) : "memory");
-            asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
-        } else {
-            asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(dst), "r"(cols) : "memory");
-            asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-        }
+        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(dst), "r"(cols) : "memory");
+        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
     }
     if (EPI == EPI_QHEAD) {
         for (int i = threadIdx.x; i < p.n_act * p.N; i += THREADS) qw_s[i / p.N][i % p.N] = __ldg(p.q_w + i);
@@ -403,26 +316,19 @@ __global__ void __launch_bounds__(THREADS, 1) linear_tc_kernel(const TcArgs p) {
     }
     tc_fence_before();
     __syncthreads();
-    if (p.csz > 1) cluster_sync_all();  // peers' barriers are initialised before anyone signals them
     tc_fence_after();
     const uint32_t tmem_base = tmem_base_smem;
-    pdl_wait();  // barriers and TMEM are set up: from here on the kernel reads what its predecessors wrote
 
-    // Work units: (group of csz consecutive M tiles, one N tile).  The CTAs of a cluster walk the same
-    // unit list in lockstep; CTA `rank` owns M tile mg*csz + rank and 1/csz of every weight stage copy.
-    const int csz = p.csz;
-    const int rank = csz > 1 ? (int)cluster_ctarank() : 0;
-    const uint16_t mc_mask = (uint16_t)((1u << csz) - 1u);
+    // Work units: (M tile, N tile), unit u of the grid at mt = u / n_tiles, nt = u % n_tiles; CTA b takes units b, b + grid, ...
     const int n_tiles = p.n_tiles;
-    const int n_clusters = (int)gridDim.x / csz, cluster_id = (int)blockIdx.x / csz;
-    const int total_units = ((p.m_tiles + csz - 1) / csz) * n_tiles;
-    // LayerNormLSTM: a CTA owns whole M tiles (row statistics couple the N tiles of a row), csz == 1
-    const int my_units = LN ? ((p.m_tiles - cluster_id + n_clusters - 1) / n_clusters) * n_tiles
-                            : (total_units - cluster_id + n_clusters - 1) / n_clusters;
+    const int n_ctas = (int)gridDim.x, cta = (int)blockIdx.x;
+    // LayerNormLSTM: a CTA owns whole M tiles (row statistics couple the N tiles of a row)
+    const int my_units = LN ? ((p.m_tiles - cta + n_ctas - 1) / n_ctas) * n_tiles
+                            : (p.m_tiles * n_tiles - cta + n_ctas - 1) / n_ctas;
     const int kblocks = p.Kp / BK;
     const int kb_seg1 = p.K0p / BK;  // first k-block of segment 1
-    auto unit_mt = [&](int i) { return LN ? cluster_id + (i / n_tiles) * n_clusters : ((cluster_id + i * n_clusters) / n_tiles) * csz + rank; };
-    auto unit_nt = [&](int i) { return LN ? i % n_tiles : (cluster_id + i * n_clusters) % n_tiles; };
+    auto unit_mt = [&](int i) { return LN ? cta + (i / n_tiles) * n_ctas : (cta + i * n_ctas) / n_tiles; };
+    auto unit_nt = [&](int i) { return LN ? i % n_tiles : (cta + i * n_ctas) % n_tiles; };
 
     if (NCG == 2 && warp >= EPI_WARPS && warp < EPI_WARPS + PROD_WARPS) {
         // ================= producer: fp32 activations -> bf16 hi/lo core matrices ================
@@ -469,8 +375,8 @@ __global__ void __launch_bounds__(THREADS, 1) linear_tc_kernel(const TcArgs p) {
                 for (int u = 0; u < 3; u++) {
                     const uint32_t it = base + u;
                     if (it >= total_it) break;
-                    const int s = it % NST;
-                    const uint32_t ph = (it / NST) & 1;
+                    const int s = it % STAGES;
+                    const uint32_t ph = (it / STAGES) & 1;
                     fetch(it + 2, buf[(u + 2) % 3]);
                     const int kb = (int)(it % kblocks);
                     const bool mine = (kb >= kb_seg1) ? prod1 : prod0;
@@ -496,18 +402,15 @@ __global__ void __launch_bounds__(THREADS, 1) linear_tc_kernel(const TcArgs p) {
             constexpr uint32_t w_bytes = (PASSES == 3 ? 2 : 1) * W_PART_BYTES;
             constexpr uint32_t a_bytes = (PASSES == 3 ? 2 : 1) * A_PART_BYTES;
             const int kb0_blocks = kb_seg1, kb1_blocks = kblocks - kb_seg1;
-            const uint32_t w_slice = W_PART_BYTES / csz;  // this CTA's share of each weight part
             uint32_t it = 0;
             for (int u = 0; u < my_units; u++) {
                 const int mt = unit_mt(u), nt = unit_nt(u);
-                const bool tile_live = mt < p.m_tiles;  // a dead tile of the last group copies no activations
                 for (int kb = 0; kb < kblocks; kb++, it++) {
-                    const int s = it % NST;
-                    const uint32_t ph = (it / NST) & 1;
+                    const int s = it % STAGES;
+                    const uint32_t ph = (it / STAGES) & 1;
                     const bool seg1 = kb >= kb_seg1;
                     const uint8_t* apk = seg1 ? p.A1pk : p.A0pk;
-                    if (!tile_live) apk = nullptr;
-                    mbar_wait(bar_empty + 8 * s, ph ^ 1);  // every CTA of the cluster has retired its MMAs on this stage
+                    mbar_wait(bar_empty + 8 * s, ph ^ 1);  // the MMAs on this stage have retired
 #if GM_TC_PROBES
                     if (p.a_stages & 8) {  // GM_TC_DEBUG & 8, timing probe: no copies at all (the MMAs run on stale shared memory)
                         mbar_arrive(bar_full + 8 * s);
@@ -515,21 +418,8 @@ __global__ void __launch_bounds__(THREADS, 1) linear_tc_kernel(const TcArgs p) {
                     }
 #endif
                     mbar_arrive_expect_tx(bar_full + 8 * s, w_bytes + (apk ? a_bytes : 0u));
-                    const uint8_t* src = p.Wp + ((size_t)nt * kblocks + kb) * (2 * W_SRC_PART_BYTES);
-                    const uint32_t w_dst = smem_base + s * STAGE_BYTES + 2 * A_PART_BYTES;
-                    if (PAIR) {  // this CTA's half of the rows of each part
-#pragma unroll
-                        for (int part = 0; part < (PASSES == 3 ? 2 : 1); part++)
-                            bulk_g2s(w_dst + part * W_PART_BYTES, src + part * W_SRC_PART_BYTES + rank * W_PART_BYTES, W_PART_BYTES,
-                                     bar_full + 8 * s);
-                    } else if (csz == 1) {
-                        bulk_g2s(w_dst, src, w_bytes, bar_full + 8 * s);
-                    } else {
-#pragma unroll
-                        for (int part = 0; part < (PASSES == 3 ? 2 : 1); part++)
-                            bulk_g2s_mc(w_dst + part * W_PART_BYTES + rank * w_slice, src + part * W_PART_BYTES + rank * w_slice, w_slice,
-                                        bar_full + 8 * s, mc_mask);
-                    }
+                    const uint8_t* src = p.Wp + ((size_t)nt * kblocks + kb) * (2 * W_PART_BYTES);
+                    bulk_g2s(smem_base + s * STAGE_BYTES + 2 * A_PART_BYTES, src, w_bytes, bar_full + 8 * s);
                     if (apk) {
                         const size_t blk = seg1 ? ((size_t)mt * kb1_blocks + (kb - kb_seg1)) : ((size_t)mt * kb0_blocks + kb);
                         bulk_g2s(smem_base + s * STAGE_BYTES, apk + blk * TC_PK_BLOCK, a_bytes, bar_full + 8 * s);
@@ -540,31 +430,19 @@ __global__ void __launch_bounds__(THREADS, 1) linear_tc_kernel(const TcArgs p) {
         }
     } else if (warp == MMA_WARP) {
         // ================= MMA issuer ==================================================================
-        if (PAIR && rank != 0) {
-            // peer of a pair: no MMAs to issue; tell the leader whenever a stage of THIS CTA is full
-            if (lane == 0) {
-                const uint32_t total_it = (uint32_t)my_units * (uint32_t)kblocks;
-                for (uint32_t it = 0; it < total_it; it++) {
-                    const int s = it % NST;
-                    mbar_wait(bar_full + 8 * s, (it / NST) & 1);
-                    mbar_arrive_remote(bar_pfull + 8 * s, 0);
-                }
-            }
-        } else if (lane == 0) {
+        if (lane == 0) {
             uint32_t it = 0;
             for (uint32_t tcount = 0; tcount < (uint32_t)my_units; tcount++) {
                 const int as = tcount % ACC_STAGES;
                 const uint32_t aph = (tcount / ACC_STAGES) & 1;
-                if (PAIR) mbar_wait_cluster(bar_tempty + 8 * as, aph ^ 1);  // both CTAs' epilogues drained this accumulator
-                else mbar_wait(bar_tempty + 8 * as, aph ^ 1);               // epilogue drained this accumulator
+                mbar_wait(bar_tempty + 8 * as, aph ^ 1);  // epilogue drained this accumulator
                 tc_fence_after();
                 GM_TRACE(p.trace, tcount, 0);
                 const uint32_t d0 = tmem_base + as * ACC_COLS;
                 for (int kb = 0; kb < kblocks; kb++, it++) {
-                    const int s = it % NST;
-                    const uint32_t ph = (it / NST) & 1;
+                    const int s = it % STAGES;
+                    const uint32_t ph = (it / STAGES) & 1;
                     mbar_wait(bar_full + 8 * s, ph);
-                    if (PAIR) mbar_wait_cluster(bar_pfull + 8 * s, ph);  // ... and the peer's half of the operands
                     tc_fence_after();
                     if (kb == 0) GM_TRACE(p.trace, tcount, 1);
                     const uint32_t a_hi = smem_base + s * STAGE_BYTES, a_lo = a_hi + A_PART_BYTES;
@@ -578,15 +456,7 @@ __global__ void __launch_bounds__(THREADS, 1) linear_tc_kernel(const TcArgs p) {
                         if ((LN && (p.accumulate & 2)) || (p.a_stages & 2)) break;  // timing probes: no MMAs
 #endif
                         const uint32_t o = ks * 256;  // two 128-byte core matrices per K=16 step
-                        if (PAIR) {
-                            if (PASSES == 3) {
-                                umma2(d, umma_desc(a_lo + o), umma_desc(w_hi + o), IDESC, (kfirst | ks) != 0);
-                                umma2(d, umma_desc(a_hi + o), umma_desc(w_lo + o), IDESC, 1);
-                                umma2(d, umma_desc(a_hi + o), umma_desc(w_hi + o), IDESC, 1);
-                            } else {
-                                umma2(d, umma_desc(a_hi + o), umma_desc(w_hi + o), IDESC, (kfirst | ks) != 0);
-                            }
-                        } else if (PASSES == 3) {  // small terms first, then hi*hi
+                        if (PASSES == 3) {  // small terms first, then hi*hi
                             umma(d, umma_desc(a_lo + o), umma_desc(w_hi + o), IDESC, (kfirst | ks) != 0);
                             umma(d, umma_desc(a_hi + o), umma_desc(w_lo + o), IDESC, 1);
                             umma(d, umma_desc(a_hi + o), umma_desc(w_hi + o), IDESC, 1);
@@ -594,15 +464,10 @@ __global__ void __launch_bounds__(THREADS, 1) linear_tc_kernel(const TcArgs p) {
                             umma(d, umma_desc(a_hi + o), umma_desc(w_hi + o), IDESC, (kfirst | ks) != 0);
                         }
                     }
-                    // smem stage reusable once these MMAs retire; with multicast weights every CTA of the
-                    // cluster must know, because peers write into this CTA's stage; in a pair both CTAs' stages retire
-                    if (PAIR) umma2_commit_mc(bar_empty + 8 * s, 3);
-                    else if (csz == 1) umma_commit(bar_empty + 8 * s);
-                    else umma_commit_mc(bar_empty + 8 * s, mc_mask);
+                    umma_commit(bar_empty + 8 * s);  // smem stage reusable once these MMAs retire
                 }
                 GM_TRACE(p.trace, tcount, 2);
-                if (PAIR) umma2_commit_mc(bar_tfull + 8 * as, 3);  // accumulator complete in both CTAs
-                else umma_commit(bar_tfull + 8 * as);              // accumulator complete
+                umma_commit(bar_tfull + 8 * as);  // accumulator complete
             }
         }
     } else {
@@ -636,27 +501,14 @@ __global__ void __launch_bounds__(THREADS, 1) linear_tc_kernel(const TcArgs p) {
                     mbar_wait(bar_tfull + 8 * as, aph);
                     tc_fence_after();
                     tc_fence_before();
-                    if (PAIR) {
-                        __syncwarp();
-                        if (lane == 0) { if (rank != 0) mbar_arrive_remote(bar_tempty + 8 * as, 0); else mbar_arrive(bar_tempty + 8 * as); }
-                    } else {
-                        mbar_arrive(bar_tempty + 8 * as);
-                    }
+                    mbar_arrive(bar_tempty + 8 * as);
                     continue;
                 }
 #endif
 #include "gemm_sm100_epilogue.inc"
                 if (threadIdx.x == 0) GM_TRACE(p.trace, tcount, 4);
                 tc_fence_before();
-                if (PAIR) {  // the leader's MMA thread waits for the epilogue warps of both CTAs: one arrive per warp
-                    __syncwarp();
-                    if (lane == 0) {
-                        if (rank != 0) mbar_arrive_remote(bar_tempty + 8 * as, 0);
-                        else mbar_arrive(bar_tempty + 8 * as);
-                    }
-                } else {
-                    mbar_arrive(bar_tempty + 8 * as);
-                }
+                mbar_arrive(bar_tempty + 8 * as);
             }
         }
         (void)ln_csum; (void)ln_craw; (void)ln_ma; (void)ln_ra; (void)ln_mb; (void)ln_rb; (void)ln_prm_s; (void)ln_cin_s;
@@ -664,12 +516,10 @@ __global__ void __launch_bounds__(THREADS, 1) linear_tc_kernel(const TcArgs p) {
 
     tc_fence_before();
     __syncthreads();
-    if (p.csz > 1) cluster_sync_all();  // no CTA leaves while peers may still signal its barriers
     if (warp == MMA_WARP) {
         tc_fence_after();
         uint32_t cols = ACC_STAGES * ACC_COLS;
-        if (PAIR) asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(cols) : "memory");
-        else asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(cols) : "memory");
+        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(cols) : "memory");
     }
 }
 
@@ -815,11 +665,9 @@ int tc_pick_bn(int N, int epi) {
 
 static int64_t lnlstm_param_floats(int H) { return 2 * H + (H / 32) * 3 * 128 + 2 * H; }
 
-TcShape tc_shape(int N, int K0, int K1, int epi, int H, int ws) {
+TcShape tc_shape(int N, int K0, int K1, int epi, int H) {
     TcShape s;
     s.BN = tc_pick_bn(N, epi);
-    TcWsPlan plan;
-    if (ws && tc_ws_plan(N, K0, K1, epi, H, &plan)) s.BN = plan.BN;
     s.K0p = (int)round_up(K0, tc::BK);  // segment 1 starts on a k-block boundary
     s.Kp = s.K0p + (int)round_up(K1, tc::BK);
     s.n_tiles = (epi == EPI_LSTM) ? ceil_div(H, s.BN / 4) : (epi == EPI_LNLSTM) ? 1 + H / 32 : ceil_div(N, s.BN);
@@ -836,7 +684,7 @@ int tc_pack_lnlstm(const float* w_ih, const float* w_hh, const float* b_ih, cons
     GM_CHECK_ARG(H == 128, "fused LayerNormLSTM cell is built for hidden == 128, got %d", H);
     GM_CHECK_ARG(w_ih && w_hh && b_ih && ln_in_w && ln_in_b && ln_hid_w && ln_hid_b && ln_cell_w && ln_cell_b,
                  "LayerNormLSTM cell parameters missing");
-    TcShape sh = tc_shape(4 * H, H, H, EPI_LNLSTM, H, 0);
+    TcShape sh = tc_shape(4 * H, H, H, EPI_LNLSTM, H);
     float* params = (float*)((char*)out + sh.w_bytes);
     float* wx = (float*)((char*)params + round_up(lnlstm_param_floats(H) * 4, 256));
     tc::lnlstm_stage_kernel<<<148 * 4, 256, 0, s>>>(w_ih, w_hh, H, wx);
@@ -853,8 +701,8 @@ int tc_pack_lnlstm(const float* w_ih, const float* w_hh, const float* b_ih, cons
 }
 
 int tc_pack_weights(const float* W, int64_t ldw, const float* W1, int64_t ldw1, const float* bias, const float* bias2, int N,
-                    int K0, int K1, int epi, int H, void* out, cudaStream_t s, int ws) {
-    TcShape sh = tc_shape(N, K0, K1, epi, H, ws);
+                    int K0, int K1, int epi, int H, void* out, cudaStream_t s) {
+    TcShape sh = tc_shape(N, K0, K1, epi, H);
     int64_t total = (int64_t)sh.n_tiles * (sh.Kp / tc::BK) * sh.BN * (tc::BK / 8);
     int blocks = (int)std::min<int64_t>((total + 255) / 256, 148 * 8);
     tc::pack_w_kernel<<<blocks, 256, 0, s>>>(W, ldw, W1, ldw1, N, K0, K1, sh.K0p, sh.Kp, sh.BN, sh.n_tiles, epi == EPI_LSTM,
@@ -866,56 +714,16 @@ int tc_pack_weights(const float* W, int64_t ldw, const float* W1, int64_t ldw1, 
     return GM_OK;
 }
 
-static int tc_cluster_size() {
-    static int csz = -1;
-    if (csz < 0) {
-        const char* e = getenv("GM_TC_CLUSTER");
-        csz = e ? atoi(e) : 1;  // measured on B200: multicast of the weight stages (2, 4) brings no gain at these shapes
-        if (csz != 1 && csz != 2 && csz != 4 && csz != 8) csz = 1;
-    }
-    return csz;
-}
-
-template <int BN, int PASSES, int EPI, int NCG = 2, bool PAIR = false>
+template <int BN, int PASSES, int EPI, int NCG = 2>
 static int launch_tc(TcArgs a, cudaStream_t s) {
-    constexpr int smem = PAIR ? tc::PAIR_STAGES * (2 * tc::A_PART_BYTES + 2 * (BN / 2) * tc::BK * 2)
-                              : tc::STAGES * (2 * tc::A_PART_BYTES + 2 * BN * tc::BK * 2) +
-                                    (EPI == EPI_LNLSTM ? BN * tc::BM * 4 : 0);  // + pre-LN cell values of one M tile
+    constexpr int smem = tc::STAGES * (2 * tc::A_PART_BYTES + 2 * BN * tc::BK * 2) +
+                         (EPI == EPI_LNLSTM ? BN * tc::BM * 4 : 0);  // + pre-LN cell values of one M tile
     static bool configured = false;
-    static int max_clusters[9] = {0, 0, 0, 0, 0, 0, 0, 0, 0};
-    auto kern = tc::linear_tc_kernel<BN, PASSES, EPI, NCG, PAIR>;
+    auto kern = tc::linear_tc_kernel<BN, PASSES, EPI, NCG>;
     if (!configured) {
         GM_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
         configured = true;
     }
-    // weight stages are multicast to the CTAs of a cluster (each CTA fetches 1/csz of every weight tile);
-    // PAIR: always a 2-CTA cluster driving one cta_group::2 MMA
-    int csz = PAIR ? 2 : std::min(tc_cluster_size(), std::max(1, a.m_tiles));
-    while (!PAIR && csz > 1 && csz > a.m_tiles) csz >>= 1;
-    if (csz == 3) csz = 2;
-    if (csz > 4 && csz < 8) csz = 4;
-    cudaLaunchConfig_t cfg{};
-    cudaLaunchAttribute attr[2];
-    cfg.blockDim = dim3(tc::THREADS);
-    cfg.dynamicSmemBytes = smem;
-    cfg.stream = s;
-    attr[0].id = cudaLaunchAttributeClusterDimension;
-    attr[0].val.clusterDim.x = csz; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
-    attr[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;  // see pdl_trigger / pdl_wait in common.cuh
-    attr[1].val.programmaticStreamSerializationAllowed = pdl_enabled() ? 1 : 0;
-    cfg.attrs = attr; cfg.numAttrs = 2;
-    if (csz > 1 && max_clusters[csz] == 0) {
-        cfg.gridDim = dim3((kNumSMs / csz) * csz);
-        int n = 0;
-        cudaError_t e = cudaOccupancyMaxActiveClusters(&n, kern, &cfg);
-        if (e != cudaSuccess || n <= 0) { cudaGetLastError(); n = -1; }
-        max_clusters[csz] = n;
-    }
-    if (PAIR && max_clusters[csz] < 0) return 1;    // caller falls back to the single-CTA kernel
-    if (csz > 1 && max_clusters[csz] < 0) csz = 1;  // clusters of this size cannot be scheduled: plain launch
-    attr[0].val.clusterDim.x = csz;
-    a.csz = csz;
-    if (EPI == EPI_LNLSTM) csz = 1;
 #if GM_TC_PROBES
     {
         static int dbg = -1;
@@ -930,40 +738,20 @@ static int launch_tc(TcArgs a, cudaStream_t s) {
         a.trace = (EPI == trace_epi && (trace_kp <= 0 || a.Kp == trace_kp)) ? (void*)trace_ptr : nullptr;
     }
 #endif
-    attr[0].val.clusterDim.x = csz;
-    a.csz = csz;
     // LayerNormLSTM: a CTA owns whole M tiles
-    const int units = EPI == EPI_LNLSTM ? a.m_tiles : ((a.m_tiles + csz - 1) / csz) * a.n_tiles;
-    const int n_clusters = std::min(units, csz > 1 ? max_clusters[csz] : kNumSMs);
-    cfg.gridDim = dim3(n_clusters * csz);
+    const int units = EPI == EPI_LNLSTM ? a.m_tiles : a.m_tiles * a.n_tiles;
     ProfileScope prof(PROF_TC, s);
-    GM_CUDA(cudaLaunchKernelEx(&cfg, kern, a));
-    count_launch();
+    kern<<<std::min(units, kNumSMs), tc::THREADS, smem, s>>>(a);
+    GM_LAUNCH_CHECK();
     return GM_OK;
 }
-
-
-// A weight-stationary cluster kernel (one N slice of the weights resident per CTA, activation k-blocks multicast over the
-// cluster) was built and measured in round 1: slower than the streaming kernel at these shapes (multicast replicates
-// the bytes in flight; DESIGN.md section 5) and removed in round 2.  The plan query stays so that callers' packing code
-// keeps one code path.
-bool tc_ws_plan(int, int, int, int, int, TcWsPlan*) { return false; }
 
 // ---- fused encoder layers 1 + 2 for sparse input rows (gemm_sm100_encfused.inc) -----------------------------------
 bool enc_fused_ok(int D, int U1, int U2, int math) {
     return math == GM_MATH_BF16X3 && D >= 1 && (U1 % tc::BK) == 0 && U1 >= tc::BK && U2 >= 32 && U2 <= tc::EF_BN && (U2 % tc::BK) == 0 &&
            tc::ef_plan(D).nw >= 3;
 }
-// GM_ENC_FUSED: 0 never, 1 (default) rows of at most 6 terms supplied by the caller, 2 also 12-term rows.  Measured at
-// configs 2 / 3: the 6-term kernel beats the two separate layers (80 vs 123 us), the 12-term kernel does not (its W1^T
-// chunk allows a 3-slot ring only and the producers issue 50 shared-memory loads per k-block: 0.382 vs 0.361 ms per step
-// at 2048 envs), so it is an option.  Read on every call: the weight pack does not depend on it.
-int enc_fused_mode() {
-    const char* e = getenv("GM_ENC_FUSED");
-    return e ? atoi(e) : 1;
-}
 int64_t enc_fused_w1t_bytes(int U1, int D) { return (int64_t)(U1 / tc::BK) * tc::ef_chunk_bytes(D); }
-int64_t enc_fused_sp_bytes(int64_t R) { return ((R + tc::BM - 1) / tc::BM) * tc::EF_SP_BYTES; }
 
 // D = input width, S static rows (dense [S, D], may be 0 / NULL): the chunks hold D + S rows, or (static_only) the S rows alone
 int enc_fused_pack_w1t(const float* W1, const float* b1, int U1, int D, const float* static_rows, int S, int static_only, void* out,
@@ -973,30 +761,21 @@ int enc_fused_pack_w1t(const float* W1, const float* b1, int U1, int D, const fl
     return GM_OK;
 }
 
-// x fp32 [R, D] (row stride ldx) -> sparse rows in sp_ws -> Cpk = act(W2 act(W1 x + b1) + b2) tile-packed [R, U2]
-// (or, with sp_rows != NULL, takes the caller's sparse rows [ceil(R/128)*128][24] as they are: 12 column indices then 12 values)
-// D: rows of the W1^T chunks (input width + static rows); nnz: 12, or 6 when the rows name a static part
-int enc_fused_launch(const float* x, int64_t ldx, int64_t R, int Dx, int D, int nnz, const void* w1t, const void* W2p, int U1, int U2, int act,
-                     void* sp_ws, const int32_t* sp_rows, uint8_t* Cpk, int* overflow, cudaStream_t s) {
-    GM_CHECK_ARG(nnz == 12 || (nnz == 6 && sp_rows != nullptr), "6-term rows must be supplied by the caller");
-    GM_CHECK_ARG((x || sp_rows) && w1t && W2p && sp_ws && Cpk && R > 0, "bad fused-encoder arguments");
+// the caller's sparse rows [ceil(R/128)*128][24] (12 column indices then 12 values, of which the first 6 are read)
+// -> Cpk = act(W2 act(W1 x + b1) + b2) tile-packed [R, U2].  D: rows of the W1^T chunks (input width + static rows)
+int enc_fused_launch(const int32_t* sp_rows, int64_t R, int D, const void* w1t, const void* W2p, int U1, int U2, int act, uint8_t* Cpk,
+                     cudaStream_t s) {
+    GM_CHECK_ARG(sp_rows && w1t && W2p && Cpk && R > 0, "bad fused-encoder arguments");
     GM_CHECK_ARG(act == GM_ACT_LEAKY_RELU, "the fused encoder kernel is built for leaky_relu only");
-    GM_CHECK_ARG((((uintptr_t)w1t | (uintptr_t)W2p | (uintptr_t)sp_ws | (uintptr_t)sp_rows) & 15) == 0 && ((uintptr_t)Cpk & 127) == 0,
+    GM_CHECK_ARG((((uintptr_t)w1t | (uintptr_t)W2p | (uintptr_t)sp_rows) & 15) == 0 && ((uintptr_t)Cpk & 127) == 0,
                  "fused-encoder buffers must be 16 / 128-byte aligned");
     const int m_tiles = (int)((R + tc::BM - 1) / tc::BM);
-    const int64_t Rpad = (int64_t)m_tiles * tc::BM;
-    if (sp_rows == nullptr) {
-        tc::ef_sparsify_kernel<<<(unsigned)((Rpad + 7) / 8), 256, 0, s>>>(x, ldx, R, Rpad, Dx, (int32_t*)sp_ws, overflow);
-        GM_LAUNCH_CHECK();
-        sp_rows = (const int32_t*)sp_ws;
-    }
     const tc::EfPlan plan = tc::ef_plan(D);
     GM_CHECK_ARG(plan.nw >= 3, "fused-encoder chunk of %d rows does not fit in shared memory", D);
     const int smem = plan.smem;
     static int configured = 0;
     if (configured < smem) {
-        GM_CUDA(cudaFuncSetAttribute(tc::enc_fused_kernel<12>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-        GM_CUDA(cudaFuncSetAttribute(tc::enc_fused_kernel<6>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+        GM_CUDA(cudaFuncSetAttribute(tc::enc_fused_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
         configured = smem;
     }
     const TcShape sh = tc_shape(U2, U1, 0, EPI_LINEAR, 0);
@@ -1017,15 +796,14 @@ int enc_fused_launch(const float* x, int64_t ldx, int64_t R, int Dx, int D, int 
 #endif
     const int grid = std::min(m_tiles, kNumSMs);
     ProfileScope prof(PROF_TC, s);
-    if (nnz == 6) GM_CUDA(launch_pdl(tc::enc_fused_kernel<6>, dim3(grid), dim3(tc::THREADS), (size_t)smem, s, a));
-    else GM_CUDA(launch_pdl(tc::enc_fused_kernel<12>, dim3(grid), dim3(tc::THREADS), (size_t)smem, s, a));
-    count_launch();
+    tc::enc_fused_kernel<<<grid, tc::THREADS, smem, s>>>(a);
+    GM_LAUNCH_CHECK();
     return GM_OK;
 }
 
 int tc_launch(TcArgs a, int math, int epi, cudaStream_t s) {
     if (a.M <= 0) return GM_OK;
-    TcShape sh = tc_shape(a.N, a.K0, a.K1, epi, a.H, a.ws);
+    TcShape sh = tc_shape(a.N, a.K0, a.K1, epi, a.H);
     a.K0p = sh.K0p;
     a.Kp = sh.Kp;
     a.n_tiles = sh.n_tiles;
@@ -1040,7 +818,7 @@ int tc_launch(TcArgs a, int math, int epi, cudaStream_t s) {
                  "tile-packed segment 1: K %% 32 and 128-byte alignment");
     a.has_prod = (a.A0 != nullptr) || (a.K1 > 0 && a.A1 != nullptr);
     if (epi == EPI_LNLSTM) {
-        GM_CHECK_ARG(a.H == 128 && a.K0 == 128 && a.K1 == 128 && !a.ws, "fused LayerNormLSTM cell needs hidden == 128 and two 128-wide segments");
+        GM_CHECK_ARG(a.H == 128 && a.K0 == 128 && a.K1 == 128, "fused LayerNormLSTM cell needs hidden == 128 and two 128-wide segments");
         GM_CHECK_ARG(a.A0pk && a.A1pk, "fused LayerNormLSTM cell takes tile-packed operands only (its producer warps run the epilogue)");
         GM_CHECK_ARG(a.c_in && a.h_out && a.c_out && (a.ldc_in & 7) == 0 && (a.ldh & 7) == 0 && (a.ldco & 7) == 0 &&
                          (((uintptr_t)a.c_in | (uintptr_t)a.h_out | (uintptr_t)a.c_out) & 31) == 0 && ((uintptr_t)a.Hpk & 127) == 0,
@@ -1053,7 +831,7 @@ int tc_launch(TcArgs a, int math, int epi, cudaStream_t s) {
             a.accumulate = dbg;
         }
 #endif
-        return launch_tc<128, 3, EPI_LNLSTM, 4, false>(a, s);  // always the three-pass product (SURVEY 7.4: LN amplifies rounding)
+        return launch_tc<128, 3, EPI_LNLSTM, 4>(a, s);  // always the three-pass product (SURVEY 7.4: LN amplifies rounding)
     }
     if (epi == EPI_LSTM) {
         GM_CHECK_ARG(a.H % 64 == 0, "fused LSTM epilogue needs hidden %% 64 == 0, got %d", a.H);
@@ -1071,24 +849,9 @@ int tc_launch(TcArgs a, int math, int epi, cudaStream_t s) {
         GM_CHECK_ARG(!a.accumulate || a.C != nullptr, "accumulate needs an fp32 output");
     }
     const int passes = math == GM_MATH_BF16 ? 1 : 3;
-    GM_CHECK_ARG(!a.ws, "the weight-stationary kernel was removed");
-    // 2-CTA pairs (cta_group::2, M = 256): half the weight bytes and shared-memory operand reads per CTA.  Measured on
-    // B200 at this workload's shapes: correct but 5-15 % slower than the single-CTA kernel (the relay of "peer stage
-    // full" and the two-CTA accumulator release lengthen the per-stage loop), so it is an option: GM_TC_PAIR=1
-    static int pair = -1;
-    if (pair < 0) { const char* e = getenv("GM_TC_PAIR"); pair = e ? atoi(e) : 0; }
-    if (pair && passes == 3 && sh.BN == 256 && a.m_tiles >= 2) {
-        int rc = 1;
-        if (epi == EPI_LSTM) rc = launch_tc<256, 3, EPI_LSTM, 2, true>(a, s);
-        else if (epi == EPI_QHEAD) rc = launch_tc<256, 3, EPI_QHEAD, 2, true>(a, s);
-        else if (epi == EPI_LINEAR) rc = launch_tc<256, 3, EPI_LINEAR, 2, true>(a, s);
-        if (rc != 1) return rc;  // 1: 2-CTA clusters cannot be scheduled here
-    }
     // all operands tile-packed: the producer warps have nothing to do and run the epilogue too (4 epilogue warps per
-    // scheduler overlap MUFU and FP32 work better: GEMM time per step 0.69 -> 0.67 ms; GM_TC_WIDE=0: off)
-    static int wide = -1;
-    if (wide < 0) { const char* e = getenv("GM_TC_WIDE"); wide = e ? atoi(e) : 1; }
-    if (wide && !a.has_prod && passes == 3) {
+    // scheduler overlap MUFU and FP32 work better: GEMM time per step 0.69 -> 0.67 ms)
+    if (!a.has_prod && passes == 3) {
         if (epi == EPI_LSTM) return launch_tc<256, 3, EPI_LSTM, 4>(a, s);
         if (epi == EPI_QHEAD) return launch_tc<256, 3, EPI_QHEAD, 4>(a, s);  // Q head: 4 column groups of 64, partials summed through smem
         if (epi == EPI_LINEAR) return sh.BN == 128 ? launch_tc<128, 3, EPI_LINEAR, 4>(a, s) : launch_tc<256, 3, EPI_LINEAR, 4>(a, s);

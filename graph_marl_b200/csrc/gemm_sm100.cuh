@@ -54,8 +54,7 @@ struct TcArgs {
     uint64_t philox_seed, philox_step; const uint64_t* philox_step_dev;
     float* q_out; int* act_out;
     void* trace;  // GM_TC_PROBES builds only: per-tile timeline buffer (see gemm_sm100.cu)
-    int ws;  // use the weight-stationary cluster kernel (tc_ws_plan must hold; weights packed with ws = 1)
-    int m_tiles, n_tiles, has_prod, csz, a_stages;  // filled by tc_launch
+    int m_tiles, n_tiles, has_prod, a_stages;  // filled by tc_launch
 };
 
 __host__ __device__ inline int64_t tc_blocked_off(int64_t row, int unit, int H) {
@@ -68,31 +67,23 @@ struct TcShape {
     int64_t w_bytes, packed_bytes;  // weight tiles; weights + bias, rounded to 256
 };
 
-struct TcWsPlan {
-    int BN, csz, a_stages, smem;
-};
-// weight-stationary cluster plan for a layer whose activations are all tile-packed (false: not eligible)
-bool tc_ws_plan(int N, int K0, int K1, int epi, int H, TcWsPlan* out);
-
-TcShape tc_shape(int N, int K0, int K1, int epi, int H, int ws = 0);
+TcShape tc_shape(int N, int K0, int K1, int epi, int H);
 // W fp32 [N, K0+K1] (row stride ldw), or W [N,K0] next to W1 [N,K1] -> packed bf16 hi/lo tiles
 // (tc_shape(...).packed_bytes, 256-byte aligned destination)
 // bias (+ bias2) are summed and stored tile-ordered behind the weights (either may be NULL)
 int tc_pack_weights(const float* W, int64_t ldw, const float* W1, int64_t ldw1, const float* bias, const float* bias2, int N,
-                    int K0, int K1, int epi, int H, void* out, cudaStream_t s, int ws = 0);
+                    int K0, int K1, int epi, int H, void* out, cudaStream_t s);
 int tc_launch(TcArgs a, int math, int epi, cudaStream_t s);
 
-// Encoder layers 1 + 2 as one kernel for input rows with at most 12 non-zeros (gemm_sm100_encfused.inc): layer 1 on the
-// CUDA cores inside the producer warps, layer 2 on tcgen05.  W2 is packed by tc_pack_weights(N = U2, K0 = U1, EPI_LINEAR)
-// and must come out as ONE 256-column tile; W1 by enc_fused_pack_w1t.
+// Encoder layers 1 + 2 as one kernel for caller-supplied sparse input rows of at most 6 terms (gemm_sm100_encfused.inc):
+// layer 1 on the CUDA cores inside the producer warps, layer 2 on tcgen05.  W2 is packed by tc_pack_weights(N = U2,
+// K0 = U1, EPI_LINEAR) and must come out as ONE 256-column tile; W1 by enc_fused_pack_w1t.
 bool enc_fused_ok(int D, int U1, int U2, int math);
-int enc_fused_mode();
 int64_t enc_fused_w1t_bytes(int U1, int D);
-int64_t enc_fused_sp_bytes(int64_t R);
 int enc_fused_pack_w1t(const float* W1, const float* b1, int U1, int D, const float* static_rows, int S, int static_only, void* out,
                        cudaStream_t s);
-int enc_fused_launch(const float* x, int64_t ldx, int64_t R, int Dx, int D, int nnz, const void* w1t, const void* W2p, int U1, int U2, int act,
-                     void* sp_ws, const int32_t* sp_rows, uint8_t* Cpk, int* overflow, cudaStream_t s);
+int enc_fused_launch(const int32_t* sp_rows, int64_t R, int D, const void* w1t, const void* W2p, int U1, int U2, int act, uint8_t* Cpk,
+                     cudaStream_t s);
 
 // LayerNormLSTM cell (H == 128) -> packed weights for EPI_LNLSTM: tc_shape(4H, H, H, EPI_LNLSTM, H).packed_bytes
 // (Gram + gate tiles, LN parameters, and the staging area the packing kernels use), 256-byte aligned destination.

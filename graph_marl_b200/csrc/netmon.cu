@@ -12,9 +12,9 @@
 // Aggregation on the tensor-core path (tile-packed output, see the launch site):
 //   aggregate_pk_pipe_kernel  default: persistent CTAs, TMA bulk copies of whole graphs' hidden rows / lists into a
 //                             3-stage shared-memory ring (producer warp + mbarriers), sums from shared memory
-//   aggregate_pk_kernel       L2 gather, 8 rows x 32 columns per warp; the fallback for graphs that do not fit the ring
-//                             (GM_AGG_MAP=8 forces it).  Two more forms measured in round 1 (a 4-row-per-line gather and a
-//                             single-stage bulk-staged kernel, both slower, DESIGN.md section 5) were removed in round 2.
+//   aggregate_pk_kernel       L2 gather, 8 rows x 32 columns per warp; the fallback for graphs that do not fit the ring.
+//                             Two more forms measured in round 1 (a 4-row-per-line gather and a single-stage bulk-staged
+//                             kernel, both slower, DESIGN.md section 5) were removed in round 2.
 #include <cuda_bf16.h>
 
 #include "common.cuh"
@@ -100,40 +100,36 @@ __device__ __forceinline__ uint32_t agg_pack2(float a, float b) {
 // A block owns `rows_per_block` consecutive rows (whole graphs when the host can arrange it, a multiple of 8) and its
 // warps walk the (8-row group, k-block) tasks of those rows: every 128-byte line of h that the block gathers is
 // fetched from L2 once and re-read by the other list members (a row is in ~4 lists) from L1.
-// STAGED: the block first copies the neighbour lists and degrees of its rows into shared memory (one coalesced pass),
-// so a task's dependent chain is "hidden rows -> store" instead of "list_index -> list/degree -> hidden rows -> store";
+// The block first copies the neighbour lists and degrees of its rows into shared memory (one coalesced pass), so a
+// task's dependent chain is "hidden rows -> store" instead of "list_index -> list/degree -> hidden rows -> store";
 // with ~2.5 task rounds per warp the kernel is bound by that chain, not by bytes (ncu: DRAM 20 %, L2 18 %).
-template <bool STAGED>
-__global__ void __launch_bounds__(STAGED ? 320 : 256) aggregate_pk_kernel(const float* __restrict__ h, int64_t ldh, uint8_t* __restrict__ Mpk,
-                                                           int B, int N, int H, const int* __restrict__ nbr,
-                                                           const int* __restrict__ deg, int DM,
-                                                           const int* __restrict__ list_index, int mean, int write_lo,
-                                                           int rows_per_block) {
-    pdl_trigger();
-    pdl_wait();
-    extern __shared__ int agg_lists[];  // STAGED: lists i32[rows_per_block][DM] | degrees i32[rows_per_block]
+constexpr int AGG_THREADS = 256;
+__global__ void __launch_bounds__(AGG_THREADS) aggregate_pk_kernel(const float* __restrict__ h, int64_t ldh, uint8_t* __restrict__ Mpk,
+                                                                   int B, int N, int H, const int* __restrict__ nbr,
+                                                                   const int* __restrict__ deg, int DM,
+                                                                   const int* __restrict__ list_index, int mean, int write_lo,
+                                                                   int rows_per_block) {
+    extern __shared__ int agg_lists[];  // lists i32[rows_per_block][DM] | degrees i32[rows_per_block]
     const int lane = threadIdx.x & 31;
     const int kbs = H / TC_BK;
     const int64_t R = (int64_t)B * N;
     const int64_t row0 = (int64_t)blockIdx.x * rows_per_block;
     const int tasks = (rows_per_block >> 3) * kbs;
-    if (STAGED) {
-        int* s_deg = agg_lists + rows_per_block * DM;
-        for (int t = threadIdx.x; t < rows_per_block * DM; t += (int)blockDim.x) {
-            const int r = t / DM, q = t - r * DM;
-            const int64_t row = row0 + r;
-            int val = 0;
-            if (row < R) {
-                const unsigned row32 = (unsigned)row;
-                const int b = (int)(row32 / (unsigned)N), v = (int)(row32 - (unsigned)b * (unsigned)N);
-                const size_t node = (size_t)(list_index ? list_index[b] : b) * N + v;
-                val = nbr[node * DM + q];
-                if (q == 0) s_deg[r] = deg[node];
-            }
-            agg_lists[t] = val;
+    int* s_deg = agg_lists + rows_per_block * DM;
+    for (int t = threadIdx.x; t < rows_per_block * DM; t += (int)blockDim.x) {
+        const int r = t / DM, q = t - r * DM;
+        const int64_t row = row0 + r;
+        int val = 0;
+        if (row < R) {
+            const unsigned row32 = (unsigned)row;
+            const int b = (int)(row32 / (unsigned)N), v = (int)(row32 - (unsigned)b * (unsigned)N);
+            const size_t node = (size_t)(list_index ? list_index[b] : b) * N + v;
+            val = nbr[node * DM + q];
+            if (q == 0) s_deg[r] = deg[node];
         }
-        __syncthreads();
+        agg_lists[t] = val;
     }
+    __syncthreads();
     for (int t = threadIdx.x >> 5; t < tasks; t += (int)(blockDim.x >> 5)) {
     const int rl = (t / kbs) * 8 + (lane >> 2);
     const int64_t row = row0 + rl;
@@ -141,17 +137,8 @@ __global__ void __launch_bounds__(STAGED ? 320 : 256) aggregate_pk_kernel(const 
     if (row >= R) continue;
     const unsigned row32 = (unsigned)row;  // the host checks B*N < 2^31
     const int b = (int)(row32 / (unsigned)N);
-    const int* lst;
-    int dg;
-    if (STAGED) {
-        lst = agg_lists + rl * DM;
-        dg = agg_lists[rows_per_block * DM + rl];
-    } else {
-        const int v = (int)(row32 - (unsigned)b * (unsigned)N);
-        const int li = list_index ? list_index[b] : b;
-        lst = nbr + ((size_t)li * N + v) * DM;
-        dg = deg[(size_t)li * N + v];
-    }
+    const int* lst = agg_lists + rl * DM;
+    const int dg = s_deg[rl];
     const float* hb = h + (size_t)b * N * ldh + kb * TC_BK + part * 8;
     float x[8];
 #pragma unroll
@@ -206,6 +193,7 @@ __device__ __forceinline__ uint32_t agg_smem_u32(const void* p) { return (uint32
 // "full", form the sums from shared memory, store the packed tile rows, release the stage on its "empty" mbarrier.  No
 // consumer warp ever waits on global memory, so loads of block i+1, i+2 overlap the arithmetic and stores of block i.
 constexpr int AGG_STAGES = 3;
+constexpr int AGG_PIPE_THREADS = 32 * 11, AGG_PIPE_CTAS = 3;  // 1 producer + 10 consumer warps, 3 CTAs per SM
 
 __device__ __forceinline__ void agg_mbar_wait(uint32_t bar, uint32_t parity) {
     uint32_t done = 0, spins = 0;
@@ -221,13 +209,11 @@ __device__ __forceinline__ void agg_mbar_wait(uint32_t bar, uint32_t parity) {
 // HC / DMC: compile-time hidden size / list width (0 = use the runtime arguments); the <128, 4> instance turns the row, tile and
 // task index arithmetic of the consumer loop into shifts.
 template <int HC, int DMC>
-__global__ void __launch_bounds__(352, 3) aggregate_pk_pipe_kernel(const float* __restrict__ h, int64_t ldh, uint8_t* __restrict__ Mpk,
+__global__ void __launch_bounds__(AGG_PIPE_THREADS, AGG_PIPE_CTAS) aggregate_pk_pipe_kernel(const float* __restrict__ h, int64_t ldh, uint8_t* __restrict__ Mpk,
                                                                    int B, int N, int H_rt, const int* __restrict__ nbr,
                                                                    const int* __restrict__ deg, int DM_rt,
                                                                    const int* __restrict__ list_index, int mean, int write_lo,
                                                                    int rows_per_block, int n_blocks, int stage_bytes) {
-    pdl_trigger();
-    pdl_wait();
     const int H = HC ? HC : H_rt, DM = DMC ? DMC : DM_rt;
     extern __shared__ __align__(128) uint8_t agg_sm[];  // full[3], empty[3] mbarriers | 3 x (rows f32[rpb][H] | lists | degrees)
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -382,11 +368,8 @@ __global__ void __launch_bounds__(352, 3) aggregate_pk_pipe_kernel(const float* 
     }
 }
 
-// rows a block of aggregate_pk_kernel owns: whole graphs, a multiple of 8 rows, about 40-80 rows (GM_AGG_ROWS overrides)
+// rows a block of the aggregation kernels owns: whole graphs, a multiple of 8 rows, about 40-80 rows
 static int aggregate_rows_per_block(int N) {
-    static int forced = -1;
-    if (forced < 0) { const char* e = getenv("GM_AGG_ROWS"); forced = e ? atoi(e) : 0; }
-    if (forced > 0) return (forced + 7) / 8 * 8;
     int g = N;  // smallest whole-graph row count divisible by 8: N * 8 / gcd(N, 8)
     for (int d = 8; d > 1; d >>= 1) if (N % d == 0) { g = N * (8 / d); break; }
     if (N % 2 != 0) g = N * 8;
@@ -395,8 +378,8 @@ static int aggregate_rows_per_block(int N) {
     return rows;
 }
 
-// fp32 rows [R, H] (row stride ld) -> tile-packed bf16 hi/lo (the carried hidden state for the
-// weight-stationary rnn_obs cell).  Same thread mapping as aggregate_pk_kernel.
+// fp32 rows [R, H] (row stride ld) -> tile-packed bf16 hi/lo (the carried hidden state for the LayerNormLSTM
+// rnn_obs cell, which takes tile-packed operands only).  Same thread mapping as aggregate_pk_kernel.
 __global__ void __launch_bounds__(256) split_pk_kernel(const float* __restrict__ src, int64_t ld, uint8_t* __restrict__ dst_pk,
                                                        int64_t R, int H, int write_lo) {
     const int lane = threadIdx.x & 31;
@@ -595,8 +578,6 @@ __global__ void __launch_bounds__(256) readout_agents_pk_kernel(
     const int* __restrict__ nbr, const int* __restrict__ deg, int DM, const int* __restrict__ list_index,
     const int* __restrict__ agent_node, int A, int B, int N, int H, int use_nbr, int use_glob, int max_degree,
     float* __restrict__ out, int64_t ldo, uint8_t* __restrict__ out_pk, int write_lo) {
-    pdl_trigger();
-    pdl_wait();
     const int lane = threadIdx.x & 31;
     const int n_seg = 1 + (use_glob ? 1 : 0) + (use_nbr ? max_degree : 0);
     const int kb_per_seg = H / TC_BK, kbs = n_seg * kb_per_seg;
@@ -679,8 +660,6 @@ struct NetmonPack {
     int64_t obs, upd, total;
     bool fused_cells;
     int cell_epi;  // EPI_LSTM, or EPI_LNLSTM (LayerNormLSTM with hidden 128)
-    bool ws_enc[GM_MAX_LAYERS];  // layer runs on the weight-stationary cluster kernel (tile-packed input)
-    bool ws_cells;
     bool enc_fused;   // encoder layers 1 + 2 can run as one kernel for sparse input rows (gemm_sm100_encfused.inc)
     int64_t w1t;      // offset of layer 1's W^T chunks for that kernel
 };
@@ -698,19 +677,14 @@ static NetmonPack pack_layout(const gm_netmon_params* p) {
     const int H = p->hidden;
     L.cell_epi = p->rnn_type == GM_RNN_LNLSTM ? EPI_LNLSTM : EPI_LSTM;
     L.fused_cells = p->rnn_carryover && ((p->rnn_type == GM_RNN_LSTM && (H % 64) == 0) || (p->rnn_type == GM_RNN_LNLSTM && H == 128));
-    TcWsPlan plan;
     for (int l = 0; l < p->n_enc_layers; l++) {
         L.enc[l] = off;
-        // layers behind the first one read the previous layer's tile-packed output (fused path only)
-        L.ws_enc[l] = L.fused_cells && l >= 1 && (kin % TC_BK) == 0 && tc_ws_plan(p->enc_units[l], kin, 0, EPI_LINEAR, 0, &plan);
-        off += tc_shape(p->enc_units[l], kin, 0, EPI_LINEAR, 0, L.ws_enc[l]).packed_bytes;
+        off += tc_shape(p->enc_units[l], kin, 0, EPI_LINEAR, 0).packed_bytes;
         kin = p->enc_units[l];
     }
     L.obs = L.upd = off;
-    L.ws_cells = false;
     if (L.fused_cells) {
-        L.ws_cells = tc_ws_plan(4 * H, H, H, L.cell_epi, H, &plan);
-        int64_t cell = tc_shape(4 * H, H, H, L.cell_epi, H, L.ws_cells).packed_bytes;
+        int64_t cell = tc_shape(4 * H, H, H, L.cell_epi, H).packed_bytes;
         L.obs = off;
         L.upd = off + cell;
         off += 2 * cell;
@@ -731,7 +705,7 @@ static int netmon_pack(const gm_netmon_params* p, void* out, cudaStream_t s) {
     int kin = p->in_features, rc;
     for (int l = 0; l < p->n_enc_layers; l++) {
         if ((rc = tc_pack_weights(p->enc_w[l], kin, nullptr, 0, p->enc_b[l], nullptr, p->enc_units[l], kin, 0, EPI_LINEAR, 0,
-                                  (char*)out + L.enc[l], s, L.ws_enc[l])))
+                                  (char*)out + L.enc[l], s)))
             return rc;
         kin = p->enc_units[l];
     }
@@ -750,10 +724,10 @@ static int netmon_pack(const gm_netmon_params* p, void* out, cudaStream_t s) {
     } else if (L.fused_cells) {
         const int H = p->hidden;
         if ((rc = tc_pack_weights(p->rnn_obs.w_ih, H, p->rnn_obs.w_hh, H, p->rnn_obs.b_ih, p->rnn_obs.b_hh, 4 * H, H, H, EPI_LSTM, H,
-                                  (char*)out + L.obs, s, L.ws_cells)))
+                                  (char*)out + L.obs, s)))
             return rc;
         if ((rc = tc_pack_weights(p->rnn_update.w_ih, H, p->rnn_update.w_hh, H, p->rnn_update.b_ih, p->rnn_update.b_hh, 4 * H, H, H,
-                                  EPI_LSTM, H, (char*)out + L.upd, s, L.ws_cells)))
+                                  EPI_LSTM, H, (char*)out + L.upd, s)))
             return rc;
     }
     return GM_OK;
@@ -761,7 +735,6 @@ static int netmon_pack(const gm_netmon_params* p, void* out, cudaStream_t s) {
 
 struct NetmonWs {
     float *act0, *act1, *g0, *g1, *hA, *hB, *cA, *cB, *M, *gmean;
-    void* sp;  // sparse input rows of the fused encoder kernel (+ 256 bytes behind them: the overflow flag)
     float* ln_scratch;  // LayerNormLSTM cell: [SMs][128 units x 128 rows] sig(o) of the M tile a CTA works on
     uint8_t *pk0, *pk1, *e_pk, *m_pk, *h_pk0, *h_pk1;  // tile-packed activations of the tensor-core path
     int64_t bytes;
@@ -789,10 +762,8 @@ static NetmonWs carve(const gm_netmon_params* p, int64_t R, int B, void* base) {
     w.M = take(R * H);
     w.gmean = take((int64_t)max(B, 1) * H);
     w.pk0 = w.pk1 = w.e_pk = w.m_pk = w.h_pk0 = w.h_pk1 = nullptr;
-    w.sp = nullptr;
     w.ln_scratch = nullptr;
     if (tc_math(p->math)) {
-        w.sp = (void*)take((enc_fused_sp_bytes(R) + 256) / 4);
         auto take_pk = [&](int width) { return (uint8_t*)take(tc_pk_bytes(R, (int)round_up(width, TC_BK)) / 4 + 64); };
         w.pk0 = take_pk(maxw); w.pk1 = take_pk(maxw);
         w.e_pk = take_pk(H); w.m_pk = take_pk(H); w.h_pk0 = take_pk(H); w.h_pk1 = take_pk(H);
@@ -898,28 +869,16 @@ int gm_netmon_forward(const gm_netmon_params* p, int32_t B, int32_t N, const flo
     int64_t ldx = p->in_features;
     int kin = p->in_features;
     int l_first = 0;
-    // supplied rows of at most 6 entries (e.g. a static part named as one entry + the dynamic fields) run the 6-term kernel
+    // supplied rows of at most 6 entries (e.g. a static part named as one entry + the dynamic fields) run the fused kernel;
+    // with more entries per row it is slower than the two separate layers
     const bool six = p->sparse_input_nnz > 0 && p->sparse_input_nnz <= 6 && p->sparse_rows != nullptr;
     GM_CHECK_ARG(!p->static_only || p->sparse_rows != nullptr, "static_only: the rows must be supplied in sparse form");
-    const int fuse_mode = enc_fused_mode();  // 1: 6-term rows only (the 12-term kernel is slower than two layers), 2: both
-    if (fused && PL.enc_fused && p->sparse_input_nnz > 0 && p->sparse_input_nnz <= 12 && (fuse_mode >= 2 || (fuse_mode == 1 && six))) {
-        // layers 1 + 2 in one launch: layer 1 on the CUDA cores inside the producer warps (the caller declared rows of at
-        // most sparse_input_nnz non-zeros, e.g. the one-hot node observations of the Routing env), layer 2 on tcgen05
+    if (fused && PL.enc_fused && six) {
+        // layers 1 + 2 in one launch: layer 1 on the CUDA cores inside the producer warps, layer 2 on tcgen05
         uint8_t* ypk = (L == 2) ? w.e_pk : w.pk1;
-        int* overflow = (int*)((char*)w.sp + enc_fused_sp_bytes(R));
-        static int check = -1;
-        if (check < 0) { const char* e = getenv("GM_CHECK_SPARSE"); check = e ? atoi(e) : 0; }
-        if (check) GM_CUDA(cudaMemsetAsync(overflow, 0, 4, s));
-        int rc = enc_fused_launch(node_obs, p->in_features, R, p->in_features, chunk_rows(p), six ? 6 : 12, packed + PL.w1t,
-                                  packed + PL.enc[1], p->enc_units[0], p->enc_units[1], p->activation, w.sp, p->sparse_rows, ypk,
-                                  check ? overflow : nullptr, s);
+        int rc = enc_fused_launch(p->sparse_rows, R, chunk_rows(p), packed + PL.w1t, packed + PL.enc[1], p->enc_units[0],
+                                  p->enc_units[1], p->activation, ypk, s);
         if (rc) return rc;
-        if (check) {  // debug runs: the declared sparsity must hold
-            int flag = 0;
-            GM_CUDA(cudaMemcpyAsync(&flag, overflow, 4, cudaMemcpyDeviceToHost, s));
-            GM_CUDA(cudaStreamSynchronize(s));
-            GM_CHECK_ARG(flag == 0, "node observation rows have more than 12 non-zeros but sparse_input_nnz was declared");
-        }
         xpk = ypk;
         x = nullptr;
         kin = p->enc_units[1];
@@ -940,8 +899,6 @@ int gm_netmon_forward(const gm_netmon_params* p, int32_t B, int32_t N, const flo
             if (out_pk) a.Cpk = ypk; else { a.C = y; a.ldc = U; }
             a.act = p->activation;
             a.M = R; a.N = U;
-            a.ws = PL.ws_enc[l] && xpk != nullptr;
-            GM_CHECK_ARG(a.ws == (int)PL.ws_enc[l], "encoder layer %d: weights were packed for the weight-stationary kernel", l);
             rc = tc_launch(a, math, EPI_LINEAR, s);
             xpk = out_pk ? ypk : nullptr;
         } else {
@@ -981,10 +938,9 @@ int gm_netmon_forward(const gm_netmon_params* p, int32_t B, int32_t N, const flo
             a.Hpk = hn_pk;
             a.ln_scratch = w.ln_scratch;
             a.H = H; a.M = R; a.N = 4 * H;
-            a.ws = PL.ws_cells;
             return tc_launch(a, math, PL.cell_epi, s);
         };
-        // rnn_obs (:491): x = encoder output, (h, c) = carried state.  The weight-stationary kernel takes
+        // rnn_obs (:491): x = encoder output, (h, c) = carried state.  The LayerNormLSTM cell takes
         // tile-packed operands only, so the carried h is split once by a small kernel; otherwise the
         // producer warps split it on the fly.
         const int kbs = H / TC_BK;
@@ -994,7 +950,7 @@ int gm_netmon_forward(const gm_netmon_params* p, int32_t B, int32_t N, const flo
         const uint8_t* hpk_in = state_in ? (const uint8_t*)state_h_pk_in : nullptr;
         if (hpk_in && xpk) {
             rc = cell(PL.obs, xpk, e, hpk_in, nullptr, 0, st_in + H, S, hbuf[0], H, cbuf[0], -1, hpk[0]);
-        } else if (PL.ws_cells || PL.cell_epi == EPI_LNLSTM) {
+        } else if (PL.cell_epi == EPI_LNLSTM) {
             GM_CHECK_ARG(xpk != nullptr, "LayerNormLSTM cells need a tile-packed encoder output");
             const unsigned blocks = (unsigned)((((R + 7) / 8) * kbs + 7) / 8);
             split_pk_kernel<<<blocks, 256, 0, s>>>(st_in, S, hpk[1], R, H, math != GM_MATH_BF16);
@@ -1012,27 +968,16 @@ int gm_netmon_forward(const gm_netmon_params* p, int32_t B, int32_t N, const flo
             {
                 ProfileScope prof(PROF_AGG, s);
                 const int rpb = aggregate_rows_per_block(N);
-                static int agg_threads = -1;
-                if (agg_threads < 0) { const char* e = getenv("GM_AGG_THREADS"); agg_threads = e ? atoi(e) : 256; }
-                static int agg_staged = -1;
-                if (agg_staged < 0) { const char* e = getenv("GM_AGG_STAGE_LISTS"); agg_staged = e ? atoi(e) : 1; }
                 const unsigned agg_blocks = (unsigned)((R + rpb - 1) / rpb);
-                static int agg_map = -1;
-                if (agg_map < 0) { const char* e = getenv("GM_AGG_MAP"); agg_map = e ? atoi(e) : 2; }  // 2: pipelined (default), anything else: the L2 gather kernel
+                const int mean = p->agg_type == GM_AGG_MEAN, write_lo = math != GM_MATH_BF16;
                 const int pipe_stage = (int)round_up((int64_t)rpb * H * 4 + (int64_t)rpb * (DM + 1) * (int64_t)sizeof(int), 128);
                 const size_t pipe_smem = 128 + (size_t)AGG_STAGES * pipe_stage;
-                if (agg_map == 2 && rpb % N == 0 && rpb / N <= 32 && pipe_smem <= 72 * 1024 && ((uintptr_t)h & 15) == 0) {
-                    static int pipe_threads = -1, pipe_ctas = -1;
-                    if (pipe_threads < 0) {
-                        const char* e = getenv("GM_AGG_PIPE_WARPS");  // consumer warps per CTA
-                        int cw = e ? atoi(e) : 10;
-                        cw = cw < 1 ? 1 : (cw > 10 ? 10 : cw);
-                        const char* f = getenv("GM_AGG_PIPE_CTAS");  // CTAs per SM
-                        pipe_ctas = f ? atoi(f) : 3;
-                        pipe_ctas = pipe_ctas < 1 ? 1 : (pipe_ctas > 3 ? 3 : pipe_ctas);
+                if (rpb % N == 0 && rpb / N <= 32 && pipe_smem <= 72 * 1024 && ((uintptr_t)h & 15) == 0) {
+                    static bool configured = false;
+                    if (!configured) {
                         GM_CUDA(cudaFuncSetAttribute(aggregate_pk_pipe_kernel<0, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, 72 * 1024));
                         GM_CUDA(cudaFuncSetAttribute(aggregate_pk_pipe_kernel<128, 4>, cudaFuncAttributeMaxDynamicSharedMemorySize, 72 * 1024));
-                        pipe_threads = 32 * (cw + 1);
+                        configured = true;
                     }
                     int sms = 148;
                     {
@@ -1040,24 +985,14 @@ int gm_netmon_forward(const gm_netmon_params* p, int32_t B, int32_t N, const flo
                         cudaGetDevice(&dev);
                         cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
                     }
-                    const unsigned grid = std::min<unsigned>(agg_blocks, (unsigned)(sms * pipe_ctas));
-                    static int pipe_generic = -1;
-                    if (pipe_generic < 0) { const char* e = getenv("GM_AGG_PIPE_GENERIC"); pipe_generic = e ? atoi(e) : 0; }
-                    if (H == 128 && DM == 4 && !pipe_generic)
-                        GM_CUDA(launch_pdl(aggregate_pk_pipe_kernel<128, 4>, dim3(grid), dim3(pipe_threads), pipe_smem, s, h, H, w.m_pk, B, N, H,
-                                           nbr_all, deg, DM, list_index, (int)(p->agg_type == GM_AGG_MEAN), (int)(math != GM_MATH_BF16), rpb,
-                                           (int)agg_blocks, pipe_stage));
-                    else
-                        GM_CUDA(launch_pdl(aggregate_pk_pipe_kernel<0, 0>, dim3(grid), dim3(pipe_threads), pipe_smem, s, h, H, w.m_pk, B, N, H,
-                                           nbr_all, deg, DM, list_index, (int)(p->agg_type == GM_AGG_MEAN), (int)(math != GM_MATH_BF16), rpb,
-                                           (int)agg_blocks, pipe_stage));
+                    const unsigned grid = std::min<unsigned>(agg_blocks, (unsigned)(sms * AGG_PIPE_CTAS));
+                    auto kern = (H == 128 && DM == 4) ? aggregate_pk_pipe_kernel<128, 4> : aggregate_pk_pipe_kernel<0, 0>;
+                    kern<<<grid, AGG_PIPE_THREADS, pipe_smem, s>>>(h, H, w.m_pk, B, N, H, nbr_all, deg, DM, list_index, mean, write_lo, rpb,
+                                                                  (int)agg_blocks, pipe_stage);
+                } else {
+                    aggregate_pk_kernel<<<agg_blocks, AGG_THREADS, (size_t)rpb * (DM + 1) * sizeof(int), s>>>(
+                        h, H, w.m_pk, B, N, H, nbr_all, deg, DM, list_index, mean, write_lo, rpb);
                 }
-                else if (agg_staged)
-                    aggregate_pk_kernel<true><<<agg_blocks, agg_threads, (size_t)rpb * (DM + 1) * sizeof(int), s>>>(
-                        h, H, w.m_pk, B, N, H, nbr_all, deg, DM, list_index, p->agg_type == GM_AGG_MEAN, math != GM_MATH_BF16, rpb);
-                else
-                    aggregate_pk_kernel<false><<<agg_blocks, agg_threads, 0, s>>>(
-                        h, H, w.m_pk, B, N, H, nbr_all, deg, DM, list_index, p->agg_type == GM_AGG_MEAN, math != GM_MATH_BF16, rpb);
             }
             GM_LAUNCH_CHECK();
             float* hn = final_it ? state_out : hbuf[cur ^ 1];  // the last cell writes the new state in place (:562-564)
@@ -1207,9 +1142,9 @@ int gm_netmon_forward(const gm_netmon_params* p, int32_t B, int32_t N, const flo
         const unsigned blocks = (unsigned)((((rows + 7) / 8) * n_seg + 7) / 8);
         {
             ProfileScope prof(PROF_READOUT, s);
-            GM_CUDA(launch_pdl(readout_agents_pk_kernel, dim3(blocks), dim3(256), 0, s, h, ldh_cur, last, (int64_t)H, w.gmean, nbr_all, deg, DM,
-                               list_index, agent_node, A, B, N, H, use_nbr, use_glob, max_degree, agent_out, agent_out_ld,
-                               (uint8_t*)agent_out_pk, (int)(math != GM_MATH_BF16)));
+            readout_agents_pk_kernel<<<blocks, 256, 0, s>>>(h, ldh_cur, last, (int64_t)H, w.gmean, nbr_all, deg, DM, list_index, agent_node, A,
+                                                            B, N, H, use_nbr, use_glob, max_degree, agent_out, agent_out_ld,
+                                                            (uint8_t*)agent_out_pk, (int)(math != GM_MATH_BF16));
         }
         GM_LAUNCH_CHECK();
     } else if (agent_out) {

@@ -20,8 +20,6 @@ struct ReplayFields {
 // grid.y = field, grid.x strides over (transition, 16 / 8 / 4 / 1-byte unit)
 __global__ void replay_insert_kernel(ReplayFields F, int64_t capacity, int64_t index0, const int64_t* __restrict__ index_dev,
                                      int64_t n) {
-    pdl_trigger();
-    pdl_wait();
     const int64_t index = index0 + (index_dev ? *index_dev : 0);
     const gm_replay_field fd = F.f[blockIdx.y];
     const int64_t eb = fd.elem_bytes;
@@ -146,7 +144,7 @@ int gm_replay_insert(const gm_replay_field* fields, int32_t n_fields, int64_t ca
     dim3 grid((unsigned)blocks, n_fields);
     {
         ProfileScope prof(PROF_REPLAY, (cudaStream_t)stream);
-        GM_CUDA(launch_pdl(replay_insert_kernel, grid, dim3(256), 0, (cudaStream_t)stream, F, capacity, index, index_dev, n));
+        replay_insert_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(F, capacity, index, index_dev, n);
     }
     GM_LAUNCH_CHECK();
     return GM_OK;

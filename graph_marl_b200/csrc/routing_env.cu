@@ -262,8 +262,6 @@ template <int MODE, int WPE, bool SIMPLE>
 __global__ void __launch_bounds__(WARPS_PER_CTA * 32, GM_ROUTING_MIN_CTAS)
 routing_kernel(const gm_routing_desc d, const gm_routing_io io, const RoutingLayout L) {
     extern __shared__ __align__(16) uint8_t smem[];
-    pdl_trigger();
-    pdl_wait();
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int role = WPE == 2 ? (warp & 1) : 0;
     const int slot_in_cta = WPE == 2 ? (warp >> 1) : warp;
@@ -862,7 +860,7 @@ static int launch_routing(int mode, const gm_routing_desc* d, const gm_routing_i
 #define GM_ROUTING_LAUNCH(MODE_, WPE_, SIMPLE_)                                                                              \
     do {                                                                                                                     \
         GM_CUDA(cudaFuncSetAttribute(routing_kernel<MODE_, WPE_, SIMPLE_>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
-        GM_CUDA(launch_pdl(routing_kernel<MODE_, WPE_, SIMPLE_>, grid, block, smem, s, dd, *io, L));                         \
+        routing_kernel<MODE_, WPE_, SIMPLE_><<<grid, block, smem, s>>>(dd, *io, L);                                          \
     } while (0)
 #define GM_ROUTING_VARIANT(MODE_)                                 \
     do {                                                          \

@@ -1,6 +1,5 @@
 // runtime.cu -- error reporting, device check, launch accounting.
 #include <stdarg.h>
-#include <stdlib.h>
 
 #include <vector>
 
@@ -22,15 +21,6 @@ void profile_begin(int category, cudaStream_t s) {
 }
 void profile_end(cudaStream_t s) {
     if (!g_prof_events.empty()) cudaEventRecord(g_prof_events.back().e1, s);
-}
-
-bool pdl_enabled() {
-    static int on = -1;
-    if (on < 0) {
-        const char* e = getenv("GM_PDL");
-        on = e ? atoi(e) : 0;  // measured: 0.815-0.829 ms per step with it, 0.775-0.785 without (DESIGN.md section 5)
-    }
-    return on != 0;
 }
 
 void set_error(const char* fmt, ...) {

@@ -509,9 +509,10 @@ class NetMon(nn.Module):
         want_agent_pk (tensor-core modes): the agents' graph observation is written ONCE, tile-packed, and
         returned as PackedRows (no fp32 rows).  state_out: optional f32 [B,N,S] tensor that receives the new state (e.g.
         a block of the replay ring's node_state field, so that the state is never copied).  sparse_nnz > 0: the caller
-        guarantees rows of x with at most that many (<= 12) non-zeros (the Routing env's one-hot node observations have 12):
-        the tensor-core path then runs encoder layers 1 + 2 as one kernel.  sparse_rows: those rows already in sparse form
-        (int32 [B,N,24] on a 128-row padded allocation, Routing's `node_sparse` output); None = derived from x.
+        guarantees rows of x with at most that many (<= 12) non-zeros (the Routing env's one-hot node observations have 12).
+        sparse_rows: those rows already in sparse form (int32 [B,N,24] on a 128-row padded allocation, Routing's
+        `node_sparse` output); when they are given with sparse_nnz <= 6, the tensor-core path runs encoder layers 1 + 2 as
+        one kernel (other rows take the two-layer path).
         static_rows: f32 [S, Dn] dictionary of row parts (Routing's `node_static_rows`; layer 1 applied to them is folded
         into the weight pack): the supplied sparse rows index it (static_only, Routing's form), or name static row s as
         column Dn + s next to ordinary input columns (static_only=False)."""

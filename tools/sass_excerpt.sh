@@ -16,8 +16,8 @@ OUT=${1:-profiles/sass_linear_tc.txt}
     /LDTM/ { c++ } /UTCBAR/ { d++ } /UBLKCP/ { e++ } /SYNCS/ { f++ }
     END { if (fn != "") print fn " | " a " | " b " | " c " | " d " | " e " | " f }' | awk -F'|' '$2+$4+$6 > 0' | c++filt | cut -c1-220
   echo
-  echo "# excerpt: the MMA issue loop of linear_tc_kernel<256,3,EPI_LSTM,4,false> (first 60 tensor-core / barrier lines)"
-  cuobjdump -sass "$LIB" | awk '/Function : .*linear_tc_kernelILi256ELi3ELi1ELi4ELb0/ {p=1} p && /Function :/ && !/linear_tc_kernelILi256ELi3ELi1ELi4ELb0/ {p=0} p' \
+  echo "# excerpt: the MMA issue loop of linear_tc_kernel<256,3,EPI_LSTM,4> (first 60 tensor-core / barrier lines)"
+  cuobjdump -sass "$LIB" | awk '/Function : .*linear_tc_kernelILi256ELi3ELi1ELi4EE/ {p=1} p && /Function :/ && !/linear_tc_kernelILi256ELi3ELi1ELi4EE/ {p=0} p' \
     | grep -E "UTCHMMA|UTCBAR|LDTM|UBLKCP|SYNCS|UTCATOMSWS|UTCCP" | head -60
 } > "$OUT"
 wc -l "$OUT"
