@@ -96,6 +96,22 @@ class NetmonGrads(C.Structure):
                 ("rnn_obs", CellGrads), ("rnn_update", CellGrads)]
 
 
+GM_LEARNER_PARTIALS = 296
+
+
+class OptEntry(C.Structure):
+    _fields_ = [(n, C.c_void_p) for n in ("param", "grad", "exp_avg", "exp_avg_sq")] + [("numel", C.c_int64)]
+
+
+class OptPair(C.Structure):
+    _fields_ = [("online", C.c_void_p), ("target", C.c_void_p), ("numel", C.c_int64)]
+
+
+class OptHparams(C.Structure):
+    _fields_ = [(n, C.c_double) for n in ("lr", "beta1", "beta2", "eps", "weight_decay", "tau")] + \
+               [("clip_value", C.c_float), ("max_norm", C.c_float)]
+
+
 _lib = None
 
 _SIGS = {
@@ -143,6 +159,12 @@ _SIGS = {
     "gm_pcg64_seed": (None, [C.c_void_p, C.c_uint64]),
     "gm_pcg64_choice": (None, [C.c_void_p, C.c_int64, C.c_int64, C.c_void_p]),
     "gm_replay_sample_indices": (C.c_int, [C.c_void_p, C.c_int64, C.c_int64, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p]),
+    "gm_replay_sample_env_sequences": (C.c_int, [C.c_void_p, C.c_int64, C.c_int64, C.c_int32, C.c_int32, C.c_int32, C.c_void_p,
+                                                 C.c_void_p]),
+    "gm_td_grad": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, C.c_float,
+                             C.c_float, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "gm_optimizer_step": (C.c_int, [C.c_void_p, C.c_int32, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p,
+                                    C.c_void_p]),
     "gm_mlp_tape_floats": (C.c_int64, [C.c_void_p, C.c_int64]),
     "gm_mlp_train_workspace_bytes": (C.c_int64, [C.c_void_p, C.c_int64]),
     "gm_mlp_forward_train": (C.c_int, [C.c_void_p, C.c_int64, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_int64,

@@ -114,6 +114,22 @@ __global__ void replay_indices_kernel(Pcg64* __restrict__ state, int64_t count, 
     *state = g;
 }
 
+// Per-env sequences on a ring that a batched step fills with B consecutive slots (one per env): the start step is drawn
+// with the rule above counted in steps, then the env; row o is the slot of that env o steps later.
+__global__ void env_sequences_kernel(Pcg64* __restrict__ state, int64_t steps_stored, int64_t head_step, int num_envs,
+                                     int batch, int seq_len, int64_t* __restrict__ out) {
+    if (blockIdx.x || threadIdx.x) return;
+    Pcg64 g = *state;
+    const int64_t first = head_step % steps_stored;
+    for (int i = 0; i < batch; i++) out[i] = (first + pcg_bounded(g, steps_stored - seq_len)) % steps_stored;
+    for (int i = 0; i < batch; i++) {
+        const int64_t env = pcg_bounded(g, num_envs);
+        const int64_t s0 = out[i];
+        for (int o = 0; o < seq_len; o++) out[(int64_t)o * batch + i] = ((s0 + o) % steps_stored) * num_envs + env;
+    }
+    *state = g;
+}
+
 }  // namespace gm
 
 using namespace gm;
@@ -157,6 +173,17 @@ int gm_replay_sample_indices(uint64_t* state_dev, int64_t count, int64_t index, 
     GM_CHECK_ARG(count > 0 && count <= 0xFFFFFFFFll && (seq_len <= 1 || count - seq_len > 0), "count %lld / sequence length %d",
                  (long long)count, seq_len);
     replay_indices_kernel<<<1, 32, 0, (cudaStream_t)stream>>>((Pcg64*)state_dev, count, index, batch, seq_len, out);
+    GM_LAUNCH_CHECK();
+    return GM_OK;
+}
+
+int gm_replay_sample_env_sequences(uint64_t* state_dev, int64_t steps_stored, int64_t head_step, int32_t num_envs,
+                                   int32_t batch, int32_t seq_len, int64_t* out, void* stream) {
+    GM_CHECK_ARG(state_dev && out && batch > 0 && num_envs > 0 && seq_len >= 1, "bad sampler arguments");
+    GM_CHECK_ARG(steps_stored - seq_len > 0 && steps_stored <= 0xFFFFFFFFll && head_step >= 0,
+                 "%lld stored steps / sequence length %d", (long long)steps_stored, seq_len);
+    env_sequences_kernel<<<1, 32, 0, (cudaStream_t)stream>>>((Pcg64*)state_dev, steps_stored, head_step, num_envs, batch,
+                                                             seq_len, out);
     GM_LAUNCH_CHECK();
     return GM_OK;
 }

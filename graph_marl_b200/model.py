@@ -83,7 +83,7 @@ class _PackedWeights:
     parameter's storage or version counter changes (optimizer step, load_state_dict, .to())."""
 
     def __init__(self):
-        self.buf, self.key = None, None
+        self.buf, self.key, self._pack_fn = None, None, None
 
     def get(self, module, extra, nbytes_fn, pack_fn):
         params = list(module.parameters())
@@ -95,8 +95,15 @@ class _PackedWeights:
                 self.buf = torch.empty(max(n, 256), dtype=torch.uint8, device=dev)
             assert self.buf.data_ptr() % 256 == 0
             pack_fn(self.buf)
-            self.key = key
+            self.key, self._pack_fn = key, pack_fn
         return self.buf
+
+    def refresh(self):
+        """Repack the current parameter values into the existing buffer, with the layout of the last pack.  For writers
+        that change parameters without moving their version counters (the learner's optimizer kernel writes through
+        raw pointers): captured CUDA graphs hold this buffer's address and keep reading it."""
+        if self._pack_fn is not None:
+            self._pack_fn(self.buf)
 
 
 # ---- training path: device-side backward (csrc/train.cu) behind torch.autograd ---------------------

@@ -294,15 +294,52 @@ class CompactReplayBuffer(_RingSampler):
         b = (int(t) % self.M) * self._B
         return self.node_state[b:b + self._B]
 
-    def _state_slots(self, idx):
-        """Ring slots (device int64) -> rows of the state ring: slot s was written by step t = T - 1 - age."""
+    def _state_slots(self, idx, clock=None):
+        """Ring slots (device int64) -> rows of the state ring: slot s was written by step t = T - 1 - age.  clock: the
+        (head step, steps_total) pair as device int64 tensors instead of the host counters (captured CUDA graphs)."""
         if not self.state_ring:
             return idx
         B, cap = self._B, self.cap_steps
-        j_now = (self.index // B) % cap
+        j_now, total = clock if clock is not None else ((self.index // B) % cap, self.steps_total)
         age = (j_now - 1 - idx // B) % cap
-        t = self.steps_total - 1 - age
+        t = total - 1 - age
         return (t % self.M) * B + idx % B
+
+    def clock(self):
+        """(head step, steps_total): the host counters _state_slots() reads, for a device copy of them."""
+        return (self.index // self._B) % self.cap_steps, self.steps_total
+
+    def sample_env_sequences(self, batch_size, seq_len, out=None):
+        """[seq_len, batch_size] ring slots (device int64) of per-env sequences in state-ring mode: row k holds the slot
+        of row 0's env k batched steps later.  Start steps follow get_batch's sequence rule counted in steps (the whole
+        sequence stays behind the ring head), then one env per sample is drawn (csrc/replay_sampler.cu,
+        gm_replay_sample_env_sequences).  Needs device_sampler=True; `out` receives the slots in place."""
+        assert self.state_ring and self._pcg_dev is not None, "per-env sequences need the state ring and the device sampler"
+        _lib.require_device()
+        T = int(seq_len)
+        if out is None:
+            out = torch.empty((T, batch_size), dtype=torch.int64, device=self.device)
+        assert out.shape == (T, batch_size) and out.dtype == torch.int64 and out.is_contiguous()
+        B = self._B
+        with torch.cuda.device(self.device):
+            _lib.check(_lib.lib().gm_replay_sample_env_sequences(self._pcg_dev.data_ptr(), self.count // B, self.index // B,
+                                                                 B, batch_size, T, out.data_ptr(), _lib.current_stream()))
+        return out
+
+    def learner_views(self, idx, clock=None):
+        """What a learner that recomputes the graph observation needs of the transitions at ring slots `idx` (device
+        int64 [n]): the gathered compact fields (rec / next_rec / topo / action / reward / done / episode_done /
+        node_state), the agent observations, node observations and agent nodes of both sides (`obs`, `node_obs`,
+        `agent_node`, `next_obs`, `next_node_obs`, `next_agent_node`, plus the env's sparse node rows `node_sparse` /
+        `next_node_sparse` for NetMon's sparse encoder) -- no NetMon forwards, unlike get_batch.
+        clock: see _state_slots."""
+        be = self.env.get()
+        g = self._gather(idx, clock)
+        cur = be.observe_records(g["rec"], g["topo"])
+        nxt = be.observe_records(g["next_rec"], g["topo"])
+        for k in ("obs", "node_obs", "agent_node", "node_sparse"):
+            g[k], g["next_" + k] = cur[k], nxt[k]
+        return g
 
     def bytes_per_transition(self):
         return sum(getattr(self, f)[0].numel() * getattr(self, f).element_size() for f in self.FIELDS)
@@ -388,7 +425,7 @@ class CompactReplayBuffer(_RingSampler):
         self.steps_total += 1
 
     # ---- sample: gather the compact fields, rebuild the reference's 17 dense fields ----------------
-    def _gather(self, idx):
+    def _gather(self, idx, clock=None):
         n = idx.shape[0]
         spec = [("rec", torch.uint8, 0), ("next_rec", torch.uint8, 0), ("topo", torch.int32, 0), ("action", torch.int64, 2),
                 ("reward", torch.float32, 0), ("done", torch.bool, 0), ("episode_done", torch.bool, 0),
@@ -402,7 +439,7 @@ class CompactReplayBuffer(_RingSampler):
             fields[k].elem_bytes = ring[0].numel() * ring.element_size()
         with torch.cuda.device(self.device):
             if self.state_ring:  # the state field has its own modulus: gather it with its own row indices
-                sidx = self._state_slots(idx).contiguous()
+                sidx = self._state_slots(idx, clock).contiguous()
                 _lib.check(_lib.lib().gm_replay_sample(fields, len(spec) - 1, idx.data_ptr(), n, _lib.current_stream()))
                 last = (_lib.ReplayField * 1)()
                 C.memmove(last, C.byref(fields[len(spec) - 1]), C.sizeof(_lib.ReplayField))

@@ -362,6 +362,12 @@ GM_API void gm_pcg64_choice(uint64_t* state, int64_t n, int64_t size, int64_t* o
  * and row o = (start + o) % count.  No host round trip. */
 GM_API int gm_replay_sample_indices(uint64_t* state_dev, int64_t count, int64_t index, int32_t batch,
                              int32_t seq_len, int64_t* out, void* stream);
+/* Per-env sequences on a ring that each batched step fills with num_envs consecutive slots (one per env), for the
+ * batched learner: with S = steps_stored, start_i = (head_step % S + choice(S - seq_len)) % S for i < batch (the rule
+ * above counted in steps), then env_i = choice(num_envs) for i < batch, both from the same device PCG64 state;
+ * out i64[seq_len, batch] row o = ((start_i + o) % S) * num_envs + env_i. */
+GM_API int gm_replay_sample_env_sequences(uint64_t* state_dev, int64_t steps_stored, int64_t head_step, int32_t num_envs,
+                                   int32_t batch, int32_t seq_len, int64_t* out, void* stream);
 
 /* ======================================================================== */
 /* Training path: forward with a tape + backward (replaces the torch autograd */
@@ -436,6 +442,39 @@ GM_API int gm_nccl_comm_destroy(void* comm);
 GM_API int gm_allreduce_grads(void* comm, float* flat, int64_t n, int32_t average, void* stream);
 /* start-up: every rank's flat parameter buffer <- rank root's */
 GM_API int gm_broadcast_weights(void* comm, float* flat, int64_t n, int32_t root, void* stream);
+
+/* ======================================================================== */
+/* Batched DQN learner (graph_marl_b200/learner.py): TD gradient + optimizer */
+/* tail.  Fixed-order reductions (no float atomics): eager calls and CUDA-   */
+/* graph replays agree bit for bit.  `partials` is a device workspace of     */
+/* GM_LEARNER_PARTIALS doubles.                                              */
+/* ======================================================================== */
+#define GM_LEARNER_PARTIALS 296
+/* q, q_next f32[rows, n_actions] (online / target network), action i64[rows], reward f32[rows], done bool[rows]:
+ * y = reward + (!done) * gamma * max_a q_next (a NaN in a q_next row propagates, like torch.max); dq = 2 * scale * (q - y)
+ * at the taken action, 0 elsewhere;
+ * *loss (device f32) += scale * sum_rows (q[action] - y)^2 */
+GM_API int gm_td_grad(const float* q, const float* q_next, const int64_t* action, const float* reward, const uint8_t* done,
+               int64_t rows, int32_t n_actions, float gamma, float scale, float* dq, float* loss, double* partials,
+               void* stream);
+typedef struct gm_opt_entry {           /* one optimised tensor (device pointers) */
+    float *param, *grad, *exp_avg, *exp_avg_sq;
+    int64_t numel;
+} gm_opt_entry;
+typedef struct gm_opt_pair {            /* one tensor of the target network and its online counterpart */
+    const float* online;
+    float* target;
+    int64_t numel;
+} gm_opt_pair;
+typedef struct gm_opt_hparams {
+    double lr, beta1, beta2, eps, weight_decay, tau;
+    float clip_value, max_norm;
+} gm_opt_hparams;
+/* One update over the device tables: grads clamped to +-clip_value in place; their global L2 norm; grads scaled by
+ * min(1, max_norm / (norm + 1e-6)) in place; *step_dev += 1; AdamW in the operation order of
+ * torch.optim.AdamW(foreach=False); then target = tau * online + (1 - tau) * target for every pair. */
+GM_API int gm_optimizer_step(const gm_opt_entry* table_dev, int32_t n_entries, const gm_opt_pair* pairs_dev,
+                      int32_t n_pairs, int64_t* step_dev, const gm_opt_hparams* h, double* partials, void* stream);
 
 /* ======================================================================== */
 /* building blocks exposed for tests / profiling                             */
