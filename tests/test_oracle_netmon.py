@@ -31,6 +31,36 @@ def test_netmon_recurrent_rollout(entry):
         assert np.abs(ao2 - G[name + "_agent_out"][t]).max() < tol
 
 
+@pytest.mark.parametrize("entry", [str(x) for x in G["case_names"] if str(x).split("|")[1] in ("lstm", "lnlstm")
+                                   and netmon_case(G, x)[1]["rnn_carryover"]])
+def test_fp64_autograd_reference_reproduces_recording(entry):
+    """`NetMon._forward_autograd` of a `.double()` module, the fp64 reference that tests/test_gpu_train_kernels.py
+    differentiates, reproduces the reference's recorded agent outputs and carried states."""
+    import torch
+    import torch.nn.functional as F
+
+    from graph_marl_b200.model import NetMon
+
+    name, cfg = netmon_case(G, entry)
+    X, ADJ, NAM = G["node_obs"], G["node_adj"], G["node_agent"]
+    T, B, N, Dn = X.shape
+    nm = NetMon(Dn, cfg["hidden"], cfg["enc"], cfg["iterations"], F.leaky_relu, rnn_type=cfg["rnn_type"],
+                agg_type=cfg["agg_type"], output_neighbor_hidden=cfg["output_neighbor_hidden"],
+                output_global_hidden=cfg["output_global_hidden"])
+    w = det_weights(netmon_shapes(Dn, cfg["hidden"], cfg["enc"], cfg["rnn_type"]), cfg["wseed"])
+    nm.load_state_dict({k: torch.from_numpy(v) for k, v in w.items()})
+    nm.double()
+    nm.state = torch.zeros((B, N, nm.state_size), dtype=torch.float64)
+    tol = TOL[cfg["rnn_type"]]
+    with torch.no_grad():
+        for t in range(T):
+            out = nm._forward_autograd(torch.from_numpy(X[t]).double(), torch.from_numpy(ADJ[t]).double(),
+                                       torch.from_numpy(NAM[t]).double(), None, False)
+            assert out.dtype == torch.float64 and out.shape == G[name + "_agent_out"][t].shape
+            assert np.abs(out.numpy() - G[name + "_agent_out"][t]).max() < tol, t
+            assert np.abs(nm.state.numpy() - G[name + "_state"][t]).max() < tol, t
+
+
 def test_netmon_simple_env_degree2_readout():
     cfg = dict(hidden=8, iterations=2, rnn_type="lstm", rnn_carryover=True, agg_type="sum",
                output_neighbor_hidden=True, output_global_hidden=False)
