@@ -14,6 +14,7 @@ LIB_PATH = os.environ.get("GM_LIB_PATH") or os.path.join(_HERE, "lib", "libgraph
 GM_MAX_LAYERS = 8
 GM_REPLAY_MAX_FIELDS = 24
 GM_MT_STATE_WORDS = 625
+GM_TOPOLOGY_MAX_NODES = 512
 GM_PCG64_STATE_WORDS = 6
 GM_NCCL_UNIQUE_ID_BYTES = 128
 RNN_TYPES = {"lstm": 0, "lnlstm": 1, "gru": 2, "none": 3}
@@ -43,6 +44,11 @@ class RoutingIO(C.Structure):
                                           "ring_episode_done")] + \
                [("ring_capacity", C.c_int64), ("ring_index", C.c_int64), ("ring_index_dev", C.c_void_p),
                 ("ring_episode_flag", C.c_int32), ("ring_pad", C.c_int32)]
+
+
+class TopologyTables(C.Structure):
+    _fields_ = [("P", C.c_int32), ("N", C.c_int32)] + \
+               [(n, C.c_void_p) for n in ("edges", "node_edges", "node_nbrs", "apsp", "nbr_all", "deg")]
 
 
 class CellParams(C.Structure):
@@ -131,6 +137,8 @@ _SIGS = {
                                        C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                        C.c_void_p, C.c_void_p, C.c_void_p]),
     "gm_topology_apsp": (C.c_int, [C.c_int32, C.c_int32, C.c_void_p, C.c_void_p]),
+    "gm_topology_generate_device": (C.c_int, [C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32,
+                                              C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "gm_routing_state_layout": (C.c_int, [C.c_int32, C.c_int32, C.c_int32, C.c_void_p]),
     "gm_routing_reset": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p]),
     "gm_routing_step": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p]),

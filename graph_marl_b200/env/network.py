@@ -158,6 +158,18 @@ class Network:
             topology_seed = np.random.choice(seed_list)
         return int(topology_seed), no_seed_provided
 
+    def pick_fresh_seeds(self, n):
+        """n fresh topology seeds (int64 [n]) drawn from the global stream exactly as n calls of pick_seed() without a
+        seed list draw them, this network's exclusion list included: one vectorised draw, replayed call by call from the
+        same stream state when it hit an excluded seed (which pick_seed redraws at once)."""
+        state = np.random.get_state()
+        seeds = np.random.randint(2**31 - 1, size=n).astype(np.int64)
+        ex = self.exclude_seeds
+        if ex and np.isin(seeds, np.fromiter(ex, np.int64, len(ex))).any():
+            np.random.set_state(state)
+            seeds = np.array([self.pick_seed(None, None, ex)[0] for _ in range(n)], np.int64)
+        return seeds
+
     def _create_valid_network(self, seed_list=None, seed_index=None, seeds_exclude=None):
         seed, fresh = self.pick_seed(seed_list, seed_index, seeds_exclude)
         t = generate_tables(self.n_nodes, seed, allow_reseed=fresh, exclude=seeds_exclude)

@@ -55,6 +55,7 @@ class TopologyPool:
         self.deg = torch.from_numpy(np.stack([l[1] for l in lists])).to(device)
         self.seeds = [t.get("seed") for t in tables]
         self.edges_host = np.array(tables[0]["edges"], copy=True) if self.T == 1 else None
+        self.fresh = False  # slots() pools: filled by generate()
         # The constant part of every node observation row (routing.py:193-234: one-hot of the node, of its three
         # neighbours, the three edge lengths) as dense rows, for small pools: NetMon folds layer 1 applied to them into
         # its weight pack and the env then names that part of a row as ONE sparse entry (model.NetMon).  The five
@@ -78,6 +79,61 @@ class TopologyPool:
             for q in range(3):
                 rows[dyn + 2 + q, N + 2 + q * (N + 2) + N + 1] = 1.0
             self.static_rows = torch.from_numpy(rows).to(device)
+
+    @classmethod
+    def slots(cls, P, n_nodes, device):
+        """P empty slots at fixed device addresses, filled by generate() (Routing's fresh-topology mode).  Such a pool has
+        no static rows: its slots change from episode to episode, NetMon's weight pack could not fold them in."""
+        pool = cls.__new__(cls)
+        N, E = int(n_nodes), 3 * int(n_nodes) // 2
+        z = lambda *shape: torch.zeros(shape, dtype=torch.int32, device=device)
+        pool.T = int(P)
+        pool.node_edges, pool.node_nbrs, pool.edges, pool.apsp = z(P, N, 3), z(P, N, 3), z(P, E, 4), z(P, N, N)
+        pool.nbr_all, pool.deg = z(P, N, 4), z(P, N)
+        pool.seeds = [None] * pool.T
+        pool.edges_host = None
+        pool.static_rows = None
+        pool.fresh = True
+        return pool
+
+    def generate(self, seeds, slot, exclude=None, max_attempts=10000):
+        """Generate topology b from seeds[b] (gm_topology_generate_device: what generate_tables(N, seeds[b],
+        allow_reseed=True, exclude) builds) into slot slot[b] (device int32 [B]), in place, and refresh the lazily built
+        caches of those slots.  exclude: device int64 tensor of seeds a reseed must skip.  Returns the host arrays
+        (seed_used int64 [B], repetitions int32 [B]); raises GraphMarlError when an env found no valid topology within
+        `max_attempts` graphs."""
+        _lib.require_device()
+        dev, N, B = self.apsp.device, self.apsp.shape[-1], len(seeds)
+        seeds = np.ascontiguousarray(seeds, dtype=np.int64)
+        seeds_d = torch.from_numpy(seeds).to(dev)
+        used = torch.empty((B,), dtype=torch.int64, device=dev)
+        reps = torch.empty((B,), dtype=torch.int32, device=dev)
+        status = torch.zeros((1,), dtype=torch.int32, device=dev)
+        t = _lib.TopologyTables(P=self.T, N=N, edges=self.edges.data_ptr(), node_edges=self.node_edges.data_ptr(),
+                                node_nbrs=self.node_nbrs.data_ptr(), apsp=self.apsp.data_ptr(), nbr_all=self.nbr_all.data_ptr(),
+                                deg=self.deg.data_ptr())
+        n_ex = 0 if exclude is None else exclude.numel()
+        with torch.cuda.device(dev):
+            _lib.check(_lib.lib().gm_topology_generate_device(C.byref(t), B, seeds_d.data_ptr(), slot.data_ptr(),
+                                                              _lib.ptr(exclude) if n_ex else None, n_ex, int(max_attempts),
+                                                              used.data_ptr(), reps.data_ptr(), status.data_ptr(),
+                                                              _lib.current_stream()))
+        st = int(status.item())
+        if st > 0:
+            raise _lib.GraphMarlError(f"no valid {N}-node topology within {max_attempts} attempts from seed {int(seeds[st - 1])}")
+        if st < 0:
+            raise _lib.GraphMarlError(f"env {-st - 1}: topology slot outside the pool's {self.T} slots")
+        sl = slot.long()
+        if getattr(self, "apsp_f32", None) is not None:
+            self.apsp_f32[sl] = self.apsp[sl].float()
+        if getattr(self, "node_adj", None) is not None:
+            adj = torch.zeros((B, N, N), dtype=torch.int8, device=dev)
+            adj.scatter_(2, self.nbr_all[sl].long(), 1)
+            self.node_adj[sl] = adj
+        used, reps = used.cpu().numpy(), reps.cpu().numpy()
+        for s_, u in zip(slot.cpu().tolist(), used.tolist()):
+            self.seeds[s_] = u
+        return used, reps
 
 
 class Routing(NetworkEnv):
@@ -121,6 +177,9 @@ class Routing(NetworkEnv):
         self._state = None
         self._pool = None
         self._topo_index = None
+        self._topo_episodes = 1  # fresh-topology mode: episodes whose pool slots are kept (set_topology_episodes)
+        self._episode = 0
+        self._exclude_dev = None
         self._draws = None
         self._ring = None  # set_ring(): the next step writes its compact replay transition itself
         self._out = {}
@@ -171,6 +230,17 @@ class Routing(NetworkEnv):
     def set_topology_pool(self, pool: TopologyPool, topo_index=None):
         self._pool = pool
         self._topo_index = topo_index
+
+    def set_topology_episodes(self, S):
+        """Fresh-topology mode (batched, Network(random_topology=True) without a seed list): the pool keeps the topologies
+        of the last S episodes, B * S slots at fixed addresses; env b's topology of episode e lives in slot
+        (e mod S) * B + b.  A compact replay ring names a transition's topology by its slot, so S must exceed the number
+        of episodes whose transitions the ring can still hold.  Default 1: a reset overwrites the previous episode's
+        topologies.  Takes effect at the next reset (a pool of another size is allocated then)."""
+        S = int(S)
+        if S < 1:
+            raise ValueError(f"set_topology_episodes needs S >= 1, got {S}")
+        self._topo_episodes = S
 
     def set_draws(self, start, target, size):
         """Host-supplied packet draws for the NEXT reset/step: arrays [B,A] (or [A]); slot s
@@ -282,17 +352,37 @@ class Routing(NetworkEnv):
                 self._pool = TopologyPool([generate_tables(net.n_nodes, s) for s in net.seeds], self.device)
             idx = np.random.randint(len(net.seeds), size=B).astype(np.int32)
             net.reset()
-        else:  # a fresh random topology per env and episode
-            tabs = []
-            for _ in range(B):
-                net.reset()
-                tabs.append(net.tables)
-            self._pool = TopologyPool(tabs, self.device)
-            idx = np.arange(B, dtype=np.int32)
+        else:  # a fresh random topology per env and episode, generated on the device into this episode's slots
+            P = B * self._topo_episodes
+            if self._pool is None or not self._pool.fresh or self._pool.T != P:
+                self._pool = TopologyPool.slots(P, net.n_nodes, self.device)
+                self._episode = 0
+            idx = np.arange(B, dtype=np.int32) + (self._episode % self._topo_episodes) * B
+            self._episode += 1
         if self._topo_index is not None and self._topo_index.shape[0] == B:
             self._topo_index.copy_(torch.from_numpy(idx))  # same device address: captured CUDA graphs keep reading it
         else:
             self._topo_index = torch.from_numpy(idx).to(self.device)
+        if len(net.seeds) == 0:
+            self._generate_fresh(B)
+
+    def _generate_fresh(self, B):
+        """B calls of network.reset() without a seed list, on the device: the seeds come from the global stream as
+        pick_seed draws them, the topologies are built into the slots _topo_index names, and the Network ends as after
+        those calls (sampled_topology_seeds extended by the B seeds used, its tables the last env's topology)."""
+        net = self.network
+        ex = net.exclude_seeds
+        if ex and self._exclude_dev is None:
+            self._exclude_dev = torch.from_numpy(np.array(sorted(ex), np.int64)).to(self.device)
+        seeds = net.pick_fresh_seeds(B)
+        used, _ = self._pool.generate(seeds, self._topo_index, self._exclude_dev if ex else None)
+        net.sampled_topology_seeds.extend(int(s) for s in used[:-1])
+        # the last env's topology once more on the host, for the Network's attribute views (nodes, edges, adj_matrix)
+        net._install(generate_tables(net.n_nodes, int(seeds[-1]), allow_reseed=True, exclude=ex))
+        if net.current_topology_seed != int(used[-1]):
+            raise _lib.GraphMarlError(f"device topology from seed {int(seeds[-1])} ended on seed {int(used[-1])}, "
+                                      f"the host generator on {net.current_topology_seed}")
+        net.sampled_topology_seeds.append(net.current_topology_seed)
 
     def reset(self):
         _lib.require_device()

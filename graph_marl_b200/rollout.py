@@ -31,6 +31,10 @@ CONFIGS = {
     # reference generator (network.py:100-120), 50-step episodes, K=1 (16384 envs over 8 GPUs = 2048 per GPU)
     "cfg3": dict(n_nodes=20, n_data=20, topo_seed=476, random_topology=True, n_topologies=4096, congestion=False, K=1,
                  rnn="lstm", H=128, enc=(512, 256), dqn=(512, 256), episode_steps=50),
+    # configs[2] as the reference trains it without a seed list (Network(random_topology=True)): a fresh topology per env
+    # and episode, generated on the device into the env's topology pool (Routing.set_topology_episodes)
+    "cfg3fresh": dict(n_nodes=20, n_data=20, topo_seed=476, random_topology=True, n_topologies=None, congestion=False,
+                      K=1, rnn="lstm", H=128, enc=(512, 256), dqn=(512, 256), episode_steps=50),
     # BASELINE.json configs[3]: synthetic large graph 200 nodes / 100 agents, lnlstm, K=4
     "cfg4": dict(n_nodes=200, n_data=100, topo_seed=476, congestion=True, K=4, rnn="lnlstm", H=128,
                  enc=(512, 256), dqn=(512, 256), episode_steps=300),
@@ -71,7 +75,7 @@ class Rollout:
         torch.manual_seed(seed)
         np.random.seed(seed)
         if c.get("random_topology"):
-            net = Network(N, random_topology=True, n_random_seeds=c["n_topologies"], topology_init_seed=c["topo_seed"])
+            net = Network(N, random_topology=True, n_random_seeds=c.get("n_topologies"), topology_init_seed=c["topo_seed"])
         else:
             net = Network(N, random_topology=False, topology_init_seed=c["topo_seed"])
         self.base_env = Routing(net, A, 1, enable_congestion=c["congestion"], num_envs=num_envs, device=device,
@@ -105,6 +109,11 @@ class Rollout:
                 self.buff = ReplayBuffer(seed, cap, A, Dj, 0, N, Dn, self.netmon.get_state_size(), N, device=device,
                                          device_sampler=device_sampler)
         self.state_ring = self.compact and self.buff.state_ring
+        if c.get("random_topology") and not c.get("n_topologies") and self.buff is not None:
+            # fresh topologies: keep the pool slots of every episode the ring can still hold transitions of, plus the
+            # current one (the compact ring names a transition's topology by its pool slot)
+            cap_steps = -(-self.buff.buffer_size // num_envs)
+            self.base_env.set_topology_episodes(-(-cap_steps // c["episode_steps"]) + 1)
         # state-ring mode: the env's step kernel writes the transition into the ring itself (gm_routing_io.ring_*)
         self.fused_insert = bool(fused_insert) and self.state_ring and hasattr(self.base_env, "set_ring")
         self.sizes = dict(N=N, A=A, Dn=Dn, Da=Da, Dj=Dj, H=c["H"], K=c["K"])

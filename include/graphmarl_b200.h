@@ -83,6 +83,28 @@ GM_API int gm_topology_generate(uint32_t* global_state, int32_t n_nodes, int32_t
 /* apsp only, after edge lengths changed (network.py:292-329 randomize_edge_weights) */
 GM_API int gm_topology_apsp(int32_t n_nodes, int32_t n_edges, const int32_t* edges, int32_t* apsp);
 
+/* Device-resident topology tables of P pool slots (all int32, device pointers), the layout Routing reads. */
+#define GM_TOPOLOGY_MAX_NODES 512
+typedef struct gm_topology_tables {
+    int32_t P, N;          /* slots, nodes (E = 3N/2 edges) */
+    int32_t* edges;        /* [P,E,4] (start, end, length, 0) in creation order, start < end */
+    int32_t* node_edges;   /* [P,N,3] incident edge ids ordered by neighbour id */
+    int32_t* node_nbrs;    /* [P,N,3] those neighbours */
+    int32_t* apsp;         /* [P,N,N] shortest-path weights */
+    int32_t* nbr_all;      /* [P,N,4] the node and its three neighbours, ascending (NetMon's adjacency lists) */
+    int32_t* deg;          /* [P,N]   4 */
+} gm_topology_tables;
+/* B topologies in one launch: env b's topology is gm_topology_generate(seed_mode 2, seeds[b], exclude) -- bit-identical
+ * tables, seed_used[b] and repetitions[b] -- written into pool slot slot[b] (device arrays seeds i64[B], slot i32[B],
+ * exclude i64[n_exclude], seed_used i64[B], repetitions i32[B]).  Each env builds at most `max_attempts` graphs; *status
+ * (device i32, zeroed by the caller) is left 0 on success, else set to b + 1 for an env b that ran out of attempts or
+ * -(b + 1) for one whose slot lies outside [0, P) (nothing is written for that env).  N even,
+ * 4 <= N <= GM_TOPOLOGY_MAX_NODES.  Asynchronous on `stream`. */
+GM_API int gm_topology_generate_device(const gm_topology_tables* tables, int32_t B, const int64_t* seeds,
+                                       const int32_t* slot, const int64_t* exclude, int32_t n_exclude,
+                                       int32_t max_attempts, int64_t* seed_used, int32_t* repetitions, int32_t* status,
+                                       void* stream);
+
 /* ======================================================================== */
 /* Routing environment (replaces src/env/routing.py:119-178, 187-235,        */
 /* 256-358, 360-539 for B independent env instances advanced in place)       */
