@@ -29,7 +29,7 @@ class GraphMarlError(RuntimeError):
 
 class RoutingDesc(C.Structure):
     _fields_ = [(n, C.c_int32) for n in ("B", "N", "A", "E", "T", "env_var", "k", "congestion",
-                                         "action_mask", "ttl", "state_stride", "node_sparse_static", "store_mode")] + \
+                                         "action_mask", "ttl", "state_stride", "node_sparse_static")] + \
                [(n, C.c_void_p) for n in ("node_edges", "node_nbrs", "edges", "apsp", "topo_index", "state")]
 
 

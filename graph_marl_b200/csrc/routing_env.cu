@@ -7,14 +7,12 @@
 // observation field is bit-identical to the Python reference), writes the record back,
 // and then builds the dense agent / node observations in a shared-memory staging tile
 // that is zero-filled, scattered with the few non-zero fields per row and pushed to HBM
-// either with 16-byte vector stores or with one cp.async.bulk (TMA bulk) store per tile.
+// with one cp.async.bulk (TMA bulk) store per tile.
 //
 // Reference semantics: src/env/routing.py:119-144 (reset_packet), :160-178 (reset),
 // :187-235 (node obs), :256-267 (node-agent matrix), :269-358 (agent obs), :360-520 (step),
 // :522-539 (agent adjacency).  SURVEY.md Appendix A is the distilled spec.
 #include "common.cuh"
-
-#include <stdlib.h>
 
 #include <algorithm>
 
@@ -46,13 +44,13 @@ static RoutingLayout make_layout(int N, int A, int E, int stage_bytes, int stage
 enum { MODE_RESET = 0, MODE_STEP = 1, MODE_OBSERVE = 2 };
 
 // -DGM_ROUTING_PROBES=1 (GM_NVCC_EXTRA): per-env SM-clock stamps at the phase boundaries of the step kernel, read back
-// with gm_routing_probe_read (tools/env_probe.py).  The default build contains none of this.
+// with gm_routing_probe_read (tools/env_only.py).  The default build contains none of this.
 #ifdef GM_ROUTING_PROBES
 constexpr int PROBE_ENVS = 16384, PROBE_N = 10;
 __device__ long long g_probe[PROBE_ENVS][PROBE_N];
 #define GM_PROBE(k)                                                                      \
     do {                                                                                 \
-        if (MODE == MODE_STEP && lane == 0 && b < PROBE_ENVS) g_probe[b][(k) + (role ? 0 : 0)] = clock64(); \
+        if (MODE == MODE_STEP && lane == 0 && b < PROBE_ENVS) g_probe[b][k] = clock64(); \
     } while (0)
 #else
 #define GM_PROBE(k) do {} while (0)
@@ -126,7 +124,7 @@ __device__ __forceinline__ void spawn_packet(const EnvView& v, const RoutingLayo
 // so that the interior of every tile moves as 16-byte units).
 template <class ScatterRows>
 __device__ __forceinline__ void emit_f32_block(float* g, int total, int W, float* stage, int stage_floats,
-                                               int lane, int store_mode, ScatterRows scatter_rows) {
+                                               int lane, ScatterRows scatter_rows) {
     int tile_cap = stage_floats - 4;
     for (int f0 = 0; f0 < total; f0 += tile_cap) {
         int nfl = min(tile_cap, total - f0);
@@ -148,27 +146,17 @@ __device__ __forceinline__ void emit_f32_block(float* g, int total, int W, float
         if (head > nfl) head = nfl;
         int body4 = (nfl - head) >> 2;
         int tail = nfl - head - 4 * body4;
-        if (store_mode == 2) {
-            asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-        }
+        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
         __syncwarp();
         if (lane < head) gt[lane] = s[lane];
         if (lane < tail) gt[head + 4 * body4 + lane] = s[head + 4 * body4 + lane];
-        if (body4 > 0) {
-            if (store_mode == 2) {
-                if (lane == 0) {
-                    uint32_t saddr = (uint32_t)__cvta_generic_to_shared(s + head);
-                    asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" ::"l"(gt + head),
-                                 "r"(saddr), "r"(body4 * 16)
-                                 : "memory");
-                    asm volatile("cp.async.bulk.commit_group;" ::: "memory");
-                    asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
-                }
-            } else {
-                const float4* s4 = (const float4*)(s + head);
-                float4* g4 = (float4*)(gt + head);
-                for (int q = lane; q < body4; q += 32) __stcs(g4 + q, s4[q]);
-            }
+        if (body4 > 0 && lane == 0) {
+            uint32_t saddr = (uint32_t)__cvta_generic_to_shared(s + head);
+            asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" ::"l"(gt + head),
+                         "r"(saddr), "r"(body4 * 16)
+                         : "memory");
+            asm volatile("cp.async.bulk.commit_group;" ::: "memory");
+            asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
         }
         __syncwarp();
     }
@@ -255,7 +243,7 @@ __device__ __noinline__ void emit_node_agent_rows(const int* now, int8_t* g, int
 // leave half of an SM's warp slots empty): the pair shares the env's shared-memory record; warp 0 advances it, then --
 // after a 64-thread named barrier -- emits the agent observations and adjacency while warp 1 builds the waiting-packet
 // sums, the node observations and the node-agent matrix (each warp has its own staging tile).
-// SIMPLE: the common configuration (env_var 1, staged bulk stores, no action mask, no evaluation extras) compiled
+// SIMPLE: the common configuration (env_var 1, no action mask, no evaluation extras) compiled
 // without the other variants' code: the general kernel is 5.4 K SASS instructions and 16 % of its stall samples were
 // instruction fetches (ncu, profiles/r2_env_step_ncu.md).
 template <int MODE, int WPE, bool SIMPLE>
@@ -547,7 +535,6 @@ routing_kernel(const gm_routing_desc d, const gm_routing_io io, const RoutingLay
     };
 
     float* stage = (float*)(sm + L.sm_stage + (WPE == 2 && role == 1 ? L.stage_floats * 4 + 32 : 0));
-    const int store_mode = SIMPLE ? 2 : d.store_mode;
 
     // waiting packets per node: count and fp64 size sum in packet-id order (routing.py:200-205); needed by
     // the node observations and by the GLOBAL agent observation
@@ -612,9 +599,9 @@ routing_kernel(const gm_routing_desc d, const gm_routing_io io, const RoutingLay
                               : make_int4(__float_as_int(x[0]), __float_as_int(x[1]), __float_as_int(x[2]), __float_as_int(x[3]));
         }
     };
-    // the GLOBAL agent observation embeds node rows and the direct store mode emits everything in one pass: both need the
-    // sums (and, to keep one code path, the record write-back) first
-    const bool early = !SIMPLE && (env_var == 3 || store_mode == 3);
+    // the GLOBAL agent observation embeds node rows: it needs the sums (and, to keep one code path, the record
+    // write-back) first
+    const bool early = !SIMPLE && env_var == 3;
     if (early) {
         if (role == 0) finish_record();
         if (need_wait) waiting_sums();
@@ -637,82 +624,13 @@ routing_kernel(const gm_routing_desc d, const gm_routing_io io, const RoutingLay
         }
     };
 
-    // ---- store mode 3 ("direct"): no staging tile.  The env's dense blocks are zero-filled in HBM with 16-byte
-    // stores, then every row's few non-zero fields are written over them by the lane that owns the row, which keeps
-    // the row's packet / node view in registers (one pass, no per-tile re-scan, no bounds checks, no wait on a bulk
-    // store).  __syncwarp() orders a lane's field stores after the other lanes' zero stores to the same sectors; L2
-    // merges both before anything reaches DRAM.  Used for env_var 1 when both blocks are 16-byte granular.
-    if (!SIMPLE && store_mode == 3) {
-        const float4 z4 = make_float4(0.f, 0.f, 0.f, 0.f);
-        const int W0 = 6 * N + 10, Wn = 4 * N + 8;
-        float* go = io.obs ? io.obs + (size_t)b * A * W0 : nullptr;
-        float* gn = io.node_obs ? io.node_obs + (size_t)b * N * Wn : nullptr;
-        if (go) {
-            float4* g4 = (float4*)go;
-            const int n4 = (A * W0) >> 2;
-#pragma unroll 4
-            for (int q = lane; q < n4; q += 32) g4[q] = z4;
-        }
-        if (gn) {
-            float4* g4 = (float4*)gn;
-            const int n4 = (N * Wn) >> 2;
-#pragma unroll 4
-            for (int q = lane; q < n4; q += 32) g4[q] = z4;
-        }
-        __syncwarp();
-        if (go) {
-            for (int i = lane; i < A; i += 32) {
-                float* r = go + (size_t)i * W0;
-                const int nw = v.now[i], e = v.edge[i];
-                r[nw] = 1.f;
-                r[N + v.target[i]] = 1.f;
-                if (e != -1) {
-                    const int4 ee = ed[e];
-                    r[2 * N] = 1.f;
-                    r[2 * N + 1 + ((ee.x == nw) ? ee.y : ee.x)] = 1.f;
-                }
-                r[3 * N + 1] = (float)v.time[i];
-                r[3 * N + 2] = (float)v.size[i];
-                r[3 * N + 3] = (float)i;
-#pragma unroll
-                for (int q = 0; q < 3; q++) {
-                    const int k = ne[nw * 3 + q], o = nb[nw * 3 + q];
-                    float* rb = r + 3 * N + 4 + q * (N + 2);
-                    rb[o] = 1.f;
-                    rb[N] = (float)ed[k].z;
-                    rb[N + 1] = (float)v.load[k];
-                }
-            }
-        }
-        if (gn) {
-            for (int j = lane; j < N; j += 32) {
-                float* r = gn + (size_t)j * Wn;
-                r[j] = 1.f;
-                r[N] = (float)v.cnt[j];
-                r[N + 1] = (float)v.tl[j];
-#pragma unroll
-                for (int q = 0; q < 3; q++) {
-                    const int k = ne[j * 3 + q], o = nb[j * 3 + q];
-                    float* rb = r + N + 2 + q * (N + 2);
-                    rb[o] = 1.f;
-                    rb[N] = (float)ed[k].z;
-                    rb[N + 1] = (float)v.load[k];
-                }
-            }
-        }
-        emit_node_sparse();
-        if (io.adj) emit_adj_rows(v.now, nb, io.adj + (size_t)b * A * A, N, A, lane);
-        if (io.node_agent) emit_node_agent_rows(v.now, io.node_agent + (size_t)b * N * A, N, A, lane);
-        return;
-    }
-
     // ---- agent observations (routing.py:277-358) ------------------------------------------
     // row = 6N+10 packet/edge fields | env_var 2: 5 fields of up to k neighbouring agents (:328-348)
     //                                | env_var 3: flattened node adjacency + node observations (:271-275,353-354)
     if (io.obs && do_agent) {
         const int W0 = 6 * N + 10;
         const int W = W0 + (env_var == 2 ? 5 * d.k : 0) + (env_var == 3 ? N * N + N * (4 * N + 8) : 0);
-        emit_f32_block(io.obs + (size_t)b * A * W, A * W, W, stage, L.stage_floats, lane, store_mode,
+        emit_f32_block(io.obs + (size_t)b * A * W, A * W, W, stage, L.stage_floats, lane,
                        [&](int r0, int r1, auto put) {
                            // four lanes per row (8 rows per pass): the ~16 fields of a row are written by four lanes
                            // side by side instead of one lane after the other (a tile holds 7-9 rows at N = 20)
@@ -779,7 +697,7 @@ routing_kernel(const gm_routing_desc d, const gm_routing_io io, const RoutingLay
     // ---- node observations (routing.py:193-234), row width 4N+8 ------------------------
     if (io.node_obs && do_node) {
         const int W = 4 * N + 8;
-        emit_f32_block(io.node_obs + (size_t)b * N * W, N * W, W, stage, L.stage_floats, lane, store_mode,
+        emit_f32_block(io.node_obs + (size_t)b * N * W, N * W, W, stage, L.stage_floats, lane,
                        [&](int r0, int r1, auto put) {
                            for (int j = r0 + (lane >> 2); j <= r1; j += 8) node_row(j, 0, j, lane & 3, put);
                        });
@@ -806,46 +724,24 @@ static int launch_routing(int mode, const gm_routing_desc* d, const gm_routing_i
     GM_CHECK_ARG(mode != MODE_STEP || io->actions, "step needs actions");
     GM_CHECK_ARG(io->info == nullptr || ((uintptr_t)io->info & 15) == 0, "info must be 16-byte aligned");
 
-    gm_routing_desc dd = *d;
-    static int store_env = -1;
-    if (store_env < 0) {
-        const char* e = getenv("GM_ROUTING_STORE_MODE");  // 1 staged + vector stores, 2 staged + bulk stores, 3 direct
-        store_env = e ? atoi(e) : 0;
-    }
-    // direct stores need env_var 1 and 16-byte granular per-env blocks (e.g. A = 35 is not: rows of 130 floats)
-    const bool direct_ok = d->env_var == 1 && (((int64_t)d->A * (6 * d->N + 10)) & 3) == 0 && (((int64_t)d->N * (4 * d->N + 8)) & 3) == 0 &&
-                           ((uintptr_t)io->obs & 15) == 0 && ((uintptr_t)io->node_obs & 15) == 0;
-    // default 2: the direct mode measured slower (37 vs 29 us per launch at config 2: its per-row field stores are 32
-    // different lines per warp instruction); kept as an option and parity-tested
-    if (dd.store_mode == 0) dd.store_mode = store_env ? store_env : 2;
-    if (dd.store_mode == 3 && !direct_ok) dd.store_mode = 2;
-
     // staging tile: 4 KiB per warp keeps >= 7 CTAs (28 warps) resident per SM, so 4096 envs run as ONE wave
     // (measured: 30.8 us vs 37.9 us with 16 KiB tiles; double-buffered tiles were slower, they halve residency)
     const int64_t W_obs = 6 * d->N + 10 + (d->env_var == 2 ? 5 * d->k : 0) + (d->env_var == 3 ? d->N * d->N + d->N * (4 * d->N + 8) : 0);
     int64_t need = 4ll * (int64_t)std::max((int64_t)d->A * W_obs, (int64_t)d->N * (4 * d->N + 8)) + 32;
-    static int stage_cap = -1;
-    if (stage_cap < 0) {
-        const char* e = getenv("GM_ROUTING_STAGE_BYTES");
-        stage_cap = e ? atoi(e) : 4096;
-        if (stage_cap < 1024 || stage_cap > 65536) stage_cap = 4096;
-    }
-    int stage_bytes = dd.store_mode == 3 ? 16 : (int)std::min<int64_t>(stage_cap, round_up(need, 256));  // direct mode stages nothing
+    int stage_bytes = (int)std::min<int64_t>(4096, round_up(need, 256));
     // the common configuration runs the specialised instance; batches that would leave at least half of the warp slots
-    // of every SM empty (2 B <= SMs x 28) give each env two warps
-    const bool simple = d->env_var == 1 && dd.store_mode == 2 && !d->action_mask && io->eval_f64 == nullptr &&
+    // of every SM empty (2 B <= SMs x 28) give each env two warps (inside the bench step: 23.0 vs 27.1 us per launch at
+    // cfg3's 2048 envs, 0.33 vs 0.42 ms at cfg4's 1024 envs against one warp per env)
+    const bool simple = d->env_var == 1 && !d->action_mask && io->eval_f64 == nullptr &&
                         io->sum_packets_per_node == nullptr && io->action_mask_out == nullptr;
-    static int wpe_env = -1, sms = 0;
-    if (wpe_env < 0) {
-        const char* e = getenv("GM_ROUTING_WPE");
-        wpe_env = e ? atoi(e) : 0;
+    static int sms = 0;
+    if (sms == 0) {
         int dev = 0;
         cudaGetDevice(&dev);
         cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
         if (sms <= 0) sms = kNumSMs;
     }
-    int wpe = (simple && 2ll * d->B <= (int64_t)sms * WARPS_PER_CTA * GM_ROUTING_MIN_CTAS) ? 2 : 1;
-    if (wpe_env == 1 || (wpe_env == 2 && simple)) wpe = wpe_env;
+    const int wpe = (simple && 2ll * d->B <= (int64_t)sms * WARPS_PER_CTA * GM_ROUTING_MIN_CTAS) ? 2 : 1;
     RoutingLayout L = make_layout(d->N, d->A, d->E, stage_bytes, wpe);
     GM_CHECK_ARG(d->state_stride == L.stride, "state_stride %d != %d", d->state_stride, L.stride);
     while (L.sm_per_warp * (WARPS_PER_CTA / wpe) > 200 * 1024 && stage_bytes > 2048) {
@@ -860,7 +756,7 @@ static int launch_routing(int mode, const gm_routing_desc* d, const gm_routing_i
 #define GM_ROUTING_LAUNCH(MODE_, WPE_, SIMPLE_)                                                                              \
     do {                                                                                                                     \
         GM_CUDA(cudaFuncSetAttribute(routing_kernel<MODE_, WPE_, SIMPLE_>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
-        routing_kernel<MODE_, WPE_, SIMPLE_><<<grid, block, smem, s>>>(dd, *io, L);                                          \
+        routing_kernel<MODE_, WPE_, SIMPLE_><<<grid, block, smem, s>>>(*d, *io, L);                                          \
     } while (0)
 #define GM_ROUTING_VARIANT(MODE_)                                 \
     do {                                                          \

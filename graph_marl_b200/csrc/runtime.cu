@@ -33,7 +33,7 @@ void set_error(const char* fmt, ...) {
 
 extern "C" {
 const char* gm_last_error(void) { return gm::g_err; }
-int gm_abi_version(void) { return 5; }
+int gm_abi_version(void) { return 6; }
 int64_t gm_kernel_launch_count(void) { return gm::g_launches.load(); }
 
 void gm_profile_enable(int on) { gm::g_profile = on != 0; }

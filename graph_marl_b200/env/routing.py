@@ -140,8 +140,7 @@ class Routing(NetworkEnv):
     """Packet routing on a random 3-regular graph (routing.py:43-552)."""
 
     def __init__(self, network: Network, n_data, env_var, k=3, enable_congestion=True,
-                 enable_action_mask=False, ttl=0, num_envs=1, device=None, seed=0, store_mode=0,
-                 batched=None):
+                 enable_action_mask=False, ttl=0, num_envs=1, device=None, seed=0, batched=None):
         super().__init__()
         assert isinstance(network, Network)
         self.network = network
@@ -167,7 +166,6 @@ class Routing(NetworkEnv):
         self.device = torch.device(device if device is not None else "cuda")
         self._seed = int(seed)
         self._calls = 0
-        self._store_mode = store_mode
         N, A = network.n_nodes, n_data
         self._N, self._A, self._E = N, A, 3 * N // 2
         lay = np.zeros(8, np.int32)
@@ -261,7 +259,7 @@ class Routing(NetworkEnv):
         d.B, d.N, d.A, d.E, d.T = self.num_envs, self._N, self._A, self._E, p.T
         d.env_var, d.k = self.env_var.value, self.k
         d.congestion, d.action_mask, d.ttl = int(self.enable_congestion), int(self.enable_action_mask), int(self.ttl)
-        d.state_stride, d.store_mode = self._layout["stride"], self._store_mode
+        d.state_stride = self._layout["stride"]
         d.node_sparse_static = 2 if p.static_rows is not None else 0
         d.node_edges, d.node_nbrs, d.edges, d.apsp = (p.node_edges.data_ptr(), p.node_nbrs.data_ptr(),
                                                       p.edges.data_ptr(), p.apsp.data_ptr())

@@ -41,7 +41,7 @@ typedef enum {
 
 GM_API const char* gm_last_error(void);
 /* ABI version, bumped on any signature/struct change. */
-GM_API int gm_abi_version(void);   /* currently 5 */
+GM_API int gm_abi_version(void);   /* currently 6 */
 /* 0 if a CUDA device with compute capability 10.x is present, else GM_ERR_NO_DEVICE. */
 GM_API int gm_device_check(void);
 
@@ -122,8 +122,6 @@ typedef struct gm_routing_desc {
                                     for the constant part of the row, then #waiting, size sum and the three edge loads;
                                     2: the same 6 entries as indices into a dictionary of T*N + 5 rows: topology*N + node,
                                     then T*N + 0..4 for #waiting, size sum and the three loads (static_only packs) */
-    int32_t store_mode;          /* 0 auto, 1 smem staging + vector stores, 2 smem staging + cp.async.bulk,
-                                    3 direct: zero-fill + per-row field stores (env_var 1, 16-byte granular blocks) */
     /* topology pool (device, int32) */
     const int32_t* node_edges;   /* [T,N,3] edge ids of node n sorted by neighbour id */
     const int32_t* node_nbrs;    /* [T,N,3] the neighbour reached by action 1..3 */

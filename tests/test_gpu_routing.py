@@ -14,14 +14,13 @@ CASES = ["routing_A_seed923430603_cong", "routing_B_nocong", "routing_C_mask", "
          "routing_E_a35_nocong_mask_ttl", "routing_F_n200", "routing_G_var2", "routing_H_var3", "routing_I_evalinfo"]
 
 
-def _make_env(g, c, num_envs=1, store_mode=0, batched=None):
+def _make_env(g, c, num_envs=1, batched=None):
     from graph_marl_b200.env.network import Network
     from graph_marl_b200.env.routing import Routing
 
     net = Network(c["n_nodes"], random_topology=False, topology_init_seed=c["topo_seed"])
     return Routing(net, c["n_data"], c["env_var"], k=c["k"], enable_congestion=c["congestion"],
-                   enable_action_mask=c["mask"], ttl=c["ttl"], num_envs=num_envs, store_mode=store_mode,
-                   batched=batched)
+                   enable_action_mask=c["mask"], ttl=c["ttl"], num_envs=num_envs, batched=batched)
 
 
 def _check_state(env, g, t):
@@ -30,13 +29,12 @@ def _check_state(env, g, t):
         assert np.array_equal(s[k][0], g["s_" + k][t]), (k, t)
 
 
-@pytest.mark.parametrize("store_mode", [1, 2, 3])
 @pytest.mark.parametrize("case", CASES)
-def test_golden_trajectory(case, store_mode):
+def test_golden_trajectory(case):
     g = load_golden(case)
     c = cfg_from_golden(g)
     A = c["n_data"]
-    env = _make_env(g, c, store_mode=store_mode)
+    env = _make_env(g, c)
     env.set_eval_info(c["eval_info"])
     ds, dt, dz, n = draws_for_step(g, -1, A)
     env.set_draws(ds, dt, dz)

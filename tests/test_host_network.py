@@ -25,7 +25,7 @@ def test_library_exports_every_declared_symbol():
     L = _lib.lib()
     for name in declared:
         assert hasattr(L, name), name
-    assert L.gm_abi_version() == 5
+    assert L.gm_abi_version() == 6
 
 
 def test_native_mt19937_matches_numpy_legacy_stream():

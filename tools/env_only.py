@@ -37,7 +37,7 @@ for i in range(iters):
 ts.sort()
 med = ts[len(ts) // 2]
 by = env_step_bytes(N, A, sparse_rows=env._out.get("node_sparse") is not None) * B
-print(f"B={B} store_mode={os.environ.get('GM_ROUTING_STORE_MODE', 'default')} median {med:.2f} us  min {ts[0]:.2f} us  "
+print(f"B={B} median {med:.2f} us  min {ts[0]:.2f} us  "
       f"roofline frac (median) {by / (med * 1e-6) / 1e9 / peaks()['hbm_gbs']:.3f}")
 
 try:  # probe build (-DGM_ROUTING_PROBES=1): mean SM clocks between the phase boundaries of the last launch
@@ -52,13 +52,10 @@ try:  # probe build (-DGM_ROUTING_PROBES=1): mean SM clocks between the phase bo
     out = np.zeros((n, 10), np.int64)
     fn.argtypes, fn.restype = [C.c_void_p, C.c_int], C.c_int
     assert fn(out.ctypes.data, n) == 0
-    names = ["load record", "loop 1", "loop 2 + outputs", "write-back", "(pair barrier) + waiting sums", "agent obs tiles",
-             "node obs tiles"]
     t = out - out[:, :1]
-    wpe2 = bool((out[:, 9] != out[:, 8]).any()) and False
     print("phase ends (mean SM clocks since the warp started):")
-    for k, nm in zip(range(1, 8), ["record loaded", "loop 1 done", "loop 2 done", "record written back", "waiting sums done",
-                                   "agent obs emitted", "node obs emitted"]):
+    for k, nm in zip(range(1, 8), ["record loaded", "loop 1 done", "loop 2 done", "agent obs emitted", "record written back",
+                                   "waiting sums done", "node obs emitted"]):
         print(f"  {nm:24s} {t[:, k].mean():9.0f}   (+{(t[:, k] - t[:, k - 1]).mean():8.0f})")
     print(f"  {'adj / node-agent done':24s} {max(t[:, 8].mean(), t[:, 9].mean()):9.0f}")
     print(f"  warp start spread: {(out[:, 0].max() - out[:, 0].min())} clocks; last end - first start: {out[:, 8:].max() - out[:, 0].min()} clocks")
