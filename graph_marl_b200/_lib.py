@@ -132,6 +132,8 @@ _SIGS = {
     "gm_mt_random": (C.c_double, [C.c_void_p]),
     "gm_mt_randint": (C.c_uint32, [C.c_void_p, C.c_uint32]),
     "gm_mt_packet_draws": (None, [C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "gm_mt_reset_draws": (C.c_int, [C.c_void_p, C.c_int32, C.c_void_p, C.c_int32, C.c_void_p, C.c_int32, C.c_int32,
+                                    C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "gm_mt_policy_draws": (None, [C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p]),
     "gm_topology_generate": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.c_int64, C.c_void_p, C.c_int32,
                                        C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
@@ -139,6 +141,7 @@ _SIGS = {
     "gm_topology_apsp": (C.c_int, [C.c_int32, C.c_int32, C.c_void_p, C.c_void_p]),
     "gm_topology_generate_device": (C.c_int, [C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32,
                                               C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "gm_topology_next_hops": (C.c_int, [C.c_void_p, C.c_int32, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p]),
     "gm_routing_state_layout": (C.c_int, [C.c_int32, C.c_int32, C.c_int32, C.c_void_p]),
     "gm_routing_reset": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p]),
     "gm_routing_step": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p]),

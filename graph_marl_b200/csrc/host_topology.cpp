@@ -175,6 +175,37 @@ void gm_mt_packet_draws(uint32_t* state, int32_t n_nodes, int32_t n, int32_t* st
     }
 }
 
+int gm_mt_reset_draws(uint32_t* state, int32_t seed_mode, const int64_t* seed_list, int32_t n_seeds,
+                      const int64_t* exclude, int32_t n_exclude, int32_t n_nodes, int32_t S, int32_t A, int64_t* seeds,
+                      int32_t* start, int32_t* target, double* size) {
+    GM_CHECK_ARG(state && S >= 0 && A >= 0 && n_nodes > 0 && (S == 0 || seeds), "bad reset-draw arguments");
+    GM_CHECK_ARG(A == 0 || S == 0 || (start && target && size), "null packet-draw output");
+    GM_CHECK_ARG(seed_mode >= 0 && seed_mode <= 2, "seed_mode must be 0, 1 or 2, got %d", seed_mode);
+    GM_CHECK_ARG(seed_mode == 0 || (seed_list && n_seeds > 0), "seed_mode %d needs a seed list", seed_mode);
+    GM_CHECK_ARG(n_exclude >= 0 && (n_exclude == 0 || exclude), "bad exclusion list");
+    std::vector<int64_t> ex(exclude, exclude + n_exclude);
+    std::sort(ex.begin(), ex.end());
+    LegacyMT r(state);
+    for (int s = 0; s < S; ++s) {
+        if (seed_mode == 0) {  // pick_seed without a seed list: randint(2**31 - 1), redrawn on excluded seeds
+            int64_t v;
+            do v = r.below(2147483647u); while (std::binary_search(ex.begin(), ex.end(), v));
+            seeds[s] = v;
+        } else if (seed_mode == 1) {  // the sample's seed is given: no draw
+            seeds[s] = seed_list[s];
+        } else {  // np.random.choice(seed_list): randint(len); a one-seed list draws nothing
+            seeds[s] = seed_list[r.below((uint32_t)n_seeds)];
+        }
+        const size_t o = (size_t)s * A;
+        for (int i = 0; i < A; ++i) {  // routing.py:130-135
+            start[o + i] = (int32_t)r.below((uint32_t)n_nodes);
+            target[o + i] = (int32_t)r.below((uint32_t)n_nodes);
+            size[o + i] = r.uniform();
+        }
+    }
+    return GM_OK;
+}
+
 void gm_mt_policy_draws(uint32_t* state, int32_t n_actions, int32_t n, int32_t* rand_action, double* rand_u) {
     LegacyMT r(state);
     for (int i = 0; i < n; ++i) rand_action[i] = (int32_t)r.below((uint32_t)n_actions);

@@ -1,5 +1,6 @@
 // topology.cu -- the random 3-regular geometric graph generator of host_topology.cpp (network.py:122-272) for B envs in
-// one launch, writing each topology straight into a slot of the device topology pool (gm_topology_generate_device).
+// one launch, writing each topology straight into a slot of the device topology pool (gm_topology_generate_device), and
+// the pool's next-hop tables in networkx's tie-breaking order (gm_topology_next_hops, further down).
 //
 // One warp per env.  Lane 0 runs everything that is sequential in the reference -- the env's private legacy MT19937
 // stream (shared memory), the node positions, the edge rule, the validity check and the reseed loop -- and the warp
@@ -251,8 +252,113 @@ __global__ void __launch_bounds__(kTopoMaxWarps * 32) topology_generate_kernel(
     }
 }
 
+// ---- next-hop tables: networkx's single-source Dijkstra paths, tie for tie ----
+//
+// nx.shortest_path(G, weight=...) runs _dijkstra_multisource from every source: neighbours in G._adj order (edge
+// creation order, the order G.add_edge inserted them), a heap popped by (distance, push counter), a push and
+// pred[u] = [v] only on a strictly shorter distance, and paths[u] = paths[pred[u][0]] + [u].  The entry popped next is
+// always the current entry of an unsettled node -- an older entry of a node has a larger distance than its current one
+// -- so keeping one (distance, counter) per node and taking the warp arg-min over the unsettled nodes pops in the heap's
+// order without a heap.  The first hop of u is u itself when its predecessor is the source and its predecessor's first
+// hop otherwise; a settled node's predecessor no longer changes, so it is final when u is relaxed from it.
+constexpr int kHopWarps = 8;
+constexpr int kHopSmemBudget = 48 * 1024;
+constexpr int kHopUnseen = 0x7fffffff;
+
+__global__ void __launch_bounds__(kHopWarps * 32) topology_next_hops_kernel(gm_topology_tables t, int n,
+                                                                          const int32_t* __restrict__ slots,
+                                                                          int8_t* __restrict__ next_hop) {
+    extern __shared__ __align__(16) int hop_smem[];
+    const int N = t.N, E = 3 * N / 2;
+    const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+    const int64_t g = (int64_t)blockIdx.x * (blockDim.x >> 5) + w;  // (listed slot, source) pair of this warp
+    if (g >= (int64_t)n * N) return;  // whole warps leave together
+    const int i = (int)(g / N), src = (int)(g - (int64_t)i * N);
+    const int s = slots[i];
+    int8_t* out = next_hop + ((size_t)i * N + src) * N;
+    if (s < 0 || s >= t.P) {  // a slot outside the pool: the row is marked, nothing is read
+        for (int v = lane; v < N; v += 32) out[v] = -1;
+        return;
+    }
+    int* dist = hop_smem + (size_t)w * 3 * N;  // tentative or final distance; kHopUnseen before the first push
+    int* cnt = dist + N;                       // push counter of the current entry; -1 once settled
+    int* hop = cnt + N;                        // first hop of the current predecessor's path
+    for (int v = lane; v < N; v += 32) dist[v] = kHopUnseen, cnt[v] = 0, hop[v] = -1;
+    __syncwarp();
+    if (lane == 0) dist[src] = 0;
+    __syncwarp();
+    const int32_t* node_edges = t.node_edges + (size_t)s * N * 3;
+    const int32_t* edges = t.edges + (size_t)s * E * 4;
+    int counter = 1;  // the source's entry took counter 0
+    for (;;) {
+        // pop: the unsettled node of least (distance, counter)
+        int bd = kHopUnseen, bc = 0x7fffffff, bv = -1;
+        for (int v = lane; v < N; v += 32) {
+            const int d = dist[v], c = cnt[v];
+            if (c >= 0 && d != kHopUnseen && (d < bd || (d == bd && c < bc))) bd = d, bc = c, bv = v;
+        }
+#pragma unroll
+        for (int o = 16; o; o >>= 1) {
+            const int od = __shfl_xor_sync(FULL, bd, o), oc = __shfl_xor_sync(FULL, bc, o), ov = __shfl_xor_sync(FULL, bv, o);
+            if (od < bd || (od == bd && oc < bc)) bd = od, bc = oc, bv = ov;
+        }
+        if (bv < 0) break;
+        const int v = bv;
+        // relax v's three edges in creation (edge id) order: lane q takes the q-th smallest incident edge id
+        bool improve = false;
+        int u = 0, nd = 0;
+        if (lane < 3) {
+            const int e0 = node_edges[3 * v], e1 = node_edges[3 * v + 1], e2 = node_edges[3 * v + 2];
+            const int lo = min(e0, min(e1, e2)), hi = max(e0, max(e1, e2));
+            const int e = lane == 0 ? lo : lane == 2 ? hi : e0 + e1 + e2 - lo - hi;
+            const int a = edges[4 * e], b = edges[4 * e + 1];
+            u = a == v ? b : a;
+            nd = bd + edges[4 * e + 2];
+            improve = cnt[u] >= 0 && nd < dist[u];  // (u == v, the self-loop of two coincident nodes, never improves)
+        }
+        const unsigned mask = __ballot_sync(FULL, improve);
+        __syncwarp();
+        if (lane == 0) cnt[v] = -1;  // settled
+        if (improve) {
+            dist[u] = nd;
+            cnt[u] = counter + __popc(mask & ((1u << lane) - 1));
+            hop[u] = v == src ? u : hop[v];
+        }
+        counter += __popc(mask);
+        __syncwarp();
+    }
+    // the entry of (src, t): 1 + the index in node_edges[src] of the edge towards hop[t]
+    const int32_t* nb = t.node_nbrs + ((size_t)s * N + src) * 3;
+    const int n0 = nb[0], n1 = nb[1], n2 = nb[2];
+    for (int v = lane; v < N; v += 32) {
+        const int h = hop[v];
+        out[v] = (int8_t)(v == src || h < 0 ? 0 : h == n0 ? 1 : h == n1 ? 2 : h == n2 ? 3 : 0);
+    }
+}
+
 }  // namespace
 }  // namespace gm
+
+extern "C" int gm_topology_next_hops(const gm_topology_tables* tables, int32_t P, const int32_t* slots, int32_t n,
+                                     int8_t* next_hop, void* stream) {
+    using namespace gm;
+    GM_CHECK_ARG(tables, "null topology tables");
+    gm_topology_tables t = *tables;
+    GM_CHECK_ARG(t.N >= 4 && t.N % 2 == 0 && t.N <= GM_TOPOLOGY_MAX_NODES,
+                 "n_nodes must be even and in [4, %d] for the next-hop tables, got %d", GM_TOPOLOGY_MAX_NODES, t.N);
+    GM_CHECK_ARG(P > 0 && P <= t.P && t.edges && t.node_edges && t.node_nbrs, "bad topology tables");
+    GM_CHECK_ARG(n >= 0 && (n == 0 || (slots && next_hop)), "bad next-hop arguments");
+    if (n == 0) return GM_OK;
+    t.P = P;
+    const int per_warp = 3 * t.N * (int)sizeof(int);
+    const int warps = std::min(kHopWarps, kHopSmemBudget / per_warp);
+    const int64_t blocks = ((int64_t)n * t.N + warps - 1) / warps;
+    GM_CHECK_ARG(blocks < (int64_t)1 << 31, "too many next-hop tables in one launch: %d", n);
+    topology_next_hops_kernel<<<(unsigned)blocks, warps * 32, (size_t)warps * per_warp,
+                                (cudaStream_t)stream>>>(t, n, slots, next_hop);
+    GM_LAUNCH_CHECK();
+    return GM_OK;
+}
 
 extern "C" int gm_topology_generate_device(const gm_topology_tables* tables, int32_t B, const int64_t* seeds,
                                            const int32_t* slot, const int64_t* exclude, int32_t n_exclude,

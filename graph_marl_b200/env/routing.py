@@ -124,6 +124,8 @@ class TopologyPool:
         if st < 0:
             raise _lib.GraphMarlError(f"env {-st - 1}: topology slot outside the pool's {self.T} slots")
         sl = slot.long()
+        if getattr(self, "_next_hop", None) is not None:
+            self._next_hop[sl] = self.next_hops(slot)
         if getattr(self, "apsp_f32", None) is not None:
             self.apsp_f32[sl] = self.apsp[sl].float()
         if getattr(self, "node_adj", None) is not None:
@@ -134,6 +136,30 @@ class TopologyPool:
         for s_, u in zip(slot.cpu().tolist(), used.tolist()):
             self.seeds[s_] = u
         return used, reps
+
+    def next_hops(self, slot):
+        """Next-hop tables of the slots slot[i] (device int32 [n]) as int8 [n, N, N] (gm_topology_next_hops): entry
+        [i, v, t] is 0 for v == t, else 1 + the index in nodes[v].edges of the edge towards the first hop of
+        Network.shortest_paths[v][t] -- networkx's path, ties included."""
+        _lib.require_device()
+        dev, N, n = self.apsp.device, self.apsp.shape[-1], slot.numel()
+        out = torch.empty((n, N, N), dtype=torch.int8, device=dev)
+        t = _lib.TopologyTables(P=self.T, N=N, edges=self.edges.data_ptr(), node_edges=self.node_edges.data_ptr(),
+                                node_nbrs=self.node_nbrs.data_ptr(), apsp=self.apsp.data_ptr(), nbr_all=self.nbr_all.data_ptr(),
+                                deg=self.deg.data_ptr())
+        slot = slot.to(device=dev, dtype=torch.int32).contiguous()
+        with torch.cuda.device(dev):
+            _lib.check(_lib.lib().gm_topology_next_hops(C.byref(t), self.T, slot.data_ptr(), n, out.data_ptr(),
+                                                        _lib.current_stream()))
+        return out
+
+    @property
+    def next_hop(self):
+        """int8 [T, N, N] next-hop tables of every slot (next_hops), built on first use; generate() refreshes the
+        regenerated slots once it exists."""
+        if getattr(self, "_next_hop", None) is None:
+            self._next_hop = self.next_hops(torch.arange(self.T, dtype=torch.int32, device=self.apsp.device))
+        return self._next_hop
 
 
 class Routing(NetworkEnv):
@@ -385,6 +411,16 @@ class Routing(NetworkEnv):
     def reset(self):
         _lib.require_device()
         self._new_topologies()
+        return self._reset_envs()
+
+    def reset_on_pool(self, pool: TopologyPool, topo_index):
+        """reset() onto topologies already in `pool`: env b starts on slot topo_index[b] (device int32 [B]).  The
+        Network is neither reset nor read, so no topology seed is drawn; packets come from set_draws() as in reset()."""
+        _lib.require_device()
+        self.set_topology_pool(pool, topo_index)
+        return self._reset_envs()
+
+    def _reset_envs(self):
         B = self.num_envs
         if self._state is None:
             self._state = torch.zeros((B, self._layout["stride"]), dtype=torch.uint8, device=self.device)

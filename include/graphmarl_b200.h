@@ -60,6 +60,15 @@ GM_API uint32_t gm_mt_randint(uint32_t* state, uint32_t high);           /* np.r
  * (randint(N), randint(N), random()) in that order. */
 GM_API void gm_mt_packet_draws(uint32_t* state, int32_t n_nodes, int32_t n, int32_t* start,
                         int32_t* target, double* size);
+/* S sequential compat Routing.reset() calls (Network.reset()'s seed choice, then A packet triples as above) on the
+ * caller's stream, which is left where the S-th call leaves it.  seed_mode 0: pick_seed without a seed list,
+ * randint(2**31 - 1) redrawn while it is in exclude[n_exclude]; 1: the sample's seed is seed_list[s] (n_seeds >= S:
+ * sequential provided seeds, no draw); 2: np.random.choice(seed_list[n_seeds]), one randint(n_seeds), none when
+ * n_seeds == 1.  Outputs (host): seeds[S], start/target/size[S*A].  The topology generator draws from a private stream,
+ * so nothing else is consumed. */
+GM_API int gm_mt_reset_draws(uint32_t* state, int32_t seed_mode, const int64_t* seed_list, int32_t n_seeds,
+                             const int64_t* exclude, int32_t n_exclude, int32_t n_nodes, int32_t S, int32_t A,
+                             int64_t* seeds, int32_t* start, int32_t* target, double* size);
 /* policy draws of EpsilonGreedy.__call__ (policy.py:46-47): randint(n_act,size=n) then rand(n) */
 GM_API void gm_mt_policy_draws(uint32_t* state, int32_t n_actions, int32_t n, int32_t* rand_action,
                         double* rand_u);
@@ -104,6 +113,13 @@ GM_API int gm_topology_generate_device(const gm_topology_tables* tables, int32_t
                                        const int32_t* slot, const int64_t* exclude, int32_t n_exclude,
                                        int32_t max_attempts, int64_t* seed_used, int32_t* repetitions, int32_t* status,
                                        void* stream);
+/* Next-hop tables of the pool slots slots[0..n) (device i32[n]) into next_hop (device i8[n,N,N]): next_hop[i,v,t] is 0
+ * for v == t, else 1 + the index in node_edges[v] of the edge that carries the first hop of nx.shortest_path(G)[v][t] --
+ * networkx's Dijkstra with its tie-breaking (neighbours in edge creation order, pops by (distance, push counter), a
+ * predecessor only on a strictly shorter distance).  A slot outside [0, P) (P <= tables->P) gets rows of -1.  One warp
+ * per (slot, source), 4 <= N <= GM_TOPOLOGY_MAX_NODES.  Asynchronous on `stream`. */
+GM_API int gm_topology_next_hops(const gm_topology_tables* tables, int32_t P, const int32_t* slots, int32_t n,
+                                 int8_t* next_hop, void* stream);
 
 /* ======================================================================== */
 /* Routing environment (replaces src/env/routing.py:119-178, 187-235,        */
