@@ -174,6 +174,8 @@ _SIGS = {
                                                  C.c_void_p]),
     "gm_td_grad": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, C.c_float,
                              C.c_float, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "gm_sl_mse_grad": (C.c_int, [C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_float, C.c_void_p,
+                                 C.c_void_p, C.c_void_p, C.c_void_p]),
     "gm_optimizer_step": (C.c_int, [C.c_void_p, C.c_int32, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p,
                                     C.c_void_p]),
     "gm_mlp_tape_floats": (C.c_int64, [C.c_void_p, C.c_int64]),

@@ -1,11 +1,14 @@
-// learner.cu -- the two device pieces of the batched DQN learner's update (graph_marl_b200/learner.py):
+// learner.cu -- the device pieces of the batched DQN learner's update (graph_marl_b200/learner.py) and of sl.py's
+// supervised update (graph_marl_b200/sl_trainer.py):
 //
 //   gm_td_grad         one-step TD error of tools/train_simple.py:107-110 (the reference's main.py learner):
 //                      y = r + (!done) * gamma * max_a q_next,  loss += scale * sum (q[a] - y)^2,  dq = 2 scale (q - y) at a
+//   gm_sl_mse_grad     sl.py:395-400's MSE of the all-pairs prediction against the shortest-path weights:
+//                      loss += scale * sum (pred - y)^2,  d_pred = 2 scale (pred - y)
 //   gm_optimizer_step  clip_grad_value_ + clip_grad_norm_ + AdamW(foreach=False) + interpolate_model (main.py:1007-1020)
 //
-// Both reduce with fixed-order partials (no float atomics), so a replayed CUDA graph computes what an eager call computes,
-// bit for bit, and both keep their scalars (loss, step count) in device memory, so the launches can be captured.
+// All three reduce with fixed-order partials (no float atomics), so a replayed CUDA graph computes what an eager call computes,
+// bit for bit, and they keep their scalars (loss, step count) in device memory, so the launches can be captured.
 #include <math.h>
 
 #include <algorithm>
@@ -60,6 +63,40 @@ __global__ void __launch_bounds__(kRedThreads) td_grad_kernel(const float* __res
     }
     const double s = block_sum(acc, sh);
     if (threadIdx.x == 0) partials[blockIdx.x] = s;
+}
+
+// sl.py's all-pairs distance loss (sl.py:395-400): row b*N + v of pred against targets_all[index[b], v, :], the targets
+// read from the dataset through the sample index (no gathered target batch).  One thread per (row, column) element, so
+// a warp reads consecutive columns of a prediction row and of a target row.  The element's (b, v, u) advance by the
+// grid stride's digits in base N, so the loop divides nothing (a 64-bit division is a call that spills).
+__global__ void __launch_bounds__(kRedThreads) sl_mse_grad_kernel(const float* __restrict__ pred, int64_t ldp,
+                                                                   const int32_t* __restrict__ targets_all,
+                                                                   const int64_t* __restrict__ index, int64_t total, int N,
+                                                                   float scale, float* __restrict__ d_pred,
+                                                                   double* __restrict__ partials) {
+    __shared__ double sh[kRedThreads / 32];
+    double acc = 0.0;
+    const float g2 = __fmul_rn(2.f, scale);
+    const int start = blockIdx.x * blockDim.x + threadIdx.x, stride = gridDim.x * blockDim.x;  // < 2^31: grid <= partials
+    int u = start % N, v = (start / N) % N;
+    int64_t b = start / N / N;
+    const int du = stride % N, dv = (stride / N) % N, db = stride / N / N;
+    for (int64_t i = start; i < total; i += stride) {
+        const int64_t r = b * N + v;  // prediction row
+        const int64_t s = index ? index[b] : b;
+        const float y = (float)targets_all[(s * N + v) * N + u];
+        const float d = __fsub_rn(pred[r * ldp + u], y);
+        acc += (double)d * (double)d;
+        if (d_pred) d_pred[r * ldp + u] = __fmul_rn(g2, d);
+        u += du;
+        int carry = 0;
+        if (u >= N) u -= N, carry = 1;
+        v += dv + carry;
+        if (v >= N) v -= N, b++;
+        b += db;
+    }
+    const double t = block_sum(acc, sh);
+    if (threadIdx.x == 0) partials[blockIdx.x] = t;
 }
 
 __global__ void td_loss_kernel(const double* __restrict__ partials, int n, double scale, float* __restrict__ loss) {
@@ -159,6 +196,21 @@ int gm_td_grad(const float* q, const float* q_next, const int64_t* action, const
     const int blocks = (int)std::min<int64_t>((rows + kRedThreads - 1) / kRedThreads, kTdMaxBlocks);
     td_grad_kernel<<<blocks, kRedThreads, 0, (cudaStream_t)stream>>>(q, q_next, action, reward, done, rows, n_actions, gamma,
                                                                      scale, dq, partials);
+    GM_LAUNCH_CHECK();
+    td_loss_kernel<<<1, 32, 0, (cudaStream_t)stream>>>(partials, blocks, (double)scale, loss);
+    GM_LAUNCH_CHECK();
+    return GM_OK;
+}
+
+int gm_sl_mse_grad(const float* pred, int64_t ldp, const int32_t* targets_all, const int64_t* index, int32_t B, int32_t N,
+                   float scale, float* d_pred, float* loss, double* partials, void* stream) {
+    GM_CHECK_ARG(pred && targets_all && loss && partials, "gm_sl_mse_grad: null pointer");
+    GM_CHECK_ARG(B >= 1 && N >= 1 && ldp >= N, "gm_sl_mse_grad: %d samples x %d nodes, row stride %lld", B, N,
+                 (long long)ldp);
+    const int64_t total = (int64_t)B * N * N;
+    const int blocks = (int)std::min<int64_t>((total + kRedThreads - 1) / kRedThreads, kTdMaxBlocks);
+    sl_mse_grad_kernel<<<blocks, kRedThreads, 0, (cudaStream_t)stream>>>(pred, ldp, targets_all, index, total, N, scale,
+                                                                         d_pred, partials);
     GM_LAUNCH_CHECK();
     td_loss_kernel<<<1, 32, 0, (cudaStream_t)stream>>>(partials, blocks, (double)scale, loss);
     GM_LAUNCH_CHECK();

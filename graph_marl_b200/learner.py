@@ -15,6 +15,18 @@ from . import _lib
 from .model import _NetMonStepFn
 
 
+def netmon_step_params(nm):
+    """NetMon's parameters in the order _NetMonStepFn takes them: encoder (weight, bias) pairs, then each cell's."""
+    ps = [t for l in nm.encode.linear_layers for t in (l.weight, l.bias)]
+    for cell in (nm.rnn_obs, nm.rnn_update):
+        for path, _ in nm._cell_param_names():
+            obj = cell
+            for part in path.split("."):
+                obj = getattr(obj, part)
+            ps.append(obj)
+    return ps
+
+
 class Learner:
     def __init__(self, netmon, model, lr, gamma, tau, clip_value=0.5, max_norm=1.0, graph=True):
         """netmon / model: the online NetMon and DQN (their parameters are updated in place); the target DQN is a deepcopy
@@ -53,15 +65,7 @@ class Learner:
         return dq.view(q.shape)
 
     def _netmon_params(self):
-        nm = self.netmon
-        ps = [t for l in nm.encode.linear_layers for t in (l.weight, l.bias)]
-        for cell in (nm.rnn_obs, nm.rnn_update):
-            for path, _ in nm._cell_param_names():
-                obj = cell
-                for part in path.split("."):
-                    obj = getattr(obj, part)
-                ps.append(obj)
-        return ps
+        return netmon_step_params(self.netmon)
 
     def _new_workspaces(self):
         return type(self.netmon._ws)(), type(self.target._ws)()

@@ -493,6 +493,11 @@ GM_API int gm_broadcast_weights(void* comm, float* flat, int64_t n, int32_t root
 GM_API int gm_td_grad(const float* q, const float* q_next, const int64_t* action, const float* reward, const uint8_t* done,
                int64_t rows, int32_t n_actions, float gamma, float scale, float* dq, float* loss, double* partials,
                void* stream);
+/* sl.py:395-400 (NetMonSL's all-pairs loss): pred f32[B*N, N] (row stride ldp), targets_all i32[S, N, N], index i64[B]
+ * (NULL: sample b = row block b): y = (float)targets_all[index[b], v, u] for row b*N+v, column u;
+ * d_pred (may be NULL: evaluation) = 2 * scale * (pred - y);  *loss (device f32) += scale * sum (pred - y)^2 */
+GM_API int gm_sl_mse_grad(const float* pred, int64_t ldp, const int32_t* targets_all, const int64_t* index,
+                          int32_t B, int32_t N, float scale, float* d_pred, float* loss, double* partials, void* stream);
 typedef struct gm_opt_entry {           /* one optimised tensor (device pointers) */
     float *param, *grad, *exp_avg, *exp_avg_sq;
     int64_t numel;
