@@ -20,6 +20,7 @@
 #include "common.cuh"
 #include "gemm_sm100.cuh"
 #include "linear_simt.cuh"
+#include "netmon_rows.cuh"
 
 namespace gm {
 
@@ -409,8 +410,7 @@ __global__ void __launch_bounds__(256) split_pk_kernel(const float* __restrict__
 // ---------------------------------------------------------------------------------------
 __global__ void lstm_pointwise_kernel(const float* __restrict__ gates, const float* __restrict__ c_in, int64_t ldc_in,
                                       float* __restrict__ h_out, int64_t ldh_out, float* __restrict__ c_out,
-                                      int64_t ldc_out, float* __restrict__ h_out2, int64_t ldh_out2,
-                                      float* __restrict__ c_out2, int64_t ldc_out2, int64_t R, int H) {
+                                      int64_t ldc_out, int64_t R, int H) {
     int64_t idx = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (idx >= R * H) return;
     int64_t r = idx / H;
@@ -421,25 +421,15 @@ __global__ void lstm_pointwise_kernel(const float* __restrict__ gates, const flo
     float hh = o_ * tanhf(c);
     h_out[r * ldh_out + j] = hh;
     c_out[r * ldc_out + j] = c;
-    if (h_out2) h_out2[r * ldh_out2 + j] = hh;
-    if (c_out2) c_out2[r * ldc_out2 + j] = c;
 }
 
 // ---------------------------------------------------------------------------------------
 // LayerNormLSTM pointwise (layernormlstm.py:28-42): one warp per row.
 //   gates = LN(gi) + LN(gh) + b_ih ; c' = LN(sig(f)*c + sig(i)*tanh(g)) ; h' = sig(o)*tanh(c')
 // ---------------------------------------------------------------------------------------
-__device__ inline float warp_sum(float x) {
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) x += __shfl_xor_sync(FULL, x, o);
-    return x;
-}
-
 __global__ void lnlstm_pointwise_kernel(const float* __restrict__ gi, const float* __restrict__ gh, gm_cell_params cp,
                                         const float* __restrict__ c_in, int64_t ldc_in, float* __restrict__ h_out,
-                                        int64_t ldh_out, float* __restrict__ c_out, int64_t ldc_out,
-                                        float* __restrict__ h_out2, int64_t ldh_out2, float* __restrict__ c_out2,
-                                        int64_t ldc_out2, int64_t R, int H) {
+                                        int64_t ldh_out, float* __restrict__ c_out, int64_t ldc_out, int64_t R, int H) {
     int64_t r = (int64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
     int lane = threadIdx.x & 31;
     if (r >= R) return;
@@ -481,15 +471,13 @@ __global__ void lnlstm_pointwise_kernel(const float* __restrict__ gi, const floa
         float hh = og[nj] * tanhf(c);
         h_out[r * ldh_out + j] = hh;
         c_out[r * ldc_out + j] = c;
-        if (h_out2) h_out2[r * ldh_out2 + j] = hh;
-        if (c_out2) c_out2[r * ldc_out2 + j] = c;
     }
 }
 
 // GRU pointwise (torch.nn.GRUCell; gate order r,z,n)
 __global__ void gru_pointwise_kernel(const float* __restrict__ gi, const float* __restrict__ gh,
                                      const float* __restrict__ h_in, int64_t ldh_in, float* __restrict__ h_out,
-                                     int64_t ldh_out, float* __restrict__ h_out2, int64_t ldh_out2, int64_t R, int H) {
+                                     int64_t ldh_out, int64_t R, int H) {
     int64_t idx = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (idx >= R * H) return;
     int64_t r = idx / H;
@@ -501,7 +489,6 @@ __global__ void gru_pointwise_kernel(const float* __restrict__ gi, const float* 
     float n = tanhf(a[2 * H + j] + rg * b[2 * H + j]);
     float hh = (1.f - z) * n + z * h_in[r * ldh_in + j];
     h_out[r * ldh_out + j] = hh;
-    if (h_out2) h_out2[r * ldh_out2 + j] = hh;
 }
 
 __global__ void copy_rows_kernel(const float* __restrict__ src, int64_t lds, float* __restrict__ dst, int64_t ldd,
@@ -650,6 +637,29 @@ __global__ void map_to_agents_kernel(const float* __restrict__ node_out, const f
     float s = 0.f;
     for (int n = 0; n < N; n++) s += node_out[((size_t)b * N + n) * O + o] * nam[((size_t)b * N + n) * A + a];
     agent_out[idx] = s;
+}
+
+int aggregate_rows(const float* h, int64_t ldh, float* M, int B, int N, int H, const int* nbr, const int* deg, int DM,
+                   const int* list_index, int mean, cudaStream_t s) {
+    aggregate_kernel<<<(unsigned)(((int64_t)B * N + 3) / 4), 128, 0, s>>>(h, ldh, M, B, N, H, nbr, deg, DM, list_index, mean);
+    GM_LAUNCH_CHECK();
+    return GM_OK;
+}
+
+int readout_rows(const float* h, int64_t ldh, const float* last, int64_t ldl, const float* gmean, const int* nbr,
+                 const int* deg, int DM, const int* list_index, const int* agent_node, int rows_per_graph, int B, int N,
+                 int H, int use_nbr, int use_glob, int max_degree, float* out, int64_t ldo, cudaStream_t s) {
+    readout_kernel<<<(unsigned)(((int64_t)B * rows_per_graph + 3) / 4), 128, 0, s>>>(
+        h, ldh, last, ldl, gmean, nbr, deg, DM, list_index, agent_node, rows_per_graph, B, N, H, use_nbr, use_glob,
+        max_degree, out, ldo);
+    GM_LAUNCH_CHECK();
+    return GM_OK;
+}
+
+int copy_rows(const float* src, int64_t lds, float* dst, int64_t ldd, int64_t R, int W, cudaStream_t s) {
+    copy_rows_kernel<<<(unsigned)((R * W + 255) / 256), 256, 0, s>>>(src, lds, dst, ldd, R, W);
+    GM_LAUNCH_CHECK();
+    return GM_OK;
 }
 
 // ---------------------------------------------------------------------------------------
@@ -1004,10 +1014,9 @@ int gm_netmon_forward(const gm_netmon_params* p, int32_t B, int32_t N, const flo
             h = hn; c = cn; ldh_cur = ldn; cur ^= 1;
         }
     } else {
-    // one recurrent cell: (xin [R,H], h_prev, c_prev) -> (h_new, c_new) (+ optional second copy)
+    // one recurrent cell: (xin [R,H], h_prev, c_prev) -> (h_new, c_new)
     auto run_cell = [&](const gm_cell_params& cp, const float* xin, int64_t ldxin, const float* hp, int64_t ldhp,
-                        const float* cprev, int64_t ldcp, float* hn, int64_t ldhn, float* cn, int64_t ldcn, float* hn2,
-                        int64_t ldhn2, float* cn2, int64_t ldcn2) -> int {
+                        const float* cprev, int64_t ldcp, float* hn, int64_t ldhn, float* cn, int64_t ldcn) -> int {
         int rc;
         if (p->rnn_type == GM_RNN_LSTM) {
             LinearArgs a{xin, ldxin, cp.w_ih, H, cp.b_ih, cp.b_hh, w.g0, 4 * H, R, 4 * H, H, -1, 0};
@@ -1015,16 +1024,14 @@ int gm_netmon_forward(const gm_netmon_params* p, int32_t B, int32_t N, const flo
             LinearArgs b{hp, ldhp, cp.w_hh, H, nullptr, nullptr, w.g0, 4 * H, R, 4 * H, H, -1, 1};
             if ((rc = linear_dispatch(b, math, lin_ws, lin_ws_bytes, s))) return rc;
             int64_t tot = R * H;
-            lstm_pointwise_kernel<<<(unsigned)((tot + 255) / 256), 256, 0, s>>>(w.g0, cprev, ldcp, hn, ldhn, cn, ldcn, hn2,
-                                                                              ldhn2, cn2, ldcn2, R, H);
+            lstm_pointwise_kernel<<<(unsigned)((tot + 255) / 256), 256, 0, s>>>(w.g0, cprev, ldcp, hn, ldhn, cn, ldcn, R, H);
             GM_LAUNCH_CHECK();
         } else if (p->rnn_type == GM_RNN_LNLSTM) {
             LinearArgs a{xin, ldxin, cp.w_ih, H, nullptr, nullptr, w.g0, 4 * H, R, 4 * H, H, -1, 0};
             if ((rc = linear_dispatch(a, math, lin_ws, lin_ws_bytes, s))) return rc;
             LinearArgs b{hp, ldhp, cp.w_hh, H, nullptr, nullptr, w.g1, 4 * H, R, 4 * H, H, -1, 0};
             if ((rc = linear_dispatch(b, math, lin_ws, lin_ws_bytes, s))) return rc;
-            lnlstm_pointwise_kernel<<<(unsigned)((R + 3) / 4), 128, 0, s>>>(w.g0, w.g1, cp, cprev, ldcp, hn, ldhn, cn, ldcn,
-                                                                           hn2, ldhn2, cn2, ldcn2, R, H);
+            lnlstm_pointwise_kernel<<<(unsigned)((R + 3) / 4), 128, 0, s>>>(w.g0, w.g1, cp, cprev, ldcp, hn, ldhn, cn, ldcn, R, H);
             GM_LAUNCH_CHECK();
         } else {  // GRU
             LinearArgs a{xin, ldxin, cp.w_ih, H, cp.b_ih, nullptr, w.g0, 3 * H, R, 3 * H, H, -1, 0};
@@ -1032,21 +1039,18 @@ int gm_netmon_forward(const gm_netmon_params* p, int32_t B, int32_t N, const flo
             LinearArgs b{hp, ldhp, cp.w_hh, H, cp.b_hh, nullptr, w.g1, 3 * H, R, 3 * H, H, -1, 0};
             if ((rc = linear_dispatch(b, math, lin_ws, lin_ws_bytes, s))) return rc;
             int64_t tot = R * H;
-            gru_pointwise_kernel<<<(unsigned)((tot + 255) / 256), 256, 0, s>>>(w.g0, w.g1, hp, ldhp, hn, ldhn, hn2, ldhn2, R,
-                                                                             H);
+            gru_pointwise_kernel<<<(unsigned)((tot + 255) / 256), 256, 0, s>>>(w.g0, w.g1, hp, ldhp, hn, ldhn, R, H);
             GM_LAUNCH_CHECK();
         }
         return GM_OK;
     };
 
     // ---- rnn_obs (model.py:490-495) -------------------------------------------------------
-    int cur = 0;
+    int cur = 0, rc;
     if (p->rnn_type != GM_RNN_NONE) {
         // no-carryover keeps (h0,c0) in state columns [0,2H) (model.py:566); those columns of
         // state_out are written at the very end from the ping-pong copy to stay alias-safe.
-        int rc = run_cell(p->rnn_obs, e, H, st_in, S, lstm_like ? st_in + H : nullptr, S, hbuf[0], H, cbuf[0], H, nullptr, 0,
-                          nullptr, 0);
-        if (rc) return rc;
+        if ((rc = run_cell(p->rnn_obs, e, H, st_in, S, lstm_like ? st_in + H : nullptr, S, hbuf[0], H, cbuf[0], H))) return rc;
         h = hbuf[0]; c = cbuf[0]; cur = 0;
     }
     // h0/c0 for the no-carry state live in hbuf[0]/cbuf[0]; keep them untouched in that mode
@@ -1055,28 +1059,19 @@ int gm_netmon_forward(const gm_netmon_params* p, int32_t B, int32_t N, const flo
     float* h0_keep = nullptr; float* c0_keep = nullptr;
     if (nocarry || gru_nocarry) {
         h0_keep = w.act0; c0_keep = w.act1;  // encoder buffers are free now (e was consumed)
-        int64_t tot = R * H;
-        copy_rows_kernel<<<(unsigned)((tot + 255) / 256), 256, 0, s>>>(hbuf[0], H, h0_keep, H, R, H);
-        GM_LAUNCH_CHECK();
-        if (nocarry) {
-            copy_rows_kernel<<<(unsigned)((tot + 255) / 256), 256, 0, s>>>(cbuf[0], H, c0_keep, H, R, H);
-            GM_LAUNCH_CHECK();
-        }
+        if ((rc = copy_rows(hbuf[0], H, h0_keep, H, R, H, s))) return rc;
+        if (nocarry && (rc = copy_rows(cbuf[0], H, c0_keep, H, R, H, s))) return rc;
     }
 
     // ---- K x (aggregate, rnn_update) (model.py:509-554) ----------------------------------
     float* none_buf[2] = {w.hA, w.hB};
     for (int it = 0; it < K; it++) {
         if (it == K - 1) last = h;
-        aggregate_kernel<<<(unsigned)((R + 3) / 4), 128, 0, s>>>(h, H, w.M, B, N, H, nbr_all, deg, DM, list_index,
-                                                                p->agg_type == GM_AGG_MEAN);
-        GM_LAUNCH_CHECK();
+        if ((rc = aggregate_rows(h, H, w.M, B, N, H, nbr_all, deg, DM, list_index, p->agg_type == GM_AGG_MEAN, s))) return rc;
         if (p->rnn_type == GM_RNN_NONE) {
             // h = M; `last` may alias the previous h buffer, so ping-pong
             float* dst = none_buf[it & 1];
-            int64_t tot = R * H;
-            copy_rows_kernel<<<(unsigned)((tot + 255) / 256), 256, 0, s>>>(w.M, H, dst, H, R, H);
-            GM_LAUNCH_CHECK();
+            if ((rc = copy_rows(w.M, H, dst, H, R, H, s))) return rc;
             h = dst;
             continue;
         }
@@ -1085,32 +1080,27 @@ int gm_netmon_forward(const gm_netmon_params* p, int32_t B, int32_t N, const flo
         if (nocarry && it == 0) { hp = st_in + 2 * H; ldhp = S; cpv = st_in + 3 * H; ldcp = S; }  // :538-539
         if (gru_nocarry && it == 0) { hp = st_in + H; ldhp = S; }                                  // :546-547
         int nxt = cur ^ 1;
-        int rc = run_cell(p->rnn_update, w.M, H, hp, ldhp, cpv, ldcp, hbuf[nxt], H, cbuf[nxt], H, nullptr, 0, nullptr, 0);
-        if (rc) return rc;
+        if ((rc = run_cell(p->rnn_update, w.M, H, hp, ldhp, cpv, ldcp, hbuf[nxt], H, cbuf[nxt], H))) return rc;
         h = hbuf[nxt]; c = cbuf[nxt]; cur = nxt;
     }
 
     // ---- new state (model.py:562-578) ------------------------------------------------------
-    {
-        int64_t tot = R * H;
-        unsigned g = (unsigned)((tot + 255) / 256);
-        if (lstm_like) {
-            int o = nocarry ? 2 * H : 0;
-            if (nocarry) {
-                copy_rows_kernel<<<g, 256, 0, s>>>(h0_keep, H, state_out, S, R, H); GM_LAUNCH_CHECK();
-                copy_rows_kernel<<<g, 256, 0, s>>>(c0_keep, H, state_out + H, S, R, H); GM_LAUNCH_CHECK();
-            }
-            copy_rows_kernel<<<g, 256, 0, s>>>(h, H, state_out + o, S, R, H); GM_LAUNCH_CHECK();
-            copy_rows_kernel<<<g, 256, 0, s>>>(c, H, state_out + o + H, S, R, H); GM_LAUNCH_CHECK();
-        } else if (gru_nocarry) {
-            // model.py:571 stacks (h0, h1) as [2,1,R,H]; _state_reshape_out (:449) then transposes the two LEADING
-            // axes only, so the flat state buffer is all of h0 followed by all of h1 (not interleaved per row).
-            // Reproduced, not fixed: the next step reads row r as [state0 | state1] = flat[r*2H : (r+1)*2H].
-            copy_rows_kernel<<<g, 256, 0, s>>>(h0_keep, H, state_out, H, R, H); GM_LAUNCH_CHECK();
-            copy_rows_kernel<<<g, 256, 0, s>>>(h, H, state_out + R * H, H, R, H); GM_LAUNCH_CHECK();
-        } else {
-            copy_rows_kernel<<<g, 256, 0, s>>>(h, H, state_out, S, R, H); GM_LAUNCH_CHECK();
+    if (lstm_like) {
+        int o = nocarry ? 2 * H : 0;
+        if (nocarry) {
+            if ((rc = copy_rows(h0_keep, H, state_out, S, R, H, s))) return rc;
+            if ((rc = copy_rows(c0_keep, H, state_out + H, S, R, H, s))) return rc;
         }
+        if ((rc = copy_rows(h, H, state_out + o, S, R, H, s))) return rc;
+        if ((rc = copy_rows(c, H, state_out + o + H, S, R, H, s))) return rc;
+    } else if (gru_nocarry) {
+        // model.py:571 stacks (h0, h1) as [2,1,R,H]; _state_reshape_out (:449) then transposes the two LEADING
+        // axes only, so the flat state buffer is all of h0 followed by all of h1 (not interleaved per row).
+        // Reproduced, not fixed: the next step reads row r as [state0 | state1] = flat[r*2H : (r+1)*2H].
+        if ((rc = copy_rows(h0_keep, H, state_out, H, R, H, s))) return rc;
+        if ((rc = copy_rows(h, H, state_out + R * H, H, R, H, s))) return rc;
+    } else {
+        if ((rc = copy_rows(h, H, state_out, S, R, H, s))) return rc;
     }
     }  // unfused path
 
@@ -1126,10 +1116,9 @@ int gm_netmon_forward(const gm_netmon_params* p, int32_t B, int32_t N, const flo
     }
     const int O = H + (use_glob ? H : 0) + (use_nbr ? max_degree * H : 0);
     if (node_out) {
-        readout_kernel<<<(unsigned)((R + 3) / 4), 128, 0, s>>>(h, ldh_cur, last, H, w.gmean, nbr_all, deg, DM, list_index,
-                                                              nullptr, N, B, N, H, use_nbr, use_glob, max_degree, node_out,
-                                                              O);
-        GM_LAUNCH_CHECK();
+        int rc = readout_rows(h, ldh_cur, last, H, w.gmean, nbr_all, deg, DM, list_index, nullptr, N, B, N, H, use_nbr,
+                              use_glob, max_degree, node_out, O, s);
+        if (rc) return rc;
     }
     if (agent_out_pk) {
         GM_CHECK_ARG(agent_node && A > 0 && (H % TC_BK) == 0 && ((uintptr_t)agent_out_pk & 127) == 0 &&
@@ -1149,11 +1138,8 @@ int gm_netmon_forward(const gm_netmon_params* p, int32_t B, int32_t N, const flo
         GM_LAUNCH_CHECK();
     } else if (agent_out) {
         GM_CHECK_ARG(agent_node && A > 0 && agent_out_ld >= O, "agent readout needs agent_node, A, ld >= %d", O);
-        int64_t rows = (int64_t)B * A;
-        readout_kernel<<<(unsigned)((rows + 3) / 4), 128, 0, s>>>(h, ldh_cur, last, H, w.gmean, nbr_all, deg, DM, list_index,
-                                                                 agent_node, A, B, N, H, use_nbr, use_glob, max_degree,
-                                                                 agent_out, agent_out_ld);
-        GM_LAUNCH_CHECK();
+        return readout_rows(h, ldh_cur, last, H, w.gmean, nbr_all, deg, DM, list_index, agent_node, A, B, N, H, use_nbr,
+                            use_glob, max_degree, agent_out, agent_out_ld, s);
     }
     return GM_OK;
 }

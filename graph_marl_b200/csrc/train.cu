@@ -18,6 +18,7 @@
 
 #include "common.cuh"
 #include "linear_simt.cuh"
+#include "netmon_rows.cuh"
 
 namespace gm {
 
@@ -199,12 +200,6 @@ __global__ void lstm_bwd_kernel(const float* __restrict__ gates, const float* __
 }
 
 // ---- LayerNormLSTM cell (layernormlstm.py:24-42), one warp per row -------------------------------------------
-__device__ __forceinline__ float wsum(float x) {
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) x += __shfl_xor_sync(FULL, x, o);
-    return x;
-}
-
 // training forward: gi / gh [R,4H] hold x W_ih^T and h W_hh^T and are overwritten with their NORMALISED values
 // (the LayerNorm backward needs y_hat and 1/sigma, not the raw rows); gates <- activated (i,f,g,o);
 // chat <- normalised pre-LN cell; stats[r] = (rstd_i, rstd_h, rstd_c)
@@ -219,13 +214,13 @@ __global__ void lnlstm_train_fwd_kernel(float* __restrict__ gi, float* __restric
     float* b = gh + r * G;
     float sa = 0.f, sb = 0.f;
     for (int c = lane; c < G; c += 32) { sa += a[c]; sb += b[c]; }
-    const float ma = wsum(sa) / (float)G, mb = wsum(sb) / (float)G;
+    const float ma = warp_sum(sa) / (float)G, mb = warp_sum(sb) / (float)G;
     float va = 0.f, vb = 0.f;
     for (int c = lane; c < G; c += 32) {
         const float da = a[c] - ma, db = b[c] - mb;
         va += da * da; vb += db * db;
     }
-    const float ra = 1.f / sqrtf(wsum(va) / (float)G + 1e-5f), rb = 1.f / sqrtf(wsum(vb) / (float)G + 1e-5f);
+    const float ra = 1.f / sqrtf(warp_sum(va) / (float)G + 1e-5f), rb = 1.f / sqrtf(warp_sum(vb) / (float)G + 1e-5f);
     float* g = gates + r * G;
     for (int c = lane; c < G; c += 32) {
         const float ya = (a[c] - ma) * ra, yb = (b[c] - mb) * rb;
@@ -241,10 +236,10 @@ __global__ void lnlstm_train_fwd_kernel(float* __restrict__ gi, float* __restric
         chat[r * H + j] = cpre;
         sc += cpre;
     }
-    const float mc = wsum(sc) / (float)H;
+    const float mc = warp_sum(sc) / (float)H;
     float vc = 0.f;
     for (int j = lane; j < H; j += 32) { const float d = chat[r * H + j] - mc; vc += d * d; }
-    const float rc = 1.f / sqrtf(wsum(vc) / (float)H + 1e-5f);
+    const float rc = 1.f / sqrtf(warp_sum(vc) / (float)H + 1e-5f);
     for (int j = lane; j < H; j += 32) {
         const float yc = (chat[r * H + j] - mc) * rc;
         const float c = yc * cp.ln_cell_w[j] + cp.ln_cell_b[j];
@@ -283,7 +278,7 @@ __global__ void lnlstm_bwd_kernel(const float* __restrict__ yi, const float* __r
         s2 += dy * chat[r * H + j];
         z[3 * H + j] = dh_ * tc * g[3 * H + j] * (1.f - g[3 * H + j]);
     }
-    const float m1 = wsum(s1) / (float)H, m2 = wsum(s2) / (float)H;
+    const float m1 = warp_sum(s1) / (float)H, m2 = warp_sum(s2) / (float)H;
     for (int j = lane; j < H; j += 32) {
         const float dy = dct[r * H + j] * cp.ln_cell_w[j];
         const float dcp = rc * (dy - m1 - chat[r * H + j] * m2);
@@ -304,7 +299,7 @@ __global__ void lnlstm_bwd_kernel(const float* __restrict__ yi, const float* __r
         a1 += da; a2 += da * a[c];
         b1 += db; b2 += db * b[c];
     }
-    a1 = wsum(a1) / (float)G; a2 = wsum(a2) / (float)G; b1 = wsum(b1) / (float)G; b2 = wsum(b2) / (float)G;
+    a1 = warp_sum(a1) / (float)G; a2 = warp_sum(a2) / (float)G; b1 = warp_sum(b1) / (float)G; b2 = warp_sum(b2) / (float)G;
     for (int c = lane; c < G; c += 32) {
         dgi[r * G + c] = ra * (z[c] * cp.ln_in_w[c] - a1 - a[c] * a2);
         dgh[r * G + c] = rb * (z[c] * cp.ln_hid_w[c] - b1 - b[c] * b2);
@@ -330,25 +325,7 @@ __global__ void __launch_bounds__(256) colsum_prod_kernel(const float* __restric
     }
 }
 
-// neighbour sum / mean (model.py:213-229), one warp per row; and its transpose as a scatter (any adjacency)
-__global__ void agg_fwd_kernel(const float* __restrict__ h, float* __restrict__ M, int B, int N, int H, const int* __restrict__ nbr,
-                               const int* __restrict__ deg, int DM, const int* __restrict__ list_index, int mean) {
-    const int64_t row = (int64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
-    const int lane = threadIdx.x & 31;
-    if (row >= (int64_t)B * N) return;
-    const int b = (int)(row / N), v = (int)(row - (int64_t)b * N);
-    const int li = list_index ? list_index[b] : b;
-    const int* lst = nbr + ((size_t)li * N + v) * DM;
-    const int dg = deg[(size_t)li * N + v];
-    const float* hb = h + (size_t)b * N * H;
-    for (int c = lane; c < H; c += 32) {
-        float acc = 0.f;
-        for (int q = 0; q < dg; q++) acc += hb[(size_t)lst[q] * H + c];
-        if (mean) acc /= (float)max(dg, 1);
-        M[row * H + c] = acc;
-    }
-}
-
+// transpose of the neighbour sum / mean (netmon.cu aggregate_kernel) as a scatter (any adjacency):
 // dh[u] += sum over rows v whose list holds u of dM[v] (/ deg_v for mean)
 __global__ void agg_bwd_kernel(const float* __restrict__ dM, float* __restrict__ dh, int B, int N, int H, const int* __restrict__ nbr,
                                const int* __restrict__ deg, int DM, const int* __restrict__ list_index, int mean) {
@@ -367,33 +344,7 @@ __global__ void agg_bwd_kernel(const float* __restrict__ dM, float* __restrict__
     }
 }
 
-// node readout (model.py:582-622): out[v] = [h[v] | last[n_1(v)] | ... | last[n_maxdeg(v)]], zero padded
-__global__ void readout_fwd_kernel(const float* __restrict__ h, const float* __restrict__ last, float* __restrict__ out, int B, int N, int H,
-                                   const int* __restrict__ nbr, const int* __restrict__ deg, int DM, const int* __restrict__ list_index,
-                                   int use_nbr, int max_degree) {
-    const int64_t row = (int64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
-    const int lane = threadIdx.x & 31;
-    if (row >= (int64_t)B * N) return;
-    const int b = (int)(row / N), v = (int)(row - (int64_t)b * N);
-    const int O = H + (use_nbr ? max_degree * H : 0);
-    float* o = out + row * O;
-    for (int c = lane; c < H; c += 32) o[c] = h[row * H + c];
-    if (!use_nbr) return;
-    const int li = list_index ? list_index[b] : b;
-    const int* lst = nbr + ((size_t)li * N + v) * DM;
-    const int dg = deg[(size_t)li * N + v];
-    int slot = 0;
-    for (int q = 0; q < dg && slot < max_degree; q++) {
-        const int u = lst[q];
-        if (u == v) continue;
-        const float* lu = last + ((size_t)b * N + u) * H;
-        for (int c = lane; c < H; c += 32) o[H + slot * H + c] = lu[c];
-        slot++;
-    }
-    for (; slot < max_degree; slot++)
-        for (int c = lane; c < H; c += 32) o[H + slot * H + c] = 0.f;
-}
-
+// transpose of the node readout (model.py:582-622, netmon.cu readout_kernel):
 // dh[v] = d_out[v, 0:H]; dlast[n_k(v)] += d_out[v, H(1+k) : H(2+k)]
 __global__ void readout_bwd_kernel(const float* __restrict__ d_out, float* __restrict__ dh, float* __restrict__ dlast, int B, int N, int H,
                                    const int* __restrict__ nbr, const int* __restrict__ deg, int DM, const int* __restrict__ list_index,
@@ -425,14 +376,6 @@ __global__ void add_rows_kernel(float* __restrict__ dst, int64_t ldd, const floa
     const int64_t r = idx / W;
     const int j = (int)(idx - r * W);
     dst[r * ldd + j] += src[r * lds + j];
-}
-
-__global__ void copy2_rows_kernel(const float* __restrict__ src, int64_t lds, float* __restrict__ dst, int64_t ldd, int64_t R, int W) {
-    const int64_t idx = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (idx >= R * W) return;
-    const int64_t r = idx / W;
-    const int j = (int)(idx - r * W);
-    dst[r * ldd + j] = src[r * lds + j];
 }
 
 // ---------------------------------------------------------------------------------------
@@ -698,21 +641,18 @@ int gm_netmon_forward_train(const gm_netmon_params* p, int32_t B, int32_t N, con
     for (int it = 0; it < K; it++) {  // :509-554
         const float* h = tape + T.h + (int64_t)it * R * H;
         float* M = tape + T.M + (int64_t)it * R * H;
-        agg_fwd_kernel<<<nblk(R, 4), 128, 0, s>>>(h, M, B, N, H, nbr_all, deg, DM, list_index, p->agg_type == GM_AGG_MEAN);
-        GM_LAUNCH_CHECK();
+        if ((rc = aggregate_rows(h, H, M, B, N, H, nbr_all, deg, DM, list_index, p->agg_type == GM_AGG_MEAN, s))) return rc;
         if ((rc = cell(p->rnn_update, M, h, H, tape + T.c + (int64_t)it * R * H, H, it + 1))) return rc;
     }
     const float* hK = tape + T.h + (int64_t)K * R * H;
     const float* cK = tape + T.c + (int64_t)K * R * H;
-    copy2_rows_kernel<<<nblk(R * H), 256, 0, s>>>(hK, H, state_out, 2 * H, R, H); GM_LAUNCH_CHECK();
-    copy2_rows_kernel<<<nblk(R * H), 256, 0, s>>>(cK, H, state_out + H, 2 * H, R, H); GM_LAUNCH_CHECK();
-    if (node_out) {
-        const float* last = tape + T.h + (int64_t)(K - 1) * R * H;  // h before the final iteration's aggregation (:510-519)
-        readout_fwd_kernel<<<nblk(R, 4), 128, 0, s>>>(hK, last, node_out, B, N, H, nbr_all, deg, DM, list_index, p->output_neighbor_hidden,
-                                                     max_degree);
-        GM_LAUNCH_CHECK();
-    }
-    return GM_OK;
+    if ((rc = copy_rows(hK, H, state_out, 2 * H, R, H, s))) return rc;
+    if ((rc = copy_rows(cK, H, state_out + H, 2 * H, R, H, s))) return rc;
+    if (!node_out) return GM_OK;
+    const float* last = tape + T.h + (int64_t)(K - 1) * R * H;  // h before the final iteration's aggregation (:510-519)
+    const int use_nbr = p->output_neighbor_hidden;
+    return readout_rows(hK, H, last, H, nullptr, nbr_all, deg, DM, list_index, nullptr, N, B, N, H, use_nbr, 0, max_degree,
+                        node_out, H + (use_nbr ? max_degree * H : 0), s);
 }
 
 int gm_netmon_backward(const gm_netmon_params* p, int32_t B, int32_t N, const float* node_obs, const int32_t* nbr_all, const int32_t* deg,
@@ -743,7 +683,7 @@ int gm_netmon_backward(const gm_netmon_params* p, int32_t B, int32_t N, const fl
     }
     if (d_state_out) {
         add_rows_kernel<<<nblk(R * H), 256, 0, s>>>(dh, H, d_state_out, 2 * H, R, H); GM_LAUNCH_CHECK();
-        copy2_rows_kernel<<<nblk(R * H), 256, 0, s>>>(d_state_out + H, 2 * H, dc, H, R, H); GM_LAUNCH_CHECK();
+        if ((rc = copy_rows(d_state_out + H, 2 * H, dc, H, R, H, s))) return rc;
     } else {
         GM_CUDA(cudaMemsetAsync(dc, 0, (size_t)R * H * 4, s));
     }

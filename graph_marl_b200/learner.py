@@ -15,18 +15,6 @@ from . import _lib
 from .model import _NetMonStepFn
 
 
-def netmon_step_params(nm):
-    """NetMon's parameters in the order _NetMonStepFn takes them: encoder (weight, bias) pairs, then each cell's."""
-    ps = [t for l in nm.encode.linear_layers for t in (l.weight, l.bias)]
-    for cell in (nm.rnn_obs, nm.rnn_update):
-        for path, _ in nm._cell_param_names():
-            obj = cell
-            for part in path.split("."):
-                obj = getattr(obj, part)
-            ps.append(obj)
-    return ps
-
-
 class Learner:
     def __init__(self, netmon, model, lr, gamma, tau, clip_value=0.5, max_norm=1.0, graph=True):
         """netmon / model: the online NetMon and DQN (their parameters are updated in place); the target DQN is a deepcopy
@@ -46,8 +34,7 @@ class Learner:
         # pair it was captured with; a larger batch must not reallocate them)
         self._ws_eager = self._new_workspaces()
         self._static = {}   # (buffer, batch, seq_len) -> static index / clock tensors and workspaces of the captured update
-        self._graphs = {}
-        self._graph_pool = None
+        self._graphs = CapturedUpdates()
         self.updates = 0
 
     def td_grad(self, q, q_next, action, reward, done, scale):
@@ -63,9 +50,6 @@ class Learner:
                                              q2.shape[0], nA, self.gamma, float(scale), dq.data_ptr(), self.loss.data_ptr(),
                                              self.opt.partials.data_ptr(), _lib.current_stream()))
         return dq.view(q.shape)
-
-    def _netmon_params(self):
-        return netmon_step_params(self.netmon)
 
     def _new_workspaces(self):
         return type(self.netmon._ws)(), type(self.target._ws)()
@@ -97,7 +81,7 @@ class Learner:
         scale = 1.0 / (n * A * nA * T)
         self.loss.zero_()
         torch._foreach_zero_([p.grad for p in self.params])
-        params = self._netmon_params()
+        params = nm.step_params()
         nnz, static_rows = getattr(be, "node_obs_nnz", 0), getattr(be, "node_static_rows", None)
         qs, dqs = [], []
         state, prev_end = None, None
@@ -153,23 +137,38 @@ class Learner:
             if s.get("pool") is not pool:  # new topology tables (random-topology pools): the captured update is stale
                 self._graphs.pop(key, None)
                 s["pool"] = pool
-            g = self._graphs.get(key)
-            if g is None and not s.get("warm"):
-                self._body(buff, s["idx"], clock, s["ws"])  # warm-up: workspaces, packs and autograd state exist before capture
-                s["warm"] = True
-            else:
-                if g is None:
-                    torch.cuda.synchronize()
-                    g = torch.cuda.CUDAGraph()
-                    with torch.cuda.graph(g, pool=self._graph_pool):
-                        self._body(buff, s["idx"], clock, s["ws"])
-                    if self._graph_pool is None:
-                        self._graph_pool = g.pool()
-                    self._graphs[key] = g
-                g.replay()
+            self._graphs.run(key, lambda: self._body(buff, s["idx"], clock, s["ws"]))
         self.refresh_packs()
         self.updates += 1
         return self.loss.clone()
+
+
+class CapturedUpdates(dict):
+    """key -> captured CUDA graph of an update, all captured into one shared memory pool.  The first run of a key is
+    eager, so that workspaces, weight packs and autograd state exist before capture; the second synchronises, captures
+    and replays; later runs replay.  A key popped from the dict is captured again on its next run, without another eager
+    run."""
+
+    def __init__(self):
+        super().__init__()
+        self._warm = set()
+        self._pool = None
+
+    def run(self, key, body):
+        g = self.get(key)
+        if g is None and key not in self._warm:
+            body()
+            self._warm.add(key)
+            return
+        if g is None:
+            torch.cuda.synchronize()
+            g = torch.cuda.CUDAGraph()
+            with torch.cuda.graph(g, pool=self._pool):
+                body()
+            if self._pool is None:
+                self._pool = g.pool()
+            self[key] = g
+        g.replay()
 
 
 class FusedOptimizer:

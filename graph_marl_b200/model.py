@@ -123,19 +123,32 @@ def _note_torch_path(who, why):
         warnings.warn(f"{who}: grad-mode forward runs the torch-composed path, not the CUDA kernels ({why})", stacklevel=3)
 
 
+def _mlp_fn_args(layers, activation_fn, activation_on_output, math):
+    """(spec, params) that _MlpFn takes for the nn.Linear `layers` with activation_fn after every layer but the last,
+    and after the last too when activation_on_output."""
+    act = _lib.ACTIVATIONS[_act_name(activation_fn)]
+    acts = (act,) * (len(layers) - 1) + (act if activation_on_output else -1,)
+    return (acts, math), [t for l in layers for t in (l.weight, l.bias)]
+
+
 class _MlpFn(torch.autograd.Function):
-    """y = MLP(x) through gm_mlp_forward_train / gm_mlp_backward.  `layers`: [(weight, bias, act_id)]."""
+    """y = MLP(x) through gm_mlp_forward_train / gm_mlp_backward.  spec: (activation ids per layer, math mode);
+    params: each layer's (weight, bias)."""
+
+    @staticmethod
+    def _desc(spec, x, params):
+        acts, math = spec
+        d = _lib.MlpDesc()
+        d.n_layers, d.in_features, d.math = len(acts), x.shape[1], _lib.MATH_MODES["bf16x3" if math == "bf16" else math]
+        for l in range(len(acts)):
+            w, b = params[2 * l], params[2 * l + 1]
+            d.units[l], d.act[l], d.w[l], d.b[l] = w.shape[0], acts[l], w.data_ptr(), b.data_ptr()
+        return d
 
     @staticmethod
     def forward(ctx, spec, x, *params):
-        acts, math = spec
-        L = len(acts)
         rows = x.shape[0]
-        d = _lib.MlpDesc()
-        d.n_layers, d.in_features, d.math = L, x.shape[1], _lib.MATH_MODES["bf16x3" if math == "bf16" else math]
-        for l in range(L):
-            w, b = params[2 * l], params[2 * l + 1]
-            d.units[l], d.act[l], d.w[l], d.b[l] = w.shape[0], acts[l], w.data_ptr(), b.data_ptr()
+        d = _MlpFn._desc(spec, x, params)
         lib = _lib.lib()
         tape = torch.empty(int(lib.gm_mlp_tape_floats(C.byref(d), rows)), dtype=torch.float32, device=x.device)
         ws = torch.empty(int(lib.gm_mlp_train_workspace_bytes(C.byref(d), rows)), dtype=torch.uint8, device=x.device)
@@ -144,24 +157,19 @@ class _MlpFn(torch.autograd.Function):
                                                 ws.numel(), _lib.current_stream()))
         ctx.save_for_backward(x, tape, *params)
         ctx.spec = spec
-        out_w = params[2 * (L - 1)].shape[0]
+        out_w = params[-2].shape[0]
         return tape[tape.numel() - rows * out_w:].view(rows, out_w).clone()
 
     @staticmethod
     def backward(ctx, d_out):
         x, tape, *params = ctx.saved_tensors
-        acts, math = ctx.spec
-        L = len(acts)
         rows = x.shape[0]
-        d = _lib.MlpDesc()
-        d.n_layers, d.in_features, d.math = L, x.shape[1], _lib.MATH_MODES["bf16x3" if math == "bf16" else math]
+        d = _MlpFn._desc(ctx.spec, x, params)
         g = _lib.MlpGrads()
         grads = []
-        for l in range(L):
-            w, b = params[2 * l], params[2 * l + 1]
-            d.units[l], d.act[l], d.w[l], d.b[l] = w.shape[0], acts[l], w.data_ptr(), b.data_ptr()
-            gw = torch.empty_like(w) if ctx.needs_input_grad[2 + 2 * l] else None
-            gb = torch.empty_like(b) if ctx.needs_input_grad[3 + 2 * l] else None
+        for l in range(len(ctx.spec[0])):
+            gw = torch.empty_like(params[2 * l]) if ctx.needs_input_grad[2 + 2 * l] else None
+            gb = torch.empty_like(params[2 * l + 1]) if ctx.needs_input_grad[3 + 2 * l] else None
             g.w[l], g.b[l] = _lib.ptr(gw), _lib.ptr(gb)
             grads += [gw, gb]
         d_out = d_out.float().contiguous()
@@ -371,12 +379,10 @@ class DQN(nn.Module):
             if x.is_cuda and _act_name(self.activation_fn) in _lib.ACTIVATIONS:
                 _lib.require_device()
                 GRAD_PATH_CALLS["device"] += 1
-                act = _lib.ACTIVATIONS[_act_name(self.activation_fn)]
-                layers = list(self.encoder.linear_layers) + [self.q_net.fc]
-                acts = tuple([act] * len(self.encoder.linear_layers) + [-1])
-                params = [t for l in layers for t in (l.weight, l.bias)]
+                spec, params = _mlp_fn_args(list(self.encoder.linear_layers) + [self.q_net.fc], self.activation_fn, False,
+                                            self.math)
                 x2 = x.reshape(-1, x.shape[-1]).float().contiguous()
-                q = _MlpFn.apply((acts, self.math), x2, *params)
+                q = _MlpFn.apply(spec, x2, *params)
                 return q.reshape(*x.shape[:-1], self.num_actions)
             _note_torch_path("DQN", "CPU tensors")
             return self.q_net(self.encoder(x))
@@ -636,6 +642,18 @@ class NetMon(nn.Module):
                     ("ln_cell.weight", "ln_cell_w"), ("ln_cell.bias", "ln_cell_b")]
         return [("weight_ih", "w_ih"), ("weight_hh", "w_hh"), ("bias_ih", "b_ih"), ("bias_hh", "b_hh")]
 
+    def step_params(self):
+        """The parameters in the order _NetMonStepFn takes them: the encoder's (weight, bias) pairs, then rnn_obs' and
+        rnn_update's in _cell_param_names() order."""
+        ps = [t for l in self.encode.linear_layers for t in (l.weight, l.bias)]
+        for cell in (self.rnn_obs, self.rnn_update):
+            for path, _ in self._cell_param_names():
+                obj = cell
+                for part in path.split("."):
+                    obj = getattr(obj, part)
+                ps.append(obj)
+        return ps
+
     def _device_backward_reason(self, x):
         """None when the device-side backward (csrc/train.cu) covers this configuration, else why not."""
         if not x.is_cuda:
@@ -665,15 +683,8 @@ class NetMon(nn.Module):
             st = self.state
             if st is not None:
                 st = st.to(x.device).float().reshape(B, N, self.state_size).contiguous()
-            layers = list(self.encode.linear_layers)
-            params = [t for l in layers for t in (l.weight, l.bias)]
-            for cell in (self.rnn_obs, self.rnn_update):
-                for path, _ in self._cell_param_names():
-                    obj = cell
-                    for part in path.split("."):
-                        obj = getattr(obj, part)
-                    params.append(obj)
-            node_out, self.state = _NetMonStepFn.apply(self, x.float().contiguous(), nbr, deg, None, md, st, *params)
+            node_out, self.state = _NetMonStepFn.apply(self, x.float().contiguous(), nbr, deg, None, md, st,
+                                                       *self.step_params())
             if no_agent_mapping:
                 return node_out
             return torch.bmm(node_out.transpose(1, 2), node_agent_matrix.to(node_out.dtype)).transpose(1, 2)

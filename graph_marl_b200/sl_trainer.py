@@ -33,8 +33,8 @@ import numpy as np
 import torch
 
 from . import _lib
-from .learner import FusedOptimizer, netmon_step_params
-from .model import NetMon, _act_name, _MlpFn, _NetMonStepFn
+from .learner import CapturedUpdates, FusedOptimizer
+from .model import NetMon, _mlp_fn_args, _MlpFn, _NetMonStepFn
 
 
 def adjacency_lists(node_adj, chunk=4096):
@@ -81,10 +81,8 @@ class SLTrainer:
         if layers[0].in_features != self.out_width or layers[-1].out_features != N:
             raise _lib.GraphMarlError(f"the head maps {layers[0].in_features} -> {layers[-1].out_features} features; "
                                       f"NetMon's per-node output is {self.out_width} wide and N = {N}")
-        act = lambda: _lib.ACTIVATIONS[_act_name(head.activation_fn)]
-        self._head_spec = (tuple(act() for _ in layers[:-1]) + (act() if head.activation_on_output else -1,), netmon.math)
-        self._nm_params = netmon_step_params(netmon)
-        self._head_params = [t for l in layers for t in (l.weight, l.bias)]
+        self._head_spec, self._head_params = _mlp_fn_args(layers, head.activation_fn, head.activation_on_output, netmon.math)
+        self._nm_params = netmon.step_params()
         # AdamW alone: no target pairs, clamp at +-inf and max_norm inf leave every gradient as it is
         self.opt = FusedOptimizer(list(netmon.parameters()) + list(head.parameters()), [], lr, 0.0,
                                   clip_value=float("inf"), max_norm=float("inf"))
@@ -94,8 +92,7 @@ class SLTrainer:
         self._pcg = torch.from_numpy(st.view(np.int64)).to(self.device)
         self.loss = torch.zeros((1,), dtype=torch.float32, device=self.device)  # loss of the latest update
         self._static = {}   # (batch, seq_len) -> static index / observation tensors of that update
-        self._graphs = {}
-        self._graph_pool = None
+        self._graphs = CapturedUpdates()
         self.last_indices = None
         self.updates = 0
 
@@ -141,20 +138,10 @@ class SLTrainer:
                                          li=torch.zeros((B,), dtype=torch.int32, device=dev),
                                          x=torch.empty((B,) + tuple(self.x.shape[1:]), dtype=torch.float32, device=dev))
         with torch.cuda.device(self.device), torch.enable_grad():
-            g = self._graphs.get(key)
-            if not self.graph or (g is None and not s.get("warm")):
-                self._body(s, B, T)  # graph mode: the warm-up, so that autograd state and allocations exist before capture
-                s["warm"] = True
+            if self.graph:
+                self._graphs.run(key, lambda: self._body(s, B, T))
             else:
-                if g is None:
-                    torch.cuda.synchronize()
-                    g = torch.cuda.CUDAGraph()
-                    with torch.cuda.graph(g, pool=self._graph_pool):
-                        self._body(s, B, T)
-                    if self._graph_pool is None:
-                        self._graph_pool = g.pool()
-                    self._graphs[key] = g
-                g.replay()
+                self._body(s, B, T)
         # the optimizer kernel writes the weights through raw pointers: repack them for the inference kernels
         self.netmon._pack.refresh()
         self.last_indices = s["idx"]
