@@ -103,6 +103,9 @@ class NetmonGrads(C.Structure):
 
 
 GM_LEARNER_PARTIALS = 296
+# gm_eval_accumulate's row layout (GM_EVAL_* in the header), in field order
+EVAL_FIELDS = ("reward_sum", "agent_steps", "delay_sum", "delay_count", "arrived_delay_sum", "arrived_count", "spr_sum",
+               "looped", "throughput", "dropped", "blocked", "steps")
 
 
 class OptEntry(C.Structure):
@@ -176,6 +179,7 @@ _SIGS = {
                              C.c_float, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "gm_sl_mse_grad": (C.c_int, [C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_float, C.c_void_p,
                                  C.c_void_p, C.c_void_p, C.c_void_p]),
+    "gm_eval_accumulate": (C.c_int, [C.c_void_p] * 6 + [C.c_int32, C.c_int32, C.c_void_p, C.c_void_p]),
     "gm_optimizer_step": (C.c_int, [C.c_void_p, C.c_int32, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p,
                                     C.c_void_p]),
     "gm_mlp_tape_floats": (C.c_int64, [C.c_void_p, C.c_int64]),

@@ -18,7 +18,7 @@ LIB = os.path.join(LIBDIR, "libgraphmarl_b200.so")
 INCLUDE = os.path.join(os.path.dirname(HERE), "include")
 
 SOURCES = ["runtime.cu", "routing_env.cu", "simple_env.cu", "netmon.cu", "gemm_dispatch.cu", "linear_simt.cu",
-           "gemm_sm100.cu", "dqn.cu", "replay.cu", "replay_sampler.cu", "train.cu", "learner.cu", "topology.cu", "host_topology.cpp", "collective.cpp"]
+           "gemm_sm100.cu", "dqn.cu", "replay.cu", "replay_sampler.cu", "train.cu", "learner.cu", "eval_metrics.cu", "topology.cu", "host_topology.cpp", "collective.cpp"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC", "-Xcompiler", "-fvisibility=hidden", "-x", "cu",
               "--expt-relaxed-constexpr", "-I", INCLUDE]

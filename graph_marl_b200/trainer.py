@@ -5,6 +5,7 @@ import torch
 
 from .env.routing import Routing
 from .env.wrapper import NetMonWrapper
+from .evaluation import evaluate_topologies, run_episodes
 from .learner import Learner
 from .rollout import Rollout
 from .util import get_state_dict
@@ -83,20 +84,25 @@ class Trainer:
             # the captured rollout units read
             be._pool = r.base_env._pool
             self._eval = NetMonWrapper(be, r.netmon, 1, split_obs=True, graph_obs_fp32=True)
-        env = self._eval
         saved = r.netmon.state
         total = torch.zeros((), dtype=torch.float64, device=r.device)
         steps = 0
         with torch.no_grad():
-            for _ in range(int(episodes)):
-                (obs_a, obs_g), _ = env.reset()
-                for _ in range(c["episode_steps"]):
-                    steps += 1
-                    _, act = r.model.act(obs_a, obs_g, epsilon=float(epsilon), seed=12345, step=steps, want_q=False)
-                    (obs_a, obs_g), _, reward, _, _ = env.step(act)
-                    total += reward.double().mean()
+            for reward, _, _ in run_episodes(self._eval, r.model, episodes, c["episode_steps"], epsilon):
+                steps += 1
+                total += reward.double().mean()
         r.netmon.state = saved
         return float(total) / steps
+
+    def evaluate_topologies(self, seeds, episode_steps=None, epsilon=0.0):
+        """evaluation.evaluate_topologies of the current policy on the topologies of `seeds` (e.g. env.constants.EVAL_SEEDS),
+        with the rollout's n_data, congestion and (by default) episode length.  Works for every config: it runs on copies
+        of the modules and on a topology pool of its own, so the training run is not touched."""
+        r = self.rollout
+        c = r.cfg
+        return evaluate_topologies(r.netmon, r.model, seeds, c["n_data"],
+                                   c["episode_steps"] if episode_steps is None else episode_steps,
+                                   congestion=c["congestion"], epsilon=epsilon, env_seed=self.args["seed"] + 7919)
 
     def state_dict(self):
         """Checkpoint in the reference's layout (util.get_state_dict): loads with the reference's util.load_state_dict."""

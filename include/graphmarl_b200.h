@@ -518,6 +518,29 @@ GM_API int gm_optimizer_step(const gm_opt_entry* table_dev, int32_t n_entries, c
                       int32_t n_pairs, int64_t* step_dev, const gm_opt_hparams* h, double* partials, void* stream);
 
 /* ======================================================================== */
+/* Batched evaluation (graph_marl_b200/evaluation.py): per-env sums of the   */
+/* episode metrics, one row of GM_EVAL_FIELDS doubles per env.  No atomics:  */
+/* repeated and captured launches agree bit for bit.                         */
+/* ======================================================================== */
+#define GM_EVAL_REWARD_SUM 0         /* sum of rewards over agents and steps */
+#define GM_EVAL_AGENT_STEPS 1        /* agents x steps */
+#define GM_EVAL_DELAY_SUM 2          /* sum of delays of done packets */
+#define GM_EVAL_DELAY_COUNT 3        /* done packets */
+#define GM_EVAL_ARRIVED_DELAY_SUM 4  /* sum of delays of arrived packets */
+#define GM_EVAL_ARRIVED_COUNT 5      /* arrived packets */
+#define GM_EVAL_SPR_SUM 6            /* sum of spr of arrived packets */
+#define GM_EVAL_LOOPED 7             /* sums of info[:, 0..3] */
+#define GM_EVAL_THROUGHPUT 8
+#define GM_EVAL_DROPPED 9
+#define GM_EVAL_BLOCKED 10
+#define GM_EVAL_STEPS 11             /* env steps */
+#define GM_EVAL_FIELDS 12
+/* One env step's outputs (gm_routing_io: reward f32[B,A], done u8[B,A], arrived u8[B,A], delays i32[B,A], spr f64[B,A],
+ * info i32[B,4]) added into acc f64[B, GM_EVAL_FIELDS]. */
+GM_API int gm_eval_accumulate(const float* reward, const uint8_t* done, const uint8_t* arrived, const int32_t* delays,
+                              const double* spr, const int32_t* info, int32_t B, int32_t A, double* acc, void* stream);
+
+/* ======================================================================== */
 /* building blocks exposed for tests / profiling                             */
 /* ======================================================================== */
 /* C[M,N] = act(A[M,K] * W[N,K]^T + bias) in the requested math mode */
